@@ -215,6 +215,30 @@ def cpu_reference(phovo, K, pairs, threads, steps, warmup, lean=False, depth="u1
             "mean_iterations_per_pair": {str(l): float(it[:, l].mean()) for l in range(cfg.num_levels) if cfg.max_num_iterations[l] > 0}}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the arrays the timed path returned in its last step, as <out_dir>/<name>.npy in float64,
+    so that two builds can be compared output for output on the same seeded inputs.  When together they exceed
+    64 MB, the arrays (which then share their first axis, the pair) keep a fixed, seeded sample of pairs whose
+    indices are written as pair_index.npy."""
+    import numpy as np
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        n = {a.shape[0] for a in arrays.values()}
+        assert len(n) == 1, "outputs larger than the dump limit must share their first axis"
+        n = n.pop()
+        keep = DUMP_LIMIT_BYTES * n // (total + 8 * n)      # the index costs 8 B per kept pair
+        idx = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["pair_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def workload_config(pairs_per_gpu, depth, world):
     """`config` of the JSON line: the workload and nothing measured, identical in both arms."""
     return {"workload": "batched independent 640x480 RGB-D pairs, %s (BASELINE configs[3]), %d pairs per GPU per step" % (CONFIG, pairs_per_gpu),
@@ -447,6 +471,9 @@ def run_8k(args, phovo, rank, world, local_rank, host_threads):
             t0 = time.perf_counter(); o.optimize(); t1 = time.perf_counter()
             if s_ >= args.warmup:
                 ts.append((t1 - t0) * 1e3)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"state": o.state(),
+                                             "iterations_per_level": np.bincount([e["level"] for e in o.iter_stats()], minlength=phovo.MAXL)})
         v = float(np.mean(ts))
         assert "libphovo_b200" not in open("/proc/self/maps").read()
         print(json.dumps({"impl": "reference", "metric": METRIC_8K, "value": v, "unit": "ms", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -511,6 +538,8 @@ def run_8k(args, phovo, rank, world, local_rank, host_threads):
     barrier()
     t_all = time.perf_counter() - t_all0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"state": st, "iterations_per_level": [executed.get(l, 0) for l in range(phovo.MAXL)]})
     t = torch.tensor([float(np.mean(dev_ms)), float(np.mean(wall_ms))], dtype=torch.float64, device=dev)
     mine = torch.tensor(st, dtype=torch.float64, device=dev)
     gathered = torch.zeros((world, 6), dtype=torch.float64, device=dev)
@@ -572,6 +601,9 @@ def main():
     ap.add_argument("--secondary-frames", type=int, default=1000, help="frames of the synthetic VO sequence (BASELINE configs[1])")
     ap.add_argument("--depth", default="u16", choices=["u16", "f32"],
                     help="depth format at the boundary: raw u16 sensor units x 1/5000 m (what the reference apps read, default) or f32 metres")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (poses and iteration counts) as DIR/<name>.npy (rank 0); "
+                         "with --impl reference the number of pairs is --cpu-pairs, which defaults to one depending on the host's core count")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -590,6 +622,8 @@ def main():
             return 0
         pairs = args.cpu_pairs or max(64, 2 * host_threads)
         r = cpu_reference(phovo, K, pairs, host_threads, args.steps, max(args.warmup, 1), depth=args.depth)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"states": r["states"], "iterations": r["iters"]})
         line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "pairs/s", "n_gpus": args.gpus,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -660,6 +694,14 @@ def main():
     barrier()
     clocks = sampler.stop()
     elapsed_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:
+        iters_all = iters
+        if world > 1:
+            iters_all = torch.zeros((world * P, phovo.MAXL), dtype=torch.int32, device=dev)
+            dist.all_gather_into_tensor(iters_all, iters)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"states": (gathered if world > 1 else states).cpu().numpy(),
+                                             "iterations": iters_all.cpu().numpy()})
     launches = odo.LaunchCount() - launches0
     # per-kernel CUDA-event times (recorded inside the library on the same stream), one more step
     for _ in range(3):

@@ -9,9 +9,9 @@
  * so both apps switch to it by adding one `#elif USE_PHOTOCONSISTENCY_ODOMETRY_METHOD == 3` branch
  * (INTEGRATION.md).  The header only touches `.rows .cols .data .step` of the cv::Mat_ arguments and
  * `operator()` of the Eigen-derived matrix types, and it includes "CPhotoconsistencyOdometry.h" by
- * name: that is the reference's own header, also in this repository's tests
- * (tests/cpp/build_adapter_test.sh compiles against /root/reference/phovo/include unmodified; only
- * OpenCV and Eigen, which are not installed here, are the stand-ins of oracle/shim).
+ * name: that is the reference's own header.  tests/cpp/build_adapter_test.sh compiles against it,
+ * unmodified, when REF names a checkout of the original project, and otherwise against the stand-in
+ * tests/cpp/shim/CPhotoconsistencyOdometry.h; OpenCV and Eigen are the stand-ins of oracle/shim.
  *
  * Error behaviour: the reference returns void and never checks anything; this adapter keeps the
  * void signatures and throws std::runtime_error when the C ABI reports a failure (bad call order,

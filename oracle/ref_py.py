@@ -1,10 +1,10 @@
 """ctypes binding of oracle/_ref/libphovo_ref.so: the reference's OWN
 CPhotoconsistencyOdometryAnalytic<unsigned char,double>, compiled unmodified from
-/root/reference/phovo/include against the OpenCV/Eigen stand-ins in oracle/shim (oracle/Makefile).
+$REF/phovo/include against the OpenCV/Eigen stand-ins in oracle/shim (oracle/Makefile).
 
 TEST INFRASTRUCTURE.  Used to pin the C oracle (and through it the CUDA path) against the reference
-source itself, and to mint tests/golden/ref_*.npz.  The library is built in the build container
-(where /root/reference exists) and travels to the GPU box as a prebuilt, git-ignored file.
+source itself, and to mint tests/golden/ref_*.npz.  The library is built where REF names a checkout
+of the original project; it is git-ignored, and the tests that need it skip without it.
 """
 import ctypes as C
 import os
@@ -17,7 +17,8 @@ LIB = os.path.join(_HERE, "_ref", "libphovo_ref.so")
 
 
 def available():
-    if not os.path.exists(LIB) and os.path.isdir("/root/reference/phovo/include"):
+    ref = os.environ.get("REF")
+    if not os.path.exists(LIB) and ref and os.path.isdir(os.path.join(ref, "phovo", "include")):
         subprocess.call(["make", "-s", "-C", _HERE, "ref"], stdout=subprocess.DEVNULL)
     return os.path.exists(LIB)
 
@@ -29,7 +30,7 @@ def lib():
     global _lib
     if _lib is None:
         if not available():
-            raise RuntimeError("oracle/_ref/libphovo_ref.so is not built (needs /root/reference)")
+            raise RuntimeError("oracle/_ref/libphovo_ref.so is not built (set REF to a checkout of the original project)")
         L = C.CDLL(LIB)
         vp, dp = C.c_void_p, C.POINTER(C.c_double)
         L.ref_create.restype = vp

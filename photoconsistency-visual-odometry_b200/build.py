@@ -64,7 +64,7 @@ def _build_locked(verbose):
             raise RuntimeError("nvcc failed on %s" % src)
         objs.append(obj)
     with open(os.path.join(CSRC, "ptxas_v.log"), "w") as f:
-        # compile times differ from run to run: keep the log stable under version control
+        # compile times differ from run to run: keep logs of two builds comparable
         f.write("\n".join(ln for chunk in log for ln in chunk.splitlines() if "Compile time" not in ln) + "\n")
     tmp = LIB + ".tmp.%d" % os.getpid()
     cmd = [nvcc, "-shared", "-o", tmp] + objs + ["-gencode", "arch=compute_100a,code=sm_100a", "-lcudart"]

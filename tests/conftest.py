@@ -11,7 +11,8 @@ if os.path.join(ROOT, "oracle") not in sys.path:
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 PKG = "photoconsistency-visual-odometry_b200"
-REF_CONFIG_DIR = "/root/reference/config_files"  # only present in the build container
+# config_files/ of a checkout of the original project, named by REF (the adapter build reads the same variable)
+REF_CONFIG_DIR = os.path.join(os.environ["REF"], "config_files") if os.environ.get("REF") else ""
 
 
 def pytest_configure(config):

@@ -1,9 +1,10 @@
 #!/bin/bash
-# Compiles the drop-in C++ adapter (include/CPhotoconsistencyOdometryCuda.h) against the REFERENCE'S OWN
-# abstract class and matrix types -- /root/reference/phovo/include/CPhotoconsistencyOdometry.h + Matrix.h,
-# unmodified, where they lie -- with OpenCV / Eigen replaced by the stand-ins of oracle/shim (neither is
-# installed here), and links two programs against the in-tree libphovo_b200.so:
+# Compiles the drop-in C++ adapter (include/CPhotoconsistencyOdometryCuda.h) against the reference's
+# abstract class and matrix types, with OpenCV / Eigen replaced by the stand-ins of oracle/shim, and
+# links programs against the in-tree libphovo_b200.so:
 #   _build/frame_alignment_app      the headless mirror of both apps' main() (tests/cpp/frame_alignment_app.cpp)
+# Where REF names a checkout of the original project, the adapter is compiled against its own
+# phovo/include/CPhotoconsistencyOdometry.h + Matrix.h, unmodified, and two more programs are built:
 #   _build/reference_frame_alignment  a copy of the reference's apps/PhotoconsistencyFrameAlignment/
 #                                   PhotoconsistencyFrameAlignment.cpp with exactly the INTEGRATION.md patch
 #                                   applied (USE_PHOTOCONSISTENCY_ODOMETRY_METHOD == 3); the patched copy
@@ -11,28 +12,31 @@
 #   _build/reference_visual_odometry  the same for apps/PhotoconsistencyVisualOdometry/PhotoconsistencyVisualOdometry.cpp
 #                                   (with the reference's own CCameraRecord / CMultiSensorDataSource / CImageReader
 #                                   headers; Boost.Filesystem is std::filesystem behind oracle/shim/boost).
-# The reference tree exists only in the build container: elsewhere (the GPU box) the prebuilt binaries,
-# which travel with the snapshot, are used as they are.
+# Without REF the base class comes from tests/cpp/shim/CPhotoconsistencyOdometry.h, which declares the
+# same interface.
 set -e
 HERE="$(cd "$(dirname "$0")" && pwd)"
 ROOT="$(cd "$HERE/../.." && pwd)"
 PKG="$ROOT/photoconsistency-visual-odometry_b200"
-REF="${REF:-/root/reference}"
+REF="${REF:-}"
 OUT="$HERE/_build"
 mkdir -p "$OUT"
-if [ ! -d "$REF/phovo/include" ]; then
-  if [ -x "$OUT/frame_alignment_app" ] && [ -x "$OUT/reference_frame_alignment" ] && [ -x "$OUT/reference_visual_odometry" ]; then
-    echo "reference tree not present: using the prebuilt $OUT/{frame_alignment_app,reference_frame_alignment,reference_visual_odometry}"
-    exit 0
-  fi
-  echo "reference tree not present and no prebuilt adapter binaries under $OUT" >&2
+if [ -n "$REF" ] && [ ! -d "$REF/phovo/include" ]; then
+  echo "REF=$REF is not a checkout of the original project (no phovo/include)" >&2
   exit 1
 fi
-INC=(-I "$ROOT/include" -I "$REF/phovo/include" -I "$ROOT/oracle/shim" -I "$ROOT/oracle/shim/eigen3")
+BASE="$HERE/shim"
+[ -n "$REF" ] && BASE="$REF/phovo/include"
+INC=(-I "$ROOT/include" -I "$BASE" -I "$ROOT/oracle/shim" -I "$ROOT/oracle/shim/eigen3")
 LINK=(-L "$PKG" -lphovo_b200 -Wl,-rpath,"\$ORIGIN/../../../photoconsistency-visual-odometry_b200"
       -L /usr/local/cuda/lib64 -Wl,-rpath,/usr/local/cuda/lib64 -lcudart)
 g++ -std=c++11 -O2 -Wall -Wextra -Wno-unused-parameter "${INC[@]}" "$HERE/frame_alignment_app.cpp" -o "$OUT/frame_alignment_app" "${LINK[@]}"
 echo "built $OUT/frame_alignment_app"
+if [ -z "$REF" ]; then
+  rm -f "$OUT"/reference_* "$OUT"/Photoconsistency*_method3.cpp
+  echo "REF not set: the reference apps are not built"
+  exit 0
+fi
 
 # the reference apps themselves + the INTEGRATION.md patch
 patch_app() {   # <reference source> <patched copy> <what the object-definition branch declares>

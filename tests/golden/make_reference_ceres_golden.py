@@ -11,7 +11,8 @@ pair.  For each of the 5 levels and each of 3 states: J^T J (21), J^T r (6), cos
 non-zero residual slots formed from the functor's full output, and the functor's residual +
 1x6 Jacobian themselves on a subset of target slots (the whole level for the two coarsest levels;
 for the finer ones the two outermost rows / columns on every side -- where sample.h:36-49 clamps and
-extrapolates -- plus a seeded random sample).  State 0 is the IDENTITY the apps start from
+extrapolates -- plus a seeded random sample), of which a seeded quarter is stored so that the file
+stays under 1 MB.  State 0 is the IDENTITY the apps start from
 (every projected coordinate on an integer, CE:250-251 truncates), states 1 and 2 lie along the way.
 """
 import importlib
@@ -30,6 +31,7 @@ import ref_py  # noqa: E402
 phovo = importlib.import_module("photoconsistency-visual-odometry_b200")
 
 IDX = [(a, b) for a in range(6) for b in range(a, 6)]
+KEEP = 0.25   # share of the sampled slots whose residual + Jacobian are stored
 STATES = np.array([np.zeros(6),
                    [0.004, -0.003, 0.006, 0.003, -0.002, 0.0015],
                    [0.0195, -0.0102, 0.0153, 0.0099, -0.0081, 0.0061]])
@@ -67,6 +69,7 @@ def main():
     out = dict(gray0=g0, depth0=d0.astype(np.float32), gray1=g1, K=K, config=np.array(cfg), states=STATES)
     for lvl, shape in enumerate(level_shapes(rows, cols, 5)):
         idx = sample_slots(shape, [1000, 800, 600, 600, 0][lvl], 100 + lvl)
+        idx = np.sort(np.random.default_rng(200 + lvl).choice(idx, size=int(round(KEEP * len(idx))), replace=False))
         out["idx%d" % lvl] = idx
         for s, st in enumerate(STATES):
             res, jac = ref.evaluate(shape, st)

@@ -65,7 +65,7 @@ def test_yaml_reader(phovo, tmp_path, name):
         assert cfg.num_threads == want["num_threads"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CONFIG_DIR), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(REF_CONFIG_DIR), reason="needs the original project's config_files: set REF to a checkout of it")
 def test_config_table_matches_reference_files(phovo, tmp_path):
     """The table in configs.py against the reference's own files, read by our parser AND by
     OpenCV's FileStorage (what the reference itself uses)."""

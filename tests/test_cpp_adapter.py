@@ -1,13 +1,15 @@
-"""The C++ drop-in adapter (include/CPhotoconsistencyOdometryCuda.h), compiled against the REFERENCE'S OWN
-abstract class and matrix types (/root/reference/phovo/include/CPhotoconsistencyOdometry.h + Matrix.h,
-unmodified; only OpenCV / Eigen are the stand-ins of oracle/shim), checked against the CPU oracle:
+"""The C++ drop-in adapter (include/CPhotoconsistencyOdometryCuda.h), compiled against the reference's
+abstract class and matrix types (its own phovo/include/CPhotoconsistencyOdometry.h + Matrix.h when
+REF names a checkout of the original project, else the stand-in tests/cpp/shim/CPhotoconsistencyOdometry.h;
+OpenCV / Eigen are the stand-ins of oracle/shim), checked against the CPU oracle:
 
   * tests/cpp/frame_alignment_app.cpp -- headless mirror of both apps' main() (strided cv::Mat_ inputs,
     the VO loop, warpImage through the adapter);
   * the reference's apps/PhotoconsistencyFrameAlignment/PhotoconsistencyFrameAlignment.cpp and
     apps/PhotoconsistencyVisualOdometry/PhotoconsistencyVisualOdometry.cpp THEMSELVES with exactly the
     INTEGRATION.md patch applied (USE_PHOTOCONSISTENCY_ODOMETRY_METHOD == 3), built by
-    tests/cpp/build_adapter_test.sh into tests/cpp/_build/ (git-ignored; travels to the GPU box).
+    tests/cpp/build_adapter_test.sh into tests/cpp/_build/ (git-ignored) from the checkout REF names;
+    their tests skip without one.
 """
 import os
 import subprocess
@@ -27,6 +29,12 @@ REF_VO_APP = os.path.join(ROOT, "tests", "cpp", "_build", "reference_visual_odom
 def build_app():
     subprocess.check_call(["bash", os.path.join(ROOT, "tests", "cpp", "build_adapter_test.sh")], stdout=subprocess.DEVNULL)
     return APP
+
+
+def build_reference_apps():
+    build_app()
+    if not os.environ.get("REF"):
+        pytest.skip("the reference apps are built from a checkout of the original project: set REF to one")
 
 
 def test_adapter_compiles_and_fails_loudly_without_gpu(phovo, tmp_path):
@@ -66,8 +74,7 @@ def test_reference_app_with_the_integration_patch_builds_and_fails_loudly_withou
     """The reference's own FrameAlignment main() + the METHOD == 3 branch compiles against the real
     CPhotoconsistencyOdometry.h / Matrix.h; without a device the adapter's constructor throws (the app
     has no handler: it terminates, it does not fall back to anything)."""
-    build_app()
-    assert os.access(REF_APP, os.X_OK)
+    build_reference_apps()
     import torch
     if torch.cuda.is_available():
         pytest.skip("GPU present: covered by the gpu tests")
@@ -81,7 +88,7 @@ def test_reference_app_with_the_integration_patch_builds_and_fails_loudly_withou
 def test_reference_frame_alignment_app_method_3_matches_oracle(phovo, oracle, tmp_path):
     """apps/PhotoconsistencyFrameAlignment/PhotoconsistencyFrameAlignment.cpp, unmodified but for the
     INTEGRATION.md patch, run on the GPU: the Rt it prints (:109-110) equals the oracle's."""
-    build_app()
+    build_reference_apps()
     K, g0, d0, g1, paths = reference_app_inputs(phovo, tmp_path, 22)
     name = "config_4_level_optimization_analytic"
     yml = phovo.configs.write_yaml(name, str(tmp_path))
@@ -182,7 +189,7 @@ def test_reference_visual_odometry_app_method_3_trajectory_matches_oracle(phovo,
     """apps/PhotoconsistencyVisualOdometry/PhotoconsistencyVisualOdometry.cpp, unmodified but for the INTEGRATION.md
     patch, on a recorded sequence (rgb.txt / depth.txt + image files read by the reference's own CCameraRecord /
     CImageReader): the TUM trajectory it writes (:240-243) equals the oracle's frame-by-frame loop."""
-    build_app()
+    build_reference_apps()
     K = phovo.synth.K_VISUAL_ODOMETRY                      # hard-coded in the app (VisualOdometry.cpp:171-173)
     n = 5
     os.makedirs(tmp_path / "rgb"); os.makedirs(tmp_path / "depth")

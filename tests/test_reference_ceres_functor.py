@@ -98,7 +98,7 @@ def test_oracle_ceres_matches_reference_golden(phovo, oracle):
 def test_oracle_ceres_matches_reference_functor_live(phovo, oracle, tmp_path, cfg_name, shape, seed):
     import ref_py
     if not ref_py.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference) and no prebuilt library present")
+        pytest.skip("oracle/_ref not built: set REF to a checkout of the original project")
     K = phovo.synth.K_FRAME_ALIGNMENT.copy()
     K[:2] *= shape[1] / 640.
     g0, d0, g1, _ = phovo.synth.make_pair(shape[0], shape[1], K=K, seed=seed)

@@ -66,7 +66,7 @@ def test_oracle_matches_reference_golden(phovo, oracle, name):
 def test_oracle_matches_reference_source_live(phovo, oracle, tmp_path, cfg_name, shape, K_name):
     import ref_py
     if not ref_py.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference) and no prebuilt library present")
+        pytest.skip("oracle/_ref not built: set REF to a checkout of the original project")
     K = getattr(phovo.synth, K_name).copy()
     if shape != (480, 640):
         K[:2] *= shape[1] / 640.

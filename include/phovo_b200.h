@@ -258,12 +258,29 @@ int phovo_batch_num_iter_stats(const phovo_ctx* ctx, int pair);
 /* test hooks of the batch kernel (results must not change): bit 0 = every pixel takes the exact
  * reference warp instead of the estimate-then-verify shortcut; bit 1 = use the generic
  * thread->pixel bookkeeping even when the CTA width is a multiple of the level width; bit 2 / bit 3 = what the
- * resident kernels do not take goes through the pool of per-pair contexts / the slot waves whatever the batch size */
+ * resident kernels do not take goes through the pool of per-pair contexts / the slot waves whatever the batch size;
+ * bit 4 = the warpImage entries clear their splat keys with a memset per chunk instead of in the resolve pass */
 int phovo_batch_set_debug_flags(phovo_ctx* ctx, int flags);
+/* phovo::warpImage (BASE:73-134) + the apps' cv::absdiff for P pairs of one size and intrinsics.
+ * gray0 / depth0 / gray1 are dense [P][rows][cols], all host or all device (as phovo_batch_align);
+ * rts [P][16] row-major 4x4 (host or device) as phovo_state_to_rt / phovo_get_rt return them;
+ * outputs may each be NULL, host or device: warped / diff [P][rows][cols] u8,
+ * num_landed [P] (source pixels that landed in the target), sum_abs_diff [P] (sum of
+ * |gray1 - warped| over those pixels).  diff and sum_abs_diff need gray1.  Blocking.
+ * Every image equals what phovo_warp_image gives pair by pair, bit for bit; the summaries are integer sums, the same
+ * whatever the chunking.  A source pixel of gray 0 that lands counts in num_landed although `warped` cannot show it.
+ * PHOVO_E_INVALID: bad sizes or level, unknown depth type, P < 1, diff / sum_abs_diff without gray1, no output;
+ * PHOVO_E_UNSUPPORTED: frames of 2^31 pixels or more.  Pairs run in chunks whose splat keys (4 B per pixel) fit in
+ * half of the L2 (640x480 on B200: 51 pairs); debug flag 16 clears the keys with a memset per chunk instead of in the
+ * resolve pass (same results). */
+int phovo_batch_warp_image(phovo_ctx* ctx, int num_pairs, int rows, int cols,
+                           const uint8_t* gray0, const void* depth0, int depth_type, double depth_scale,
+                           const double* rts, const double K[9], int level, const uint8_t* gray1,
+                           uint8_t* warped, uint8_t* diff, int32_t* num_landed, int64_t* sum_abs_diff);
 /* The batch entries keep what they allocate between calls: the packed level store, the slots' arena (up to half of the
- * free device memory for frames with large active levels), the pool's contexts, pinned result buffers.  This frees all
- * of it (blocks until the device is idle); the next batch call allocates again.  Debug flags and the record-stats
- * switch return to their defaults. */
+ * free device memory for frames with large active levels), the pool's contexts, pinned result buffers, the warpImage
+ * keys and staging buffers.  This frees all of it (blocks until the device is idle); the next batch call allocates
+ * again.  Debug flags and the record-stats switch return to their defaults. */
 int phovo_batch_release_memory(phovo_ctx* ctx);
 /* bytes the last phovo_batch_align call copied host -> device.  Host batches are uploaded without
  * the source rows no active pyramid level reads (the levels are point-decimated from the original

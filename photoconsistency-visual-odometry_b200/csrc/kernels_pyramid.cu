@@ -293,72 +293,132 @@ int launch_mean_ratio(cudaStream_t stream, const double* a, const double* b, siz
 }
 
 // ---------------------------------------------------------------------------------------------
-// phovo::warpImage, CPhotoconsistencyOdometry.h:73-134 (post-hoc visualisation of both apps)
+// phovo::warpImage, CPhotoconsistencyOdometry.h:73-134 (post-hoc visualisation of both apps), for a chunk of pairs:
+// blockIdx.y is the pair, so no block spans two pairs and every pair reads its own Rt
 // ---------------------------------------------------------------------------------------------
 namespace {
-struct WarpImgParams { double R[12]; double fx, fy, ox, oy, inv_fx, inv_fy; };
+// Each thread takes kWarpPix pixels kWarpThreads apart and issues all their loads before it uses any: one pixel per
+// thread leaves a single dependent memory access in flight per thread, and both kernels then wait on latency.
+constexpr int kWarpThreads = 256, kWarpPix = 8, kWarpTile = kWarpThreads * kWarpPix;
 
 template <typename DT>
-__global__ void __launch_bounds__(256) k_warp_splat(const uint8_t* __restrict__ gray, size_t gray_step, const DT* __restrict__ depth,
-                                                    size_t depth_step, double depth_scale, int rows, int cols,
-                                                    const __grid_constant__ WarpImgParams W, unsigned long long* __restrict__ keys) {
-  const size_t n = (size_t)rows * cols;
-  for (size_t i = (size_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (size_t)gridDim.x * 256) {
-    const int r = (int)(i / cols), c = (int)(i - (size_t)r * cols);
-    const DT* drow = (const DT*)((const char*)depth + (size_t)r * depth_step);
-    double d = (double)drow[c];
-    if (sizeof(DT) == 2) d = __dmul_rn(d, depth_scale);
-    if (!(d > 0.)) continue;                                                           // BASE:106
+__global__ void __launch_bounds__(kWarpThreads) k_warp_splat(const __grid_constant__ WarpImages W, const __grid_constant__ WarpIntrinsics I,
+                                                             uint32_t* __restrict__ keys) {
+  const int p = blockIdx.y;
+  const int n = W.rows * W.cols;                                                       // < 2^31: 32-bit index arithmetic
+  const int i0 = blockIdx.x * kWarpTile + threadIdx.x;
+  const char* dbase = (const char*)W.depth + p * W.depth_pair;
+  double dv[kWarpPix];
+#pragma unroll
+  for (int j = 0; j < kWarpPix; ++j) {
+    const int i = i0 + j * kWarpThreads;
+    dv[j] = 0.;
+    if (i < n) {
+      const int r = i / W.cols, c = i - r * W.cols;
+      dv[j] = (double)__ldg((const DT*)(dbase + (size_t)r * W.depth_step) + c);
+    }
+  }
+  const double* R = W.rts + (size_t)p * 16;
+  double M[12];
+#pragma unroll
+  for (int k = 0; k < 12; ++k) M[k] = __ldg(R + k);
+  uint32_t* pk = keys + (size_t)p * n;
+#pragma unroll
+  for (int j = 0; j < kWarpPix; ++j) {
+    const int i = i0 + j * kWarpThreads;
+    double d = dv[j];
+    if (sizeof(DT) == 2) d = __dmul_rn(d, W.depth_scale);
+    if (!(d > 0.)) continue;                                                           // BASE:106 (also i >= n: d = 0)
+    const int r = i / W.cols, c = i - r * W.cols;
     // BASE:109-112, fp64, the reference's operation order, no FMA contraction
-    const double px = __dmul_rn(__dmul_rn(__dsub_rn((double)c, W.ox), d), W.inv_fx);
-    const double py = __dmul_rn(__dmul_rn(__dsub_rn((double)r, W.oy), d), W.inv_fy);
+    const double px = __dmul_rn(__dmul_rn(__dsub_rn((double)c, I.ox), d), I.inv_fx);
+    const double py = __dmul_rn(__dmul_rn(__dsub_rn((double)r, I.oy), d), I.inv_fy);
     // Eigen 4x4 * 4x1 (BASE:115): sum over k = 0..3 in order, the homogeneous 1 multiplies the translation
-    const double X = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(W.R[0], px), __dmul_rn(W.R[1], py)), __dmul_rn(W.R[2], d)), W.R[3]);
-    const double Y = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(W.R[4], px), __dmul_rn(W.R[5], py)), __dmul_rn(W.R[6], d)), W.R[7]);
-    const double Z = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(W.R[8], px), __dmul_rn(W.R[9], py)), __dmul_rn(W.R[10], d)), W.R[11]);
-    const double tc = __dadd_rn(__ddiv_rn(__dmul_rn(X, W.fx), Z), W.ox);               // BASE:118-121: true division
-    const double tr = __dadd_rn(__ddiv_rn(__dmul_rn(Y, W.fy), Z), W.oy);
+    const double X = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(M[0], px), __dmul_rn(M[1], py)), __dmul_rn(M[2], d)), M[3]);
+    const double Y = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(M[4], px), __dmul_rn(M[5], py)), __dmul_rn(M[6], d)), M[7]);
+    const double Z = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(M[8], px), __dmul_rn(M[9], py)), __dmul_rn(M[10], d)), M[11]);
+    const double tc = __dadd_rn(__ddiv_rn(__dmul_rn(X, I.fx), Z), I.ox);               // BASE:118-121: true division
+    const double tr = __dadd_rn(__ddiv_rn(__dmul_rn(Y, I.fy), Z), I.oy);
     // static_cast<int>: truncation toward zero; NaN / out-of-range (undefined in the reference) -> skipped
-    if (!(tc > -1. && tc < (double)cols && tr > -1. && tr < (double)rows)) continue;
+    if (!(tc > -1. && tc < (double)W.cols && tr > -1. && tr < (double)W.rows)) continue;
     const int tj = (int)tc, ti = (int)tr;
-    const unsigned long long key = ((unsigned long long)(i + 1) << 8) | gray[(size_t)r * gray_step + c];
-    atomicMax(keys + (size_t)ti * cols + tj, key);                                     // raster-order last writer wins
+    // raster-order last writer wins: the largest source index; 0 = nothing landed
+    atomicMax(pk + ti * W.cols + tj, (uint32_t)(i + 1));
   }
 }
 
-__global__ void __launch_bounds__(256) k_warp_resolve(const unsigned long long* __restrict__ keys, int rows, int cols,
-                                                      uint8_t* __restrict__ warped, size_t warped_step,
-                                                      const uint8_t* __restrict__ target, size_t target_step,
-                                                      uint8_t* __restrict__ diff, size_t diff_step) {
-  const size_t n = (size_t)rows * cols;
-  for (size_t i = (size_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (size_t)gridDim.x * 256) {
-    const int r = (int)(i / cols), c = (int)(i - (size_t)r * cols);
-    const unsigned long long k = keys[i];
-    const int v = k ? (int)(k & 0xffull) : 0;                                          // BASE:98 zeros()
-    warped[(size_t)r * warped_step + c] = (uint8_t)v;
-    if (diff) { const int t = target[(size_t)r * target_step + c]; diff[(size_t)r * diff_step + c] = (uint8_t)(t > v ? t - v : v - t); }
+// CLEAR: leave the keys zero for the next chunk (instead of a memset before the splat)
+template <bool CLEAR>
+__global__ void __launch_bounds__(kWarpThreads) k_warp_resolve(const __grid_constant__ WarpImages W, uint32_t* __restrict__ keys) {
+  const int p = blockIdx.y;
+  const int n = W.rows * W.cols;
+  const int i0 = blockIdx.x * kWarpTile + threadIdx.x;
+  uint32_t* pk = keys + (size_t)p * n;
+  const uint8_t* gray = W.gray + p * W.gray_pair;
+  const uint8_t* target = W.target ? W.target + p * W.target_pair : nullptr;
+  uint32_t kv[kWarpPix];
+  int tv[kWarpPix];
+#pragma unroll
+  for (int j = 0; j < kWarpPix; ++j) {
+    const int i = i0 + j * kWarpThreads;
+    kv[j] = 0; tv[j] = 0;
+    if (i < n) {
+      kv[j] = pk[i];
+      if (target) { const int r = i / W.cols; tv[j] = __ldg(target + (size_t)r * W.target_step + (i - r * W.cols)); }
+    }
+  }
+  int gv[kWarpPix];
+#pragma unroll
+  for (int j = 0; j < kWarpPix; ++j) {                                                 // BASE:98 zeros()
+    gv[j] = 0;
+    if (kv[j]) {
+      const int s = (int)(kv[j] - 1), sr = s / W.cols;
+      gv[j] = __ldg(gray + (size_t)sr * W.gray_step + (s - sr * W.cols));
+    }
+  }
+  unsigned landed = 0, absdiff = 0;
+#pragma unroll
+  for (int j = 0; j < kWarpPix; ++j) {
+    const int i = i0 + j * kWarpThreads;
+    if (i >= n) continue;
+    if (CLEAR && kv[j]) pk[i] = 0;
+    const int r = i / W.cols, c = i - r * W.cols, v = gv[j];
+    if (W.warped) W.warped[p * W.warped_pair + (size_t)r * W.warped_step + c] = (uint8_t)v;
+    const unsigned a = (unsigned)(tv[j] > v ? tv[j] - v : v - tv[j]);
+    if (W.diff) W.diff[p * W.diff_pair + (size_t)r * W.diff_step + c] = (uint8_t)a;
+    if (kv[j]) { landed += 1; absdiff += a; }
+  }
+  if (!W.num_landed) return;
+  // block sums, then one integer atomic per block and quantity: the totals do not depend on the order
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    landed += __shfl_down_sync(0xffffffffu, landed, o);
+    absdiff += __shfl_down_sync(0xffffffffu, absdiff, o);
+  }
+  __shared__ unsigned s_landed[kWarpThreads / 32], s_abs[kWarpThreads / 32];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (lane == 0) { s_landed[warp] = landed; s_abs[warp] = absdiff; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned a = 0, b = 0;
+    for (int w = 0; w < kWarpThreads / 32; ++w) { a += s_landed[w]; b += s_abs[w]; }
+    if (a) atomicAdd((unsigned*)W.num_landed + p, a);
+    if (b && W.sum_abs_diff) atomicAdd((unsigned long long*)W.sum_abs_diff + p, (unsigned long long)b);
   }
 }
 }  // namespace
 
-int launch_warp_image(cudaStream_t stream, const uint8_t* gray, size_t gray_step, const void* depth, int depth_type,
-                      size_t depth_step, double depth_scale, int rows, int cols, const double rt[16],
-                      double fx, double fy, double ox, double oy, unsigned long long* keys,
-                      uint8_t* warped, size_t warped_step, const uint8_t* target, size_t target_step,
-                      uint8_t* diff, size_t diff_step) {
-  WarpImgParams W;
-  for (int k = 0; k < 12; ++k) W.R[k] = rt[k];
-  W.fx = fx; W.fy = fy; W.ox = ox; W.oy = oy;
-  W.inv_fx = 1.f / fx; W.inv_fy = 1.f / fy;          // BASE:91-92
-  const size_t n = (size_t)rows * cols;
-  cudaMemsetAsync(keys, 0, n * sizeof(unsigned long long), stream);
-  const int blocks = (int)((n + 255) / 256 < 148 * 8 ? (n + 255) / 256 : 148 * 8);
+int launch_warp_images(cudaStream_t stream, const WarpImages& W, int depth_type, const WarpIntrinsics& I, int num_pairs,
+                       uint32_t* keys, bool clear_keys) {
+  const int n = W.rows * W.cols;
+  const dim3 grid((unsigned)((n + kWarpTile - 1) / kWarpTile), (unsigned)num_pairs);
   switch (depth_type) {
-    case SRC_F32: k_warp_splat<float><<<blocks, 256, 0, stream>>>(gray, gray_step, (const float*)depth, depth_step, depth_scale, rows, cols, W, keys); break;
-    case SRC_U16: k_warp_splat<uint16_t><<<blocks, 256, 0, stream>>>(gray, gray_step, (const uint16_t*)depth, depth_step, depth_scale, rows, cols, W, keys); break;
-    default:      k_warp_splat<double><<<blocks, 256, 0, stream>>>(gray, gray_step, (const double*)depth, depth_step, depth_scale, rows, cols, W, keys); break;
+    case SRC_F32: k_warp_splat<float><<<grid, kWarpThreads, 0, stream>>>(W, I, keys); break;
+    case SRC_U16: k_warp_splat<uint16_t><<<grid, kWarpThreads, 0, stream>>>(W, I, keys); break;
+    default:      k_warp_splat<double><<<grid, kWarpThreads, 0, stream>>>(W, I, keys); break;
   }
-  k_warp_resolve<<<blocks, 256, 0, stream>>>(keys, rows, cols, warped, warped_step, target, target_step, diff, diff_step);
+  if (clear_keys) k_warp_resolve<true><<<grid, kWarpThreads, 0, stream>>>(W, keys);
+  else k_warp_resolve<false><<<grid, kWarpThreads, 0, stream>>>(W, keys);
   return 2;
 }
 

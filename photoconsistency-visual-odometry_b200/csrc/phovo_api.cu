@@ -403,7 +403,7 @@ extern "C" int phovo_destroy(phovo_ctx* ctx) {
   cudaFree(ctx->stage_gray[0]); cudaFree(ctx->stage_gray[1]); cudaFree(ctx->stage_depth);
   cudaFree(ctx->d_pose); cudaFree(ctx->d_log); cudaFree(ctx->d_state_in); cudaFree(ctx->d_shard); cudaFree(ctx->d_level_dmin); cudaFree(ctx->d_eval);
   cudaFree(ctx->dump_res); cudaFree(ctx->dump_jac);
-  cudaFree(ctx->warp_keys); for (int k = 0; k < 3; ++k) cudaFree(ctx->warp_io[k]);
+  for (int k = 0; k < 3; ++k) cudaFree(ctx->warp_io[k]);
   for (int r = 0; r < 8; ++r)
     if (ctx->xchg_opened[r]) cudaIpcCloseMemHandle(ctx->xchg_peer[r]);
   cudaFree(ctx->xchg_own); cudaFree(ctx->xchg_peers_dev);
@@ -952,9 +952,9 @@ extern "C" int phovo_warp_image(phovo_ctx* ctx, const uint8_t* gray, size_t gray
   if (gray_step < (size_t)cols || warped_step < (size_t)cols || depth_step < (size_t)cols * depth_elt(depth_type) ||
       (diff && (target_step < (size_t)cols || diff_step < (size_t)cols)))
     return ctx->fail(PHOVO_E_INVALID, "row stride smaller than a row");
-  CK(cudaSetDevice(ctx->device));
   const size_t n = (size_t)rows * cols;
-  CK(ensure(&ctx->warp_keys, &ctx->warp_keys_cap, n));
+  if (n > (size_t)INT32_MAX) return ctx->fail(PHOVO_E_UNSUPPORTED, "warpImage: frames of 2^31 pixels or more");
+  CK(cudaSetDevice(ctx->device));
   const void* dg; size_t dgs; const void* dd; size_t dds; int rc;
   if ((rc = stage_image(ctx, gray, gray_step, 1, rows, cols, &ctx->stage_gray[0], &ctx->stage_gray_cap[0], &dg, &dgs))) return rc;
   if ((rc = stage_image(ctx, depth, depth_step, depth_elt(depth_type), rows, cols, &ctx->stage_depth, &ctx->stage_depth_cap, &dd, &dds))) return rc;
@@ -966,12 +966,19 @@ extern "C" int phovo_warp_image(phovo_ctx* ctx, const uint8_t* gray, size_t gray
   const bool w_host = !is_device_pointer(warped), d_host = diff && !is_device_pointer(diff);
   if (w_host) { CK(ensure(&ctx->warp_io[0], &ctx->warp_io_cap[0], n)); dw = (uint8_t*)ctx->warp_io[0]; dws = cols; }
   if (d_host) { CK(ensure(&ctx->warp_io[2], &ctx->warp_io_cap[2], n)); ddf = (uint8_t*)ctx->warp_io[2]; ddfs = cols; }
+  WarpImages W;
+  memset(&W, 0, sizeof(W));
+  W.rows = rows; W.cols = cols;
+  W.gray = (const uint8_t*)dg; W.gray_step = dgs;
+  W.depth = dd; W.depth_step = dds; W.depth_scale = depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0;
+  W.target = (const uint8_t*)dt; W.target_step = dts;
+  W.warped = dw; W.warped_step = dws;
+  W.diff = ddf; W.diff_step = ddfs;
   const double p = pow(2, level);                                   // BASE:89-94: K / 2^level
-  ctx->launches += launch_warp_image(ctx->stream, (const uint8_t*)dg, dgs, dd, src_type_of_depth(depth_type), dds,
-                                     depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0, rows, cols, rt,
-                                     K[0] / p, K[4] / p, K[2] / p, K[5] / p, ctx->warp_keys, dw, dws,
-                                     (const uint8_t*)dt, dts, ddf, ddfs);
-  CK(cudaGetLastError());
+  WarpIntrinsics I;
+  I.fx = K[0] / p; I.fy = K[4] / p; I.ox = K[2] / p; I.oy = K[5] / p;
+  I.inv_fx = 1.f / I.fx; I.inv_fy = 1.f / I.fy;                    // BASE:91-92
+  if ((rc = phovo_internal_warp_images(ctx, W, src_type_of_depth(depth_type), I, 1, rt))) return rc;
   if (w_host) CK(cudaMemcpy2DAsync(warped, warped_step, dw, dws, cols, rows, cudaMemcpyDeviceToHost, ctx->stream));
   if (d_host) CK(cudaMemcpy2DAsync(diff, diff_step, ddf, ddfs, cols, rows, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));

@@ -65,6 +65,15 @@ struct phovo_batch_state {
   double* h_wave_states[2] = {nullptr, nullptr}; int32_t* h_wave_iters[2] = {nullptr, nullptr}; size_t wave_cap = 0;
   uint8_t* wave_g0[2] = {nullptr, nullptr}; uint8_t* wave_g1[2] = {nullptr, nullptr}; char* wave_d0[2] = {nullptr, nullptr}; char* wave_d1[2] = {nullptr, nullptr};
   size_t wave_g_cap[2] = {0, 0}, wave_g1_cap[2] = {0, 0}, wave_d0_cap[2] = {0, 0}, wave_d1_cap[2] = {0, 0};
+  // warpImage (phovo_batch_warp_image, phovo_warp_image): splat keys of one chunk of pairs (zero between calls while
+  // warp_keys_clean), Rt of the pairs, per-pair summaries, device copies of host inputs and outputs of one chunk
+  uint32_t* warp_keys = nullptr; size_t warp_keys_cap = 0; bool warp_keys_clean = false;
+  double* warp_rts = nullptr; size_t warp_rts_cap = 0;
+  int32_t* warp_landed = nullptr; size_t warp_landed_cap = 0;
+  int64_t* warp_sum = nullptr; size_t warp_sum_cap = 0;
+  uint8_t* warp_io[4] = {nullptr, nullptr, nullptr, nullptr}; size_t warp_io_cap[4] = {0, 0, 0, 0};   // gray0, gray1, warped, diff
+  char* warp_depth = nullptr; size_t warp_depth_cap = 0;
+  int l2_bytes = 0;
 };
 
 #define CK(call)                                                      \
@@ -111,6 +120,8 @@ void phovo_batch_release(phovo_ctx* ctx) {
   }
   cudaFree(b->d_slot_args);
   cudaFree(b->arena);
+  cudaFree(b->warp_keys); cudaFree(b->warp_rts); cudaFree(b->warp_landed); cudaFree(b->warp_sum); cudaFree(b->warp_depth);
+  for (int k = 0; k < 4; ++k) cudaFree(b->warp_io[k]);
   delete b;
   ctx->batch = nullptr;
 }
@@ -121,6 +132,7 @@ static int get_state(phovo_ctx* ctx, phovo_batch_state** out) {
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, ctx->device));
     ctx->batch->sm_count = prop.multiProcessorCount;
+    ctx->batch->l2_bytes = prop.l2CacheSize;
     CK(cudaStreamCreateWithFlags(&ctx->batch->copy_stream, cudaStreamNonBlocking));
     CK(cudaMalloc((void**)&ctx->batch->next_pair, sizeof(unsigned int) * PHOVO_MAX_LEVELS));
     for (int s = 0; s < 2; ++s) {
@@ -851,4 +863,131 @@ extern "C" int phovo_batch_align_with_target_depth(phovo_ctx* ctx, int num_pairs
   phovo_batch_state* b; int rc = get_state(ctx, &b);
   if (rc) return rc;
   return batch_other(ctx, b, num_pairs, rows, cols, gray0, depth0, depth_type, depth_scale, gray1, depth1, initial_states, states, iterations);
+}
+
+// ---------------------------------------------------------------------------------------------
+// phovo::warpImage (BASE:73-134) + the apps' cv::absdiff for many pairs (kernels_pyramid.cu: k_warp_splat, k_warp_resolve)
+// ---------------------------------------------------------------------------------------------
+// Pairs per chunk: the chunk's keys (4 B per pixel) fit in half of the L2, so that they are cleared, bid on and read back
+// there and HBM sees only the images (640x480 on a 126 MB L2: 51 pairs).
+static int warp_chunk_pairs(const phovo_batch_state* b, size_t n, int num_pairs) {
+  const size_t fit = (size_t)std::max(b->l2_bytes, 1) / 2 / (n * sizeof(uint32_t));
+  return (int)std::max<size_t>(1, std::min<size_t>({fit, (size_t)num_pairs, 65535}));
+}
+
+static WarpImages offset_pairs(WarpImages W, int p0) {
+  W.gray += p0 * W.gray_pair;
+  W.depth = (const char*)W.depth + p0 * W.depth_pair;
+  if (W.target) W.target += p0 * W.target_pair;
+  if (W.warped) W.warped += p0 * W.warped_pair;
+  if (W.diff) W.diff += p0 * W.diff_pair;
+  if (W.num_landed) W.num_landed += p0;
+  if (W.sum_abs_diff) W.sum_abs_diff += p0;
+  return W;
+}
+
+// Enqueues the warp of `num_pairs` pairs described by W (device pointers; W.rts is set here from `rts`, host or device
+// [num_pairs][16]) in chunks of warp_chunk_pairs.  Debug flag 16: the keys are cleared with a memset before each chunk
+// instead of by the resolve pass (same results; a measurement hook).
+int phovo_internal_warp_images(phovo_ctx* ctx, WarpImages W, int src_type, const WarpIntrinsics& I, int num_pairs, const double* rts) {
+  phovo_batch_state* b; int rc = get_state(ctx, &b);
+  if (rc) return rc;
+  const size_t n = (size_t)W.rows * W.cols;
+  const int chunk = warp_chunk_pairs(b, n, num_pairs);
+  if (b->warp_keys_cap < (size_t)chunk * n) {
+    CK(ensure(&b->warp_keys, &b->warp_keys_cap, (size_t)chunk * n));
+    b->warp_keys_clean = false;
+  }
+  const bool memset_each = (b->debug_flags & 16) != 0;
+  if (!b->warp_keys_clean && !memset_each) CK(cudaMemsetAsync(b->warp_keys, 0, b->warp_keys_cap * sizeof(uint32_t), ctx->stream));
+  b->warp_keys_clean = false;   // until every launch below has been enqueued
+  CK(ensure(&b->warp_rts, &b->warp_rts_cap, (size_t)num_pairs * 16));
+  CK(cudaMemcpyAsync(b->warp_rts, rts, sizeof(double) * 16 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
+  for (int p0 = 0; p0 < num_pairs; p0 += chunk) {
+    const int np = std::min(chunk, num_pairs - p0);
+    WarpImages C = offset_pairs(W, p0);
+    C.rts = b->warp_rts + (size_t)p0 * 16;
+    if (memset_each) CK(cudaMemsetAsync(b->warp_keys, 0, (size_t)np * n * sizeof(uint32_t), ctx->stream));
+    ctx->launches += launch_warp_images(ctx->stream, C, src_type, I, np, b->warp_keys, !memset_each) + (memset_each ? 1 : 0);
+    CK(cudaGetLastError());
+  }
+  b->warp_keys_clean = !memset_each;
+  return PHOVO_OK;
+}
+
+extern "C" int phovo_batch_warp_image(phovo_ctx* ctx, int num_pairs, int rows, int cols, const uint8_t* gray0, const void* depth0,
+                                      int depth_type, double depth_scale, const double* rts, const double K[9], int level,
+                                      const uint8_t* gray1, uint8_t* warped, uint8_t* diff, int32_t* num_landed, int64_t* sum_abs_diff) {
+  if (!ctx) return PHOVO_E_INVALID;
+  if (!gray0 || !depth0 || !rts || !K) return ctx->fail(PHOVO_E_INVALID, "gray0, depth0, rts and K are required");
+  if (num_pairs < 1 || rows < 1 || cols < 1 || level < 0 || level > 30) return ctx->fail(PHOVO_E_INVALID, "bad batch size, image size or level");
+  if (depth_type < 0 || depth_type > 2) return ctx->fail(PHOVO_E_INVALID, "unknown depth_type");
+  if ((diff || sum_abs_diff) && !gray1) return ctx->fail(PHOVO_E_INVALID, "diff and sum_abs_diff need gray1");
+  if (!warped && !diff && !num_landed && !sum_abs_diff) return ctx->fail(PHOVO_E_INVALID, "no output requested");
+  const size_t n = (size_t)rows * cols;
+  if (n > (size_t)INT32_MAX) return ctx->fail(PHOVO_E_UNSUPPORTED, "warpImage: frames of 2^31 pixels or more");
+  CK(cudaSetDevice(ctx->device));
+  phovo_batch_state* b; int rc = get_state(ctx, &b);
+  if (rc) return rc;
+  const size_t delt = depth_elt(depth_type);
+  const bool want_sum = sum_abs_diff != nullptr, want_summary = num_landed || sum_abs_diff;
+  const uint8_t* target = diff || want_sum ? gray1 : nullptr;
+  const bool in_dev = is_device_pointer(gray0) && is_device_pointer(depth0) && (!target || is_device_pointer(target));
+  const bool w_host = warped && !is_device_pointer(warped), d_host = diff && !is_device_pointer(diff);
+  if (want_summary) {
+    CK(ensure(&b->warp_landed, &b->warp_landed_cap, (size_t)num_pairs));
+    CK(ensure(&b->warp_sum, &b->warp_sum_cap, (size_t)num_pairs));
+    CK(cudaMemsetAsync(b->warp_landed, 0, sizeof(int32_t) * num_pairs, ctx->stream));
+    CK(cudaMemsetAsync(b->warp_sum, 0, sizeof(int64_t) * num_pairs, ctx->stream));
+  }
+  WarpImages W;
+  memset(&W, 0, sizeof(W));
+  W.rows = rows; W.cols = cols;
+  W.gray = gray0; W.gray_step = cols; W.gray_pair = n;
+  W.depth = depth0; W.depth_step = cols * delt; W.depth_pair = n * delt;
+  W.depth_scale = depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0;
+  W.target = target; W.target_step = cols; W.target_pair = n;
+  W.warped = warped; W.warped_step = cols; W.warped_pair = n;
+  W.diff = diff; W.diff_step = cols; W.diff_pair = n;
+  W.num_landed = want_summary ? b->warp_landed : nullptr;
+  W.sum_abs_diff = want_sum ? b->warp_sum : nullptr;
+  const double s = pow(2, level);                                  // BASE:89-94: K / 2^level
+  WarpIntrinsics I;
+  I.fx = K[0] / s; I.fy = K[4] / s; I.ox = K[2] / s; I.oy = K[5] / s;
+  I.inv_fx = 1.f / I.fx; I.inv_fy = 1.f / I.fy;                    // BASE:91-92
+  const int src = depth_type == PHOVO_DEPTH_F64 ? SRC_F64 : depth_type == PHOVO_DEPTH_F32 ? SRC_F32 : SRC_U16;
+  if (in_dev && !w_host && !d_host) {
+    if ((rc = phovo_internal_warp_images(ctx, W, src, I, num_pairs, rts))) return rc;
+  } else {
+    // host inputs (all rows: the warp reads every one) and host outputs go through device buffers of one chunk
+    const int chunk = warp_chunk_pairs(b, n, num_pairs);
+    const size_t cn = (size_t)chunk * n;
+    if (!in_dev) {
+      CK(ensure(&b->warp_io[0], &b->warp_io_cap[0], cn));
+      CK(ensure(&b->warp_depth, &b->warp_depth_cap, cn * delt));
+      if (target) CK(ensure(&b->warp_io[1], &b->warp_io_cap[1], cn));
+    }
+    if (w_host) CK(ensure(&b->warp_io[2], &b->warp_io_cap[2], cn));
+    if (d_host) CK(ensure(&b->warp_io[3], &b->warp_io_cap[3], cn));
+    for (int p0 = 0; p0 < num_pairs; p0 += chunk) {
+      const int np = std::min(chunk, num_pairs - p0);
+      WarpImages C = offset_pairs(W, p0);
+      if (!in_dev) {
+        CK(cudaMemcpyAsync(b->warp_io[0], C.gray, n * np, cudaMemcpyDefault, ctx->stream));
+        CK(cudaMemcpyAsync(b->warp_depth, C.depth, n * np * delt, cudaMemcpyDefault, ctx->stream));
+        if (target) CK(cudaMemcpyAsync(b->warp_io[1], C.target, n * np, cudaMemcpyDefault, ctx->stream));
+        C.gray = b->warp_io[0]; C.depth = b->warp_depth;
+        if (target) C.target = b->warp_io[1];
+      }
+      if (w_host) C.warped = b->warp_io[2];
+      if (d_host) C.diff = b->warp_io[3];
+      if ((rc = phovo_internal_warp_images(ctx, C, src, I, np, rts + (size_t)p0 * 16))) return rc;
+      if (w_host) CK(cudaMemcpyAsync(warped + (size_t)p0 * n, C.warped, n * np, cudaMemcpyDeviceToHost, ctx->stream));
+      if (d_host) CK(cudaMemcpyAsync(diff + (size_t)p0 * n, C.diff, n * np, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+  }
+  if (num_landed) CK(cudaMemcpyAsync(num_landed, b->warp_landed, sizeof(int32_t) * num_pairs, cudaMemcpyDefault, ctx->stream));
+  if (sum_abs_diff) CK(cudaMemcpyAsync(sum_abs_diff, b->warp_sum, sizeof(int64_t) * num_pairs, cudaMemcpyDefault, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return PHOVO_OK;
 }

@@ -51,8 +51,7 @@ struct phovo_ctx {
   char* stage_depth = nullptr; size_t stage_depth_cap = 0;
   double* dump_res = nullptr; size_t dump_res_cap = 0;
   double* dump_jac = nullptr; size_t dump_jac_cap = 0;
-  // phovo_warp_image scratch
-  unsigned long long* warp_keys = nullptr; size_t warp_keys_cap = 0;
+  // phovo_warp_image scratch (its keys belong to the batch state)
   char* warp_io[3] = {nullptr, nullptr, nullptr}; size_t warp_io_cap[3] = {0, 0, 0};   // device copies of warped / target / diff for host callers
 
   // solver state
@@ -110,6 +109,10 @@ struct phovo_ctx {
 };
 
 void phovo_batch_release(phovo_ctx* ctx);
+// phovo::warpImage of `num_pairs` pairs (device pointers in W; rts host or device [num_pairs][16]), enqueued on the
+// context stream with the batch state's keys; W.rts is ignored
+int phovo_internal_warp_images(phovo_ctx* ctx, phovo::WarpImages W, int src_type, const phovo::WarpIntrinsics& I,
+                               int num_pairs, const double* rts);
 // a slot context on `device` (see phovo_ctx::is_slot): set the stream and the arena before the first frame
 int phovo_internal_create_slot(int device, phovo_ctx** out);
 // device bytes a slot needs for rows x cols frames under its current config (upper bound, incl. alignment)

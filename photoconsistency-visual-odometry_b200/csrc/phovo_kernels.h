@@ -42,13 +42,25 @@ int launch_mean_ratio(cudaStream_t stream, const double* a, const double* b, siz
 int launch_scharr_store(cudaStream_t stream, const double* img, int rows, int cols, double scale,
                         double* Gx, double* Gy);
 
-// phovo::warpImage (BASE:73-134): splat keys (source index << 8 | intensity) with a 64-bit atomicMax,
-// then resolve to u8 (+ optional |target - warped|).  `keys` has rows*cols entries, zeroed here.
-int launch_warp_image(cudaStream_t stream, const uint8_t* gray, size_t gray_step, const void* depth, int depth_type,
-                      size_t depth_step, double depth_scale, int rows, int cols, const double rt[16],
-                      double fx, double fy, double ox, double oy, unsigned long long* keys,
-                      uint8_t* warped, size_t warped_step, const uint8_t* target, size_t target_step,
-                      uint8_t* diff, size_t diff_step);
+// phovo::warpImage (BASE:73-134) for a chunk of pairs of one size.  Device pointers of pair 0; `*_step` bytes between
+// rows, `*_pair` bytes between pairs.  warped / target / diff / num_landed / sum_abs_diff may be NULL (diff and
+// sum_abs_diff need target); num_landed / sum_abs_diff are added to, so they start at zero.
+struct WarpImages {
+  int rows, cols;                       // rows * cols < 2^31
+  const uint8_t* gray; size_t gray_step, gray_pair;
+  const void* depth; size_t depth_step, depth_pair; double depth_scale;   // depth_scale: u16 only
+  const double* rts;                    // [pairs][16] row-major 4x4
+  const uint8_t* target; size_t target_step, target_pair;
+  uint8_t* warped; size_t warped_step, warped_pair;
+  uint8_t* diff; size_t diff_step, diff_pair;
+  int32_t* num_landed; int64_t* sum_abs_diff;   // [pairs]
+};
+struct WarpIntrinsics { double fx, fy, ox, oy, inv_fx, inv_fy; };   // K / 2^level (BASE:89-94)
+// Splat: key = source linear index + 1, u32 atomicMax per target pixel (raster-order last writer wins).  Resolve:
+// gray[key - 1], |target - warped|, per-pair count of landed pixels and sum of their |target - warped|.  `keys`
+// [num_pairs][rows * cols] must be zero on entry; with `clear_keys` the resolve leaves them zero again.
+int launch_warp_images(cudaStream_t stream, const WarpImages& W, int depth_type /* SRC_* */, const WarpIntrinsics& I,
+                       int num_pairs, uint32_t* keys, bool clear_keys);
 
 // ---- alignment (kernels_align.cu) ------------------------------------------------------------
 struct LevelPtrs {

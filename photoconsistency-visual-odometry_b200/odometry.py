@@ -57,6 +57,7 @@ class CPhotoconsistencyOdometryCuda:
     def SetIntrinsicMatrix(self, intrinsicMatrix):                  # AN:460-463
         K = np.ascontiguousarray(intrinsicMatrix, dtype=np.float64).reshape(9)
         self._check(self._L.phovo_set_intrinsics(self._h, K.ctypes.data_as(capi._dp)))
+        self._K = K.reshape(3, 3).copy()
 
     def _follow_producer_stream(self, *images):
         """A CUDA tensor is produced on torch's current stream of its device: run the context on that
@@ -247,13 +248,7 @@ class CPhotoconsistencyOdometryCuda:
         """Host (numpy / pinned torch) or device (torch) arrays [P,R,C]; returns (states[P,6], iterations[P,MAXL]).
         `depth1` (target depth, same type as depth0) is read by the photometric + depth solver only."""
         P, R, Cc = tuple(gray0.shape)
-        if isinstance(depth0, np.ndarray):
-            dtype = {np.dtype(np.float64): capi.DEPTH_F64, np.dtype(np.float32): capi.DEPTH_F32,
-                     np.dtype(np.uint16): capi.DEPTH_U16}[depth0.dtype]
-        else:
-            import torch
-            dtype = {torch.float64: capi.DEPTH_F64, torch.float32: capi.DEPTH_F32, torch.uint16: capi.DEPTH_U16,
-                     torch.int16: capi.DEPTH_U16}[depth0.dtype]
+        dtype = self._batch_depth_type(depth0)
         states = np.zeros((P, 6))
         iters = np.zeros((P, capi.MAXL), dtype=np.int32)
         init = None if initial_states is None else np.ascontiguousarray(initial_states, dtype=np.float64)
@@ -280,7 +275,58 @@ class CPhotoconsistencyOdometryCuda:
                                                      None if initial_states is None else initial_states.data_ptr(),
                                                      states_out.data_ptr(), iters_out.data_ptr()))
 
-    def AlignSequence(self, gray, depth, depth_scale=1.0):
+    def BatchWarpImage(self, gray0, depth0, rts, K, level=0, gray1=None, images=True, depth_scale=1.0):
+        """WarpImage for P pairs in one call.  gray0 / gray1 u8 [P,R,C] and depth0 [P,R,C] (f64 / f32 metres or u16 raw *
+        depth_scale), numpy or torch, all on the host or all on the device; rts [P,4,4] (numpy or torch).  Returns a dict:
+        `warped` [P,R,C] u8 (None unless `images`), `diff` = |gray1 - warped| (None unless `images` and gray1 is given) --
+        torch tensors on the device for device inputs, numpy otherwise -- and, as numpy [P], `num_landed` (source pixels
+        that land in the target), `sum_abs_diff` (sum of |gray1 - warped| over them; None without gray1) and
+        `mean_abs_diff` = sum_abs_diff / max(num_landed, 1)."""
+        def dense(a):
+            return None if a is None else np.ascontiguousarray(a) if isinstance(a, np.ndarray) else a.contiguous()
+        gray0, depth0, gray1 = dense(gray0), dense(depth0), dense(gray1)
+        P, R, Cc = tuple(gray0.shape)
+        dtype = self._batch_depth_type(depth0)
+        if tuple(depth0.shape) != (P, R, Cc) or (gray1 is not None and tuple(gray1.shape) != (P, R, Cc)):
+            raise ValueError("gray0, depth0 and gray1 must all be [P, rows, cols]")
+        on_device = not isinstance(gray0, np.ndarray) and gray0.is_cuda
+        if on_device:
+            self._follow_producer_stream(gray0)
+        if getattr(rts, "is_cuda", False):
+            import torch
+            rts = rts.to(torch.float64).contiguous()
+        else:
+            rts = np.ascontiguousarray(np.asarray(rts), dtype=np.float64)
+        if tuple(rts.shape) not in ((P, 4, 4), (P, 16)):
+            raise ValueError("rts must be [P, 4, 4]")
+        Kc = np.ascontiguousarray(K, dtype=np.float64).reshape(9)
+
+        def image():
+            if on_device:
+                import torch
+                return torch.empty((P, R, Cc), dtype=torch.uint8, device=gray0.device)
+            return np.empty((P, R, Cc), np.uint8)
+        warped = image() if images else None
+        diff = image() if images and gray1 is not None else None
+        landed = np.zeros(P, np.int32)
+        sums = np.zeros(P, np.int64) if gray1 is not None else None
+        self._check(self._L.phovo_batch_warp_image(self._h, P, R, Cc, capi._ptr(gray0), capi._ptr(depth0), dtype, float(depth_scale),
+                                                   capi._ptr(rts), Kc.ctypes.data_as(capi._dp), int(level), capi._ptr(gray1),
+                                                   capi._ptr(warped), capi._ptr(diff), landed.ctypes.data,
+                                                   None if sums is None else sums.ctypes.data))
+        return dict(warped=warped, diff=diff, num_landed=landed, sum_abs_diff=sums,
+                    mean_abs_diff=None if sums is None else sums / np.maximum(landed, 1))
+
+    @staticmethod
+    def _batch_depth_type(depth0):
+        if isinstance(depth0, np.ndarray):
+            return {np.dtype(np.float64): capi.DEPTH_F64, np.dtype(np.float32): capi.DEPTH_F32,
+                    np.dtype(np.uint16): capi.DEPTH_U16}[depth0.dtype]
+        import torch
+        return {torch.float64: capi.DEPTH_F64, torch.float32: capi.DEPTH_F32, torch.uint16: capi.DEPTH_U16,
+                torch.int16: capi.DEPTH_U16}[depth0.dtype]
+
+    def AlignSequence(self, gray, depth, depth_scale=1.0, diagnostics=False):
         """PhotoconsistencyVisualOdometry.cpp:212-259 for a whole recorded sequence in ONE batch call.
 
         The app aligns frame k-1 (source) to frame k (target) from a ZERO initial state every frame
@@ -288,7 +334,10 @@ class CPhotoconsistencyOdometryCuda:
         uploaded once and pair k reads frames k and k+1 of the same device arrays.  `gray` [N,R,C] u8 and
         `depth` [N,R,C] (f64 / f32 metres or u16 raw * depth_scale), numpy or torch (host or device).
         Returns (states [N-1,6], iterations [N-1,MAXL], poses [N,4,4]) with poses[0] = I and
-        poses[k] = poses[k-1] @ inv(Rt_k) as the app accumulates them (:234)."""
+        poses[k] = poses[k-1] @ inv(Rt_k) as the app accumulates them (:234).
+        With `diagnostics` a 4th element: BatchWarpImage's summary (num_landed, sum_abs_diff, mean_abs_diff [N-1]) of frame
+        k-1 warped onto frame k with Rt_k at full resolution -- the |target - warped| image the app shows (:247-252),
+        reduced to one number per frame."""
         import torch
         dev = torch.device("cuda", torch.cuda.current_device())
         g = gray if isinstance(gray, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(gray))
@@ -304,10 +353,16 @@ class CPhotoconsistencyOdometryCuda:
         self.SetStream(torch.cuda.current_stream(dev).cuda_stream)
         self.BatchAlignDevice(g[:-1], d[:-1], g[1:], states, iters, depth_scale=depth_scale)   # overlapping views, no copies
         st, it = states.cpu().numpy(), iters.cpu().numpy()
+        rts = np.stack([capi.state_to_rt(s) for s in st])
         poses = np.tile(np.eye(4), (n, 1, 1))
         for k in range(1, n):
-            poses[k] = poses[k - 1] @ np.linalg.inv(capi.state_to_rt(st[k - 1]))
-        return st, it, poses
+            poses[k] = poses[k - 1] @ np.linalg.inv(rts[k - 1])
+        if not diagnostics:
+            return st, it, poses
+        if getattr(self, "_K", None) is None:
+            raise ValueError("diagnostics need SetIntrinsicMatrix")
+        s = self.BatchWarpImage(g[:-1], d[:-1], rts, self._K, gray1=g[1:], images=False, depth_scale=depth_scale)
+        return st, it, poses, {k: s[k] for k in ("num_landed", "sum_abs_diff", "mean_abs_diff")}
 
     def BatchKernelTimes(self):
         """(pyramid_ms, align_ms) of the last BatchAlignDevice call, CUDA events on the context stream."""

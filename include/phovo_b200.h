@@ -277,10 +277,35 @@ int phovo_batch_warp_image(phovo_ctx* ctx, int num_pairs, int rows, int cols,
                            const uint8_t* gray0, const void* depth0, int depth_type, double depth_scale,
                            const double* rts, const double K[9], int level, const uint8_t* gray1,
                            uint8_t* warped, uint8_t* diff, int32_t* num_landed, int64_t* sum_abs_diff);
+/* Normal equations of P pairs at given states, at any pyramid level in [0, num_levels) whether or not it has iterations
+ * configured (the call builds that level itself).  For pair p it returns what phovo_eval_normal_equations(ctx, level,
+ * states[p]) returns on a context with the same configuration and intrinsics after phovo_set_source(gray0[p],
+ * depth0[p]) and phovo_set_target(gray1[p]): H [P][21] (the packed upper triangle of J^T J, in the order of
+ * phovo_iter_stats.H), g [P][6] = J^T r, cost [P] = 0.5 sum r^2 (over every target pixel some source pixel landed
+ * on), num_valid [P].  Agreement is to rounding (the sums are grouped differently); num_valid is exact.
+ * What J is: the photometric Jacobian of the analytic solver, with the image gradients multiplied by the configured
+ * imageGradientsScalingFactor of the level; in PHOVO_MODE_ANALYTIC_REF it also carries the reference's `temp11`
+ * term (AN:253), in PHOVO_MODE_ANALYTIC_FIXED it is the exact derivative.  So H is the reference's J^T J as its
+ * Gauss-Newton step uses it, not a calibrated information matrix: scale it by a noise model of your own before
+ * using it as one, and mind that in mode 0 its translation-rotation coupling is the reference's.
+ * gray0 / depth0 / gray1 are dense [P][rows][cols], all on the host (pageable or pinned) or all on the device;
+ * states [P][6] (x y z yaw pitch roll) on the host or the device; each output may be NULL, host or device, at least
+ * one must be given.  Blocking; device inputs are read on the context stream (see phovo_set_source).
+ * Results are bitwise reproducible and independent of which pairs share a call.
+ * PHOVO_E_UNSUPPORTED: Ceres mode and the photometric + depth solver, blurFilterSize[level] > 1, level 1 of a frame
+ * whose size is 3 mod 4, frames of 2^31 pixels or more.  PHOVO_E_INVALID: no intrinsics, P < 1, bad sizes or level,
+ * unknown depth type, no output.  Pairs run in chunks whose winner keys, validity flags and level records (5 B per
+ * level pixel, + 20 B above level 0) fit in half of the L2. */
+int phovo_batch_eval_normal_equations(phovo_ctx* ctx, int num_pairs, int rows, int cols,
+                                      const uint8_t* gray0, const void* depth0, int depth_type, double depth_scale,
+                                      const uint8_t* gray1, const double* states /* [P][6] */, int level,
+                                      double* H /* [P][21] */, double* g /* [P][6] */, double* cost /* [P] */,
+                                      int32_t* num_valid /* [P] */);
 /* The batch entries keep what they allocate between calls: the packed level store, the slots' arena (up to half of the
  * free device memory for frames with large active levels), the pool's contexts, pinned result buffers, the warpImage
- * keys and staging buffers.  This frees all of it (blocks until the device is idle); the next batch call allocates
- * again.  Debug flags and the record-stats switch return to their defaults. */
+ * keys and staging buffers, the keys, level records, partial sums and results of phovo_batch_eval_normal_equations.
+ * This frees all of it (blocks until the device is idle); the next batch call allocates again.  Debug flags and the
+ * record-stats switch return to their defaults. */
 int phovo_batch_release_memory(phovo_ctx* ctx);
 /* bytes the last phovo_batch_align call copied host -> device.  Host batches are uploaded without
  * the source rows no active pyramid level reads (the levels are point-decimated from the original

@@ -10,7 +10,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libphovo_b200.so")
-SOURCES = ["phovo_api.cu", "phovo_batch.cu", "kernels_pyramid.cu", "kernels_align.cu", "kernels_batch.cu", "yaml_config.cpp"]
+SOURCES = ["phovo_api.cu", "phovo_batch.cu", "kernels_pyramid.cu", "kernels_align.cu", "kernels_batch.cu", "kernels_eval.cu",
+           "yaml_config.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC,-Wall,-Wno-unused-function", "-Xptxas", "-v"]
 

@@ -103,6 +103,8 @@ SIGNATURES = {
     "phovo_batch_set_debug_flags": (C.c_int, [_vp, C.c_int]),
     "phovo_batch_warp_image": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, _dp, C.c_int, _vp,
                                          _vp, _vp, _vp, _vp]),
+    "phovo_batch_eval_normal_equations": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, _vp,
+                                                    C.c_int, _vp, _vp, _vp, _vp]),
     "phovo_batch_release_memory": (C.c_int, [_vp]),
     "phovo_batch_get_last_h2d_bytes": (C.c_int, [_vp, C.POINTER(C.c_uint64)]),
     "phovo_synchronize": (C.c_int, [_vp]),

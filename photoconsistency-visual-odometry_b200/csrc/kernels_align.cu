@@ -146,26 +146,8 @@ __global__ void __launch_bounds__(kBlock) k_normal_eq(LevelParams L, LevelPtrs P
       }
       if (DUMP && dump_res) dump_res[i] = res;
       if (!P.valid[i]) continue;                      // K3a decided (exact reference arithmetic)
-      // From here on nothing decides an integer: FMA contraction and a 1-ulp reciprocal are fine.
-      const double px = ((double)c - L.ox) * d * L.inv_fx, py = ((double)r - L.oy) * d * L.inv_fy;
-      const double q0 = fma(T.R00, px, fma(T.R01, py, T.R02 * d));
-      const double q1 = fma(T.R10, px, fma(T.R11, py, T.R12 * d));
-      const double q2 = fma(T.R20, px, fma(T.R21, py, T.R22 * d));
-      const double iz = rcp_1ulp(q2 + T.z);
-      // a = Gx1[i] fx / Z', b = Gy1[i] fy / Z'  (gradients at the SOURCE index, AN:346-347); closed form
-      // of AN:243-342 (SURVEY appendix C) with the gradient folded in
-      const double ga = __ldg(P.Gx + i) * L.fx * iz, gb = __ldg(P.Gy + i) * L.fy * iz;
-      const double A = MODE == 0 ? fma(px, T.x, q0) : q0 + T.x;   // AN:253 bug-compatible / Maxima-exact
-      const double B = q1 + T.y;
       double J[6];
-      J[0] = ga;
-      J[1] = gb;
-      J[2] = -(fma(ga, A, gb * B) * iz);
-      J[3] = fma(gb, q0, -(ga * q1));
-      const double Zp = -fma(spsr, py, fma(spcr, d, T.cp * px));
-      J[4] = fma(q2, fma(ga, T.cy, gb * T.sy), Zp * J[2]);
-      const double Zr = fma(T.R22, py, -(T.R21 * d));
-      J[5] = fma(ga, fma(T.R02, py, -(T.R01 * d)), fma(gb, fma(T.R12, py, -(T.R11 * d)), Zr * J[2]));
+      analytic_jacobian<MODE>(L, T, spsr, spcr, r, c, d, __ldg(P.Gx + i), __ldg(P.Gy + i), J);
       accumulate_row(acc, J, res);
       acc[28] += 1.;
       if (DUMP && dump_jac) for (int k = 0; k < 6; ++k) dump_jac[(size_t)i * 6 + k] = J[k];

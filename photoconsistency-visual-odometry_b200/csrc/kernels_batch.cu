@@ -35,11 +35,6 @@ __device__ __forceinline__ void linear_axis(int d, double scale, int ssize, bool
   s0 = s; w1 = f;
 }
 
-template <typename DT> __device__ __forceinline__ double depth_at(const DT* p, double scale);
-template <> __device__ __forceinline__ double depth_at<double>(const double* p, double) { return __ldg(p); }
-template <> __device__ __forceinline__ double depth_at<float>(const float* p, double) { return (double)__ldg(p); }
-template <> __device__ __forceinline__ double depth_at<uint16_t>(const uint16_t* p, double scale) { return __dmul_rn((double)__ldg(p), scale); }
-
 // K1b.  grid = (ceil(pixels of all active levels / 256), pairs).  One thread per level pixel:
 // 4 taps from each of gray0, gray1 and depth0 (the central 2x2 of the pixel's 2^level cell).
 // Consecutive threads read consecutive cells of the same two source rows, so a warp touches one

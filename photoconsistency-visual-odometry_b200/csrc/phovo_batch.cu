@@ -74,6 +74,17 @@ struct phovo_batch_state {
   uint8_t* warp_io[4] = {nullptr, nullptr, nullptr, nullptr}; size_t warp_io_cap[4] = {0, 0, 0, 0};   // gray0, gray1, warped, diff
   char* warp_depth = nullptr; size_t warp_depth_cap = 0;
   int l2_bytes = 0;
+  // normal equations at given states (phovo_batch_eval_normal_equations): winner keys (zero between calls while
+  // eval_keys_clean) and validity of one chunk, its level records and tile partials; states, poses and results of
+  // every pair.  Host inputs are staged through warp_io[0] / warp_io[1] / warp_depth.
+  uint32_t* eval_keys = nullptr; size_t eval_keys_cap = 0; bool eval_keys_clean = false;
+  uint8_t* eval_valid = nullptr; size_t eval_valid_cap = 0;
+  uint8_t* eval_store = nullptr; size_t eval_store_cap = 0;
+  double* eval_partials = nullptr; size_t eval_partials_cap = 0;
+  double* eval_states = nullptr; size_t eval_states_cap = 0;
+  PoseDev* eval_poses = nullptr; size_t eval_poses_cap = 0;
+  double* eval_out = nullptr; size_t eval_out_cap = 0;        // [P][21] H, [P][6] g, [P] cost
+  int32_t* eval_nvalid = nullptr; size_t eval_nvalid_cap = 0;
 };
 
 #define CK(call)                                                      \
@@ -122,6 +133,8 @@ void phovo_batch_release(phovo_ctx* ctx) {
   cudaFree(b->arena);
   cudaFree(b->warp_keys); cudaFree(b->warp_rts); cudaFree(b->warp_landed); cudaFree(b->warp_sum); cudaFree(b->warp_depth);
   for (int k = 0; k < 4; ++k) cudaFree(b->warp_io[k]);
+  cudaFree(b->eval_keys); cudaFree(b->eval_valid); cudaFree(b->eval_store); cudaFree(b->eval_partials);
+  cudaFree(b->eval_states); cudaFree(b->eval_poses); cudaFree(b->eval_out); cudaFree(b->eval_nvalid);
   delete b;
   ctx->batch = nullptr;
 }
@@ -150,6 +163,35 @@ static void level_size(int rows, int cols, int level, int* orows, int* ocols) {
   *ocols = level == 0 ? cols : (int)lrint(cols * f);
 }
 
+// Active level `a` of bp = pyramid level `level` of a rows x cols frame under the context's config: size, record
+// offsets (appended at *off), intrinsics, step and gradient scale.  Fails on what the pyramid kernel cannot build.
+static int fill_level(phovo_ctx* ctx, int rows, int cols, int level, int a, BatchParams* bp, unsigned long long* off) {
+  if (ctx->cfg.blur_filter_size[level] > 1) return ctx->fail(PHOVO_E_UNSUPPORTED, "batch kernel: blurFilterSize > 0 is only supported by the per-pair API");
+  // cv::resize by 1/2 averages cells cut by the image border in single precision (sizes = 3 mod 4):
+  // not representable in the exact integer tap sums the batch records keep
+  if (level == 1 && (rows % 4 == 3 || cols % 4 == 3))
+    return ctx->fail(PHOVO_E_UNSUPPORTED, "batch kernel: level 1 of an image whose size is 3 mod 4 is only supported by the per-pair API");
+  int lr, lc;
+  level_size(rows, cols, level, &lr, &lc);
+  if (lr < 1 || lc < 1) return ctx->fail(PHOVO_E_INVALID, "image too small for the number of pyramid levels");
+  const int n = lr * lc;
+  bp->level[a] = level; bp->lrows[a] = lr; bp->lcols[a] = lc;
+  bp->px_offset[a + 1] = bp->px_offset[a] + n;
+  const unsigned long long n16 = ((unsigned long long)n * 2 + 15) & ~15ull, n64 = ((unsigned long long)n * 8 + 15) & ~15ull;
+  bp->off_D0[a] = *off; *off += n64;
+  bp->off_I0[a] = *off; *off += n16;
+  bp->off_I1[a] = *off; *off += n16;
+  bp->off_D32[a] = *off; *off += ((unsigned long long)n * 4 + 15) & ~15ull;
+  // CPhotoconsistencyOdometryAnalytic.h:203-209
+  const double scaleFactor = 1.0 / pow(2, level);
+  bp->fx[a] = ctx->K[0] * scaleFactor; bp->fy[a] = ctx->K[4] * scaleFactor;
+  bp->ox[a] = ctx->K[2] * scaleFactor; bp->oy[a] = ctx->K[5] * scaleFactor;
+  bp->inv_fx[a] = 1.f / bp->fx[a]; bp->inv_fy[a] = 1.f / bp->fy[a];
+  bp->lambda[a] = ctx->cfg.lambda_step[level]; bp->min_grad[a] = ctx->cfg.min_gradient_norm[level];
+  bp->grad_k[a] = ctx->cfg.grad_scale[level] / 1020.0;
+  return PHOVO_OK;
+}
+
 // Parameter block for a rows x cols batch under the context's config; fails loudly when a
 // configuration cannot run in the shared-memory-resident kernel (there is no slower fallback
 // inside this entry point: the caller is told to use the per-pair API).
@@ -168,32 +210,12 @@ static int make_params(phovo_ctx* ctx, int num_pairs, int rows, int cols, int lo
   unsigned long long off = 0;
   for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
     if (ctx->cfg.max_num_iterations[level] <= 0) continue;
-    if (ctx->cfg.blur_filter_size[level] > 1) return ctx->fail(PHOVO_E_UNSUPPORTED, "batch kernel: blurFilterSize > 0 is only supported by the per-pair API");
-    // cv::resize by 1/2 averages cells cut by the image border in single precision (sizes = 3 mod 4):
-    // not representable in the exact integer tap sums the batch records keep
-    if (level == 1 && (rows % 4 == 3 || cols % 4 == 3))
-      return ctx->fail(PHOVO_E_UNSUPPORTED, "batch kernel: level 1 of an image whose size is 3 mod 4 is only supported by the per-pair API");
-    int lr, lc;
-    level_size(rows, cols, level, &lr, &lc);
-    if (lr < 1 || lc < 1) return ctx->fail(PHOVO_E_INVALID, "image too small for the number of pyramid levels");
-    const int n = lr * lc;
+    const int rc = fill_level(ctx, rows, cols, level, a, bp, &off);
+    if (rc) return rc;
+    const int n = bp->lrows[a] * bp->lcols[a];
     if (n > kBatchMaxLevelPixels) return ctx->fail(PHOVO_E_UNSUPPORTED, "batch kernel: an active level exceeds the shared-memory budget (about 20K px); use the per-pair API");
     nmax = std::max(nmax, n);
-    bp->level[a] = level; bp->lrows[a] = lr; bp->lcols[a] = lc;
     bp->max_iters[a] = ctx->cfg.max_num_iterations[level];
-    bp->px_offset[a + 1] = bp->px_offset[a] + n;
-    const unsigned long long n16 = ((unsigned long long)n * 2 + 15) & ~15ull, n64 = ((unsigned long long)n * 8 + 15) & ~15ull;
-    bp->off_D0[a] = off; off += n64;
-    bp->off_I0[a] = off; off += n16;
-    bp->off_I1[a] = off; off += n16;
-    bp->off_D32[a] = off; off += ((unsigned long long)n * 4 + 15) & ~15ull;
-    // CPhotoconsistencyOdometryAnalytic.h:203-209
-    const double scaleFactor = 1.0 / pow(2, level);
-    bp->fx[a] = ctx->K[0] * scaleFactor; bp->fy[a] = ctx->K[4] * scaleFactor;
-    bp->ox[a] = ctx->K[2] * scaleFactor; bp->oy[a] = ctx->K[5] * scaleFactor;
-    bp->inv_fx[a] = 1.f / bp->fx[a]; bp->inv_fy[a] = 1.f / bp->fy[a];
-    bp->lambda[a] = ctx->cfg.lambda_step[level]; bp->min_grad[a] = ctx->cfg.min_gradient_norm[level];
-    bp->grad_k[a] = ctx->cfg.grad_scale[level] / 1020.0;
     ++a;
   }
   bp->num_active = a;
@@ -988,6 +1010,112 @@ extern "C" int phovo_batch_warp_image(phovo_ctx* ctx, int num_pairs, int rows, i
   }
   if (num_landed) CK(cudaMemcpyAsync(num_landed, b->warp_landed, sizeof(int32_t) * num_pairs, cudaMemcpyDefault, ctx->stream));
   if (sum_abs_diff) CK(cudaMemcpyAsync(sum_abs_diff, b->warp_sum, sizeof(int64_t) * num_pairs, cudaMemcpyDefault, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return PHOVO_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Normal equations of many pairs at given states (kernels_eval.cu): what phovo_eval_normal_equations gives pair by pair
+// ---------------------------------------------------------------------------------------------
+// Pairs per chunk: the chunk's winner keys (4 B per pixel), validity flags (1 B) and, above level 0, its level records
+// fit in half of the L2, so that the two passes find them there (640x480 level 0 on a 126 MB L2: 41 pairs).
+static int eval_chunk_pairs(const phovo_batch_state* b, size_t n, unsigned long long record_bytes, int num_pairs) {
+  const size_t fit = (size_t)std::max(b->l2_bytes, 1) / 2 / (n * (sizeof(uint32_t) + 1) + record_bytes);
+  return (int)std::max<size_t>(1, std::min<size_t>({fit, (size_t)num_pairs, 65535}));
+}
+
+extern "C" int phovo_batch_eval_normal_equations(phovo_ctx* ctx, int num_pairs, int rows, int cols, const uint8_t* gray0,
+                                                 const void* depth0, int depth_type, double depth_scale, const uint8_t* gray1,
+                                                 const double* states, int level, double* H, double* g, double* cost,
+                                                 int32_t* num_valid) {
+  if (!ctx) return PHOVO_E_INVALID;
+  if (!gray0 || !depth0 || !gray1 || !states) return ctx->fail(PHOVO_E_INVALID, "gray0, depth0, gray1 and states are required");
+  if (!ctx->have_K) return ctx->fail(PHOVO_E_INVALID, "SetIntrinsicMatrix has not been called");
+  if (ctx->cfg.mode == PHOVO_MODE_CERES || ctx->cfg.mode == PHOVO_MODE_BIOBJECTIVE)
+    return ctx->fail(PHOVO_E_UNSUPPORTED, "batched normal equations: analytic modes only");
+  if (num_pairs < 1 || rows < 1 || cols < 1 || level < 0 || level >= ctx->cfg.num_levels)
+    return ctx->fail(PHOVO_E_INVALID, "bad batch size, image size or level");
+  if (depth_type < 0 || depth_type > 2) return ctx->fail(PHOVO_E_INVALID, "unknown depth_type");
+  if (!H && !g && !cost && !num_valid) return ctx->fail(PHOVO_E_INVALID, "no output requested");
+  const size_t n = (size_t)rows * cols;
+  if (n > (size_t)INT32_MAX) return ctx->fail(PHOVO_E_UNSUPPORTED, "batched normal equations: frames of 2^31 pixels or more");
+  BatchParams bp;
+  memset(&bp, 0, sizeof(bp));
+  bp.rows = rows; bp.cols = cols; bp.num_active = 1; bp.mode = ctx->cfg.mode;
+  bp.min_depth = ctx->cfg.min_depth; bp.max_depth = ctx->cfg.max_depth;
+  unsigned long long record_bytes = 0;
+  int rc = fill_level(ctx, rows, cols, level, 0, &bp, &record_bytes);
+  if (rc) return rc;
+  bp.record_bytes = record_bytes;
+  const bool records = level > 0;                   // level 0 is read straight from the caller's frames
+  CK(cudaSetDevice(ctx->device));
+  phovo_batch_state* b;
+  if ((rc = get_state(ctx, &b))) return rc;
+  const int ln = bp.lrows[0] * bp.lcols[0];
+  EvalLevel E;
+  memset(&E, 0, sizeof(E));
+  E.L.fx = bp.fx[0]; E.L.fy = bp.fy[0]; E.L.ox = bp.ox[0]; E.L.oy = bp.oy[0]; E.L.inv_fx = bp.inv_fx[0]; E.L.inv_fy = bp.inv_fy[0];
+  E.L.min_depth = bp.min_depth; E.L.max_depth = bp.max_depth;
+  E.L.lambda = bp.lambda[0]; E.L.min_grad_norm = bp.min_grad[0];
+  E.L.rows = bp.lrows[0]; E.L.cols = bp.lcols[0];
+  E.L.mode = bp.mode; E.L.level = level; E.L.row_begin = 0; E.L.row_end = E.L.rows;
+  E.grad_k = bp.grad_k[0];
+  E.tiles = (ln + kEvalTile - 1) / kEvalTile;
+  E.depth_scale = depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0;
+  E.record_bytes = record_bytes; E.off_I0 = bp.off_I0[0]; E.off_I1 = bp.off_I1[0]; E.off_D0 = bp.off_D0[0];
+  const int src = depth_type == PHOVO_DEPTH_F64 ? SRC_F64 : depth_type == PHOVO_DEPTH_F32 ? SRC_F32 : SRC_U16;
+  const size_t delt = depth_elt(depth_type);
+  const int chunk = eval_chunk_pairs(b, (size_t)ln, records ? record_bytes : 0, num_pairs);
+  const size_t ck = (size_t)chunk * ln;
+  if (b->eval_keys_cap < ck) {
+    CK(ensure(&b->eval_keys, &b->eval_keys_cap, ck));
+    b->eval_keys_clean = false;
+  }
+  CK(ensure(&b->eval_valid, &b->eval_valid_cap, ck));
+  CK(ensure(&b->eval_partials, &b->eval_partials_cap, (size_t)chunk * E.tiles * PHOVO_ACC_STRIDE));
+  if (records) CK(ensure(&b->eval_store, &b->eval_store_cap, (size_t)chunk * record_bytes));
+  CK(ensure(&b->eval_states, &b->eval_states_cap, (size_t)num_pairs * 6));
+  CK(ensure(&b->eval_poses, &b->eval_poses_cap, (size_t)num_pairs));
+  CK(ensure(&b->eval_out, &b->eval_out_cap, (size_t)num_pairs * 28));
+  CK(ensure(&b->eval_nvalid, &b->eval_nvalid_cap, (size_t)num_pairs));
+  const bool in_dev = is_device_pointer(gray0) && is_device_pointer(depth0) && is_device_pointer(gray1);
+  if (!in_dev) {   // host frames go through device buffers of one chunk (every row: level 0 and the pyramid read them all)
+    CK(ensure(&b->warp_io[0], &b->warp_io_cap[0], (size_t)chunk * n));
+    CK(ensure(&b->warp_io[1], &b->warp_io_cap[1], (size_t)chunk * n));
+    CK(ensure(&b->warp_depth, &b->warp_depth_cap, (size_t)chunk * n * delt));
+  }
+  if (!b->eval_keys_clean) CK(cudaMemsetAsync(b->eval_keys, 0, b->eval_keys_cap * sizeof(uint32_t), ctx->stream));
+  b->eval_keys_clean = false;   // until every launch below has been enqueued
+  CK(cudaMemcpyAsync(b->eval_states, states, sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
+  ctx->launches += launch_eval_poses(ctx->stream, b->eval_states, num_pairs, b->eval_poses);
+  double* dH = b->eval_out; double* dg = dH + (size_t)num_pairs * 21; double* dcost = dg + (size_t)num_pairs * 6;
+  E.keys = b->eval_keys; E.valid = b->eval_valid; E.partials = b->eval_partials; E.store = b->eval_store;
+  for (int p0 = 0; p0 < num_pairs; p0 += chunk) {
+    const int np = std::min(chunk, num_pairs - p0);
+    const uint8_t* c_g0 = gray0 + (size_t)p0 * n; const uint8_t* c_g1 = gray1 + (size_t)p0 * n;
+    const void* c_d = (const char*)depth0 + (size_t)p0 * n * delt;
+    if (!in_dev) {
+      CK(cudaMemcpyAsync(b->warp_io[0], c_g0, n * np, cudaMemcpyDefault, ctx->stream));
+      CK(cudaMemcpyAsync(b->warp_io[1], c_g1, n * np, cudaMemcpyDefault, ctx->stream));
+      CK(cudaMemcpyAsync(b->warp_depth, c_d, n * np * delt, cudaMemcpyDefault, ctx->stream));
+      c_g0 = b->warp_io[0]; c_g1 = b->warp_io[1]; c_d = b->warp_depth;
+    }
+    if (records) {
+      bp.num_pairs = np;
+      ctx->launches += launch_batch_pyramid(ctx->stream, bp, c_g0, c_d, src, E.depth_scale, c_g1, b->eval_store);
+    } else {
+      E.gray0 = c_g0; E.gray1 = c_g1; E.depth = c_d;
+    }
+    E.poses = b->eval_poses + p0;
+    ctx->launches += launch_eval_normal_equations(ctx->stream, E, src, records, np, dH + (size_t)p0 * 21, dg + (size_t)p0 * 6,
+                                                  dcost + p0, b->eval_nvalid + p0);
+    CK(cudaGetLastError());
+  }
+  b->eval_keys_clean = true;
+  if (H) CK(cudaMemcpyAsync(H, dH, sizeof(double) * 21 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
+  if (g) CK(cudaMemcpyAsync(g, dg, sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
+  if (cost) CK(cudaMemcpyAsync(cost, dcost, sizeof(double) * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
+  if (num_valid) CK(cudaMemcpyAsync(num_valid, b->eval_nvalid, sizeof(int32_t) * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return PHOVO_OK;
 }

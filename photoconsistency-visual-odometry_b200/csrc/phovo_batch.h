@@ -53,6 +53,27 @@ int launch_batch_align(cudaStream_t stream, const BatchParams& bp, int sm_count,
                        const double* init_states, double* states, int32_t* iters, phovo_iter_stats* log,
                        int32_t* log_counts, unsigned int* next_pair);
 size_t batch_level_smem_bytes(int rows, int cols);
+
+// Normal equations at given states for a chunk of pairs at one pyramid level (kernels_eval.cu).  Level 0 reads the
+// caller's dense frames; a level >= 1 reads the records k_batch_pyramid wrote for a BatchParams with that one level.
+constexpr int kEvalThreads = 256, kEvalPix = 8, kEvalTile = kEvalThreads * kEvalPix;   // pixels per tile: fixed
+struct EvalLevel {
+  LevelParams L;                         // K / 2^level, depth range, rows / cols of the level (rows * cols < 2^31)
+  double grad_k;                         // imageGradientsScalingFactor / 1020 (gradients from integer tap sums)
+  int tiles;                             // ceil(rows * cols / kEvalTile)
+  const uint8_t* gray0; const uint8_t* gray1; const void* depth; double depth_scale;   // level 0: [pairs][n] of pair 0
+  const uint8_t* store; unsigned long long record_bytes, off_I0, off_I1, off_D0;       // level >= 1: records of pair 0
+  const PoseDev* poses;                  // [pairs]
+  uint32_t* keys;                        // [pairs][n]: source index + 1 of the winner, 0 = none; zero on entry and exit
+  uint8_t* valid;                        // [pairs][n]: the exact warp accepted the source pixel
+  double* partials;                      // [pairs][tiles][PHOVO_ACC_STRIDE]
+};
+// Pose (rotation and trig values) of every state, as the per-pair path derives it: poses[p] from states[p * 6].
+int launch_eval_poses(cudaStream_t stream, const double* states, int num_pairs, PoseDev* poses);
+// Winner pass, accumulate pass (clears the keys) and the per-pair sums into H [21], g [6], cost, num_valid of pairs
+// [0, num_pairs) of E; `out_*` point at the chunk's first pair.  Returns the number of launches.
+int launch_eval_normal_equations(cudaStream_t stream, const EvalLevel& E, int src_type /* SRC_*; level 0 */, bool records,
+                                 int num_pairs, double* out_H, double* out_g, double* out_cost, int32_t* out_valid);
 bool batch_level_is_small(int rows, int cols);
 cudaError_t batch_align_prepare();
 

@@ -317,6 +317,43 @@ class CPhotoconsistencyOdometryCuda:
         return dict(warped=warped, diff=diff, num_landed=landed, sum_abs_diff=sums,
                     mean_abs_diff=None if sums is None else sums / np.maximum(landed, 1))
 
+    def BatchEvalNormalEquations(self, gray0, depth0, gray1, states, level=0, depth_scale=1.0):
+        """The normal equations of P pairs at the given states, at any pyramid level (built by the call, configured
+        iterations or not): what EvalNormalEquations(level, states[p]) returns after SetSourceFrame(gray0[p], depth0[p])
+        and SetTargetFrame(gray1[p]), to rounding.  gray0 / gray1 u8 [P,R,C] and depth0 [P,R,C] (f64 / f32 metres or
+        u16 raw * depth_scale), numpy or torch, all on the host or all on the device; states [P,6] (numpy or torch).
+        Returns a dict of numpy arrays: `H` [P,6,6] = J^T J (symmetric), `g` [P,6] = J^T r, `cost` [P] = 0.5 |r|^2 and
+        `num_valid` [P].  J scales the image gradients by the configured imageGradientsScalingFactor and, in mode 0,
+        carries the reference's temp11 term (AN:253): H is the solver's J^T J, not a calibrated information matrix."""
+        def dense(a):
+            return np.ascontiguousarray(a) if isinstance(a, np.ndarray) else a.contiguous()
+        gray0, depth0, gray1 = dense(gray0), dense(depth0), dense(gray1)
+        P, R, Cc = tuple(gray0.shape)
+        dtype = self._batch_depth_type(depth0)
+        if tuple(depth0.shape) != (P, R, Cc) or tuple(gray1.shape) != (P, R, Cc):
+            raise ValueError("gray0, depth0 and gray1 must all be [P, rows, cols]")
+        if not isinstance(gray0, np.ndarray) and gray0.is_cuda:
+            self._follow_producer_stream(gray0)
+        if getattr(states, "is_cuda", False):
+            import torch
+            states = states.to(torch.float64).contiguous()
+        else:
+            states = np.ascontiguousarray(np.asarray(states), dtype=np.float64)
+        if tuple(states.shape) != (P, 6):
+            raise ValueError("states must be [P, 6]")
+        Hu = np.zeros((P, 21))
+        g = np.zeros((P, 6))
+        cost = np.zeros(P)
+        nv = np.zeros(P, np.int32)
+        self._check(self._L.phovo_batch_eval_normal_equations(self._h, P, R, Cc, capi._ptr(gray0), capi._ptr(depth0), dtype,
+                                                              float(depth_scale), capi._ptr(gray1), capi._ptr(states), int(level),
+                                                              Hu.ctypes.data, g.ctypes.data, cost.ctypes.data, nv.ctypes.data))
+        iu = np.triu_indices(6)
+        H = np.zeros((P, 6, 6))
+        H[:, iu[0], iu[1]] = Hu
+        H[:, iu[1], iu[0]] = Hu
+        return dict(H=H, g=g, cost=cost, num_valid=nv)
+
     @staticmethod
     def _batch_depth_type(depth0):
         if isinstance(depth0, np.ndarray):
@@ -326,7 +363,7 @@ class CPhotoconsistencyOdometryCuda:
         return {torch.float64: capi.DEPTH_F64, torch.float32: capi.DEPTH_F32, torch.uint16: capi.DEPTH_U16,
                 torch.int16: capi.DEPTH_U16}[depth0.dtype]
 
-    def AlignSequence(self, gray, depth, depth_scale=1.0, diagnostics=False):
+    def AlignSequence(self, gray, depth, depth_scale=1.0, diagnostics=False, information_level=None):
         """PhotoconsistencyVisualOdometry.cpp:212-259 for a whole recorded sequence in ONE batch call.
 
         The app aligns frame k-1 (source) to frame k (target) from a ZERO initial state every frame
@@ -337,7 +374,10 @@ class CPhotoconsistencyOdometryCuda:
         poses[k] = poses[k-1] @ inv(Rt_k) as the app accumulates them (:234).
         With `diagnostics` a 4th element: BatchWarpImage's summary (num_landed, sum_abs_diff, mean_abs_diff [N-1]) of frame
         k-1 warped onto frame k with Rt_k at full resolution -- the |target - warped| image the app shows (:247-252),
-        reduced to one number per frame."""
+        reduced to one number per frame.
+        With `information_level` (a pyramid level) the 4th element is returned whether or not `diagnostics` is set and
+        also carries BatchEvalNormalEquations' H [N-1,6,6], g, cost and num_valid of every pair at its solved state on
+        that level: the solver's J^T J of each edge, for a pose graph or filter (scale it by a noise model)."""
         import torch
         dev = torch.device("cuda", torch.cuda.current_device())
         g = gray if isinstance(gray, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(gray))
@@ -357,12 +397,18 @@ class CPhotoconsistencyOdometryCuda:
         poses = np.tile(np.eye(4), (n, 1, 1))
         for k in range(1, n):
             poses[k] = poses[k - 1] @ np.linalg.inv(rts[k - 1])
-        if not diagnostics:
+        if not diagnostics and information_level is None:
             return st, it, poses
-        if getattr(self, "_K", None) is None:
-            raise ValueError("diagnostics need SetIntrinsicMatrix")
-        s = self.BatchWarpImage(g[:-1], d[:-1], rts, self._K, gray1=g[1:], images=False, depth_scale=depth_scale)
-        return st, it, poses, {k: s[k] for k in ("num_landed", "sum_abs_diff", "mean_abs_diff")}
+        diag = {}
+        if diagnostics:
+            if getattr(self, "_K", None) is None:
+                raise ValueError("diagnostics need SetIntrinsicMatrix")
+            s = self.BatchWarpImage(g[:-1], d[:-1], rts, self._K, gray1=g[1:], images=False, depth_scale=depth_scale)
+            diag.update({k: s[k] for k in ("num_landed", "sum_abs_diff", "mean_abs_diff")})
+        if information_level is not None:
+            diag.update(self.BatchEvalNormalEquations(g[:-1], d[:-1], g[1:], states, level=int(information_level),
+                                                      depth_scale=depth_scale))
+        return st, it, poses, diag
 
     def BatchKernelTimes(self):
         """(pyramid_ms, align_ms) of the last BatchAlignDevice call, CUDA events on the context stream."""

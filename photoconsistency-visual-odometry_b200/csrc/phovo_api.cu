@@ -25,38 +25,12 @@ int phovo_ctx::cuda_fail(const char* what, cudaError_t e) {
   return PHOVO_E_CUDA;
 }
 
-static void level_size(int rows, int cols, int level, int* orows, int* ocols) {
-  // cv::resize(img, Size(0,0), f, f): dsize = cvRound(ssize * f), f = 2^-level (AN:132,159)
-  if (level == 0) { *orows = rows; *ocols = cols; return; }
-  const double f = ldexp(1.0, -level);
-  *orows = (int)lrint(rows * f);
-  *ocols = (int)lrint(cols * f);
-}
-
 bool phovo_ctx::level_active(int l) const {
   return l < cfg.num_levels && (build_all_levels || cfg.max_num_iterations[l] > 0);
 }
 
 LevelParams phovo_ctx::level_params(int level) const {
-  LevelParams L;
-  memset(&L, 0, sizeof(L));
-  if (cfg.mode == PHOVO_MODE_CERES) {
-    // CPhotoconsistencyOdometryCeres.h:163-168
-    const double p = pow(2, (double)level);
-    L.fx = K[0] / p; L.fy = K[4] / p; L.ox = K[2] / p; L.oy = K[5] / p;
-    L.inv_fx = 1. / L.fx; L.inv_fy = 1. / L.fy;
-  } else {
-    // CPhotoconsistencyOdometryAnalytic.h:203-209
-    const double scaleFactor = 1.0 / pow(2, level);
-    L.fx = K[0] * scaleFactor; L.fy = K[4] * scaleFactor; L.ox = K[2] * scaleFactor; L.oy = K[5] * scaleFactor;
-    L.inv_fx = 1.f / L.fx; L.inv_fy = 1.f / L.fy;
-  }
-  L.min_depth = cfg.min_depth; L.max_depth = cfg.max_depth;
-  L.lambda = cfg.lambda_step[level]; L.min_grad_norm = cfg.min_gradient_norm[level];
-  L.rows = lrows[level]; L.cols = lcols[level];
-  L.max_iters = cfg.max_num_iterations[level];
-  L.mode = cfg.mode; L.level = level;
-  L.row_begin = 0; L.row_end = L.rows;
+  LevelParams L = make_level_params(cfg, K, level, lrows[level], lcols[level]);
   if (shard_world > 1) {
     L.row_begin = (int)((long long)L.rows * shard_rank / shard_world);
     L.row_end = (int)((long long)L.rows * (shard_rank + 1) / shard_world);
@@ -66,59 +40,41 @@ LevelParams phovo_ctx::level_params(int level) const {
 
 LevelPtrs phovo_ctx::level_ptrs(int level) const {
   LevelPtrs P;
-  P.I0 = I0[level]; P.D0 = D0[level]; P.I1 = I1[level]; P.Gx = Gx[level]; P.Gy = Gy[level];
-  P.winner = winner;
-  P.valid = valid;
-  P.D1 = D1[level]; P.GxD = GxD[level]; P.GyD = GyD[level]; P.gain = d_gain ? d_gain + level : nullptr;
+  P.I0 = I0[level].get(); P.D0 = D0[level].get(); P.I1 = I1[level].get(); P.Gx = Gx[level].get(); P.Gy = Gy[level].get();
+  P.winner = winner.get();
+  P.valid = valid.get();
+  P.D1 = D1[level].get(); P.GxD = GxD[level].get(); P.GyD = GyD[level].get(); P.gain = d_gain.get() ? d_gain.get() + level : nullptr;
   return P;
 }
 
-#define CK(call)                                                      \
-  do {                                                                \
-    cudaError_t e_ = (call);                                          \
-    if (e_ != cudaSuccess) return ctx->cuda_fail((std::string(__func__) + ": " #call).c_str(), e_); \
-  } while (0)
-
+// slots take views of their arena (bump pointer; arena_reset starts over), everything else allocates; *fresh as in
+// Array::ensure
 template <class T>
-static cudaError_t ensure(T** p, size_t* cap, size_t want) {
-  if (*cap >= want && *p) return cudaSuccess;
-  if (*p) cudaFree(*p);
-  *p = nullptr; *cap = 0;
-  cudaError_t e = cudaMalloc((void**)p, want * sizeof(T));
-  if (e == cudaSuccess) *cap = want;
-  return e;
-}
-
-// slots allocate from their arena (bump pointer; arena_reset starts over), everything else with cudaMalloc
-template <class T>
-static cudaError_t ctx_ensure(phovo_ctx* ctx, T** p, size_t* cap, size_t want) {
-  if (!ctx->arena_base) return ensure(p, cap, want);
-  if (*cap >= want && *p) return cudaSuccess;
+static cudaError_t ctx_ensure(phovo_ctx* ctx, DeviceArray<T>& a, size_t want, bool* fresh = nullptr) {
+  if (!ctx->arena_base) return a.ensure(want, fresh);
+  if (fresh) *fresh = false;
+  if (a.capacity() >= want && a.get()) return cudaSuccess;
   const size_t off = (ctx->arena_used + 255) & ~(size_t)255, bytes = want * sizeof(T);
   if (off + bytes > ctx->arena_bytes) return cudaErrorMemoryAllocation;
-  *p = (T*)(ctx->arena_base + off);
-  *cap = want;
+  a.view((T*)(ctx->arena_base + off), want);
+  if (fresh) *fresh = true;
   ctx->arena_used = off + bytes;
   return cudaSuccess;
 }
 
 void phovo_ctx::arena_reset(char* base, size_t bytes) {
   for (int l = 0; l < PHOVO_MAX_LEVELS; ++l) {
-    I0[l] = D0[l] = I1[l] = Gx[l] = Gy[l] = nullptr;
-    D1[l] = GxD[l] = GyD[l] = nullptr;
-    for (int a = 0; a < 5; ++a) lcap[l][a] = 0;
-    for (int a = 0; a < 3; ++a) bcap[l][a] = 0;
+    I0[l].reset(); D0[l].reset(); I1[l].reset(); Gx[l].reset(); Gy[l].reset();
+    D1[l].reset(); GxD[l].reset(); GyD[l].reset();
   }
-  winner = nullptr; winner_cap = 0; valid = nullptr; valid_cap = 0;
-  scratch64[0] = scratch64[1] = nullptr; scratch_cap[0] = scratch_cap[1] = 0;
-  partials = nullptr; partials_cap = 0;
-  d_gain = nullptr; d_pose = nullptr;
+  winner.reset(); valid.reset(); scratch64[0].reset(); scratch64[1].reset(); partials.reset();
+  d_gain.reset(); d_pose.reset();
   have_src = have_tgt = have_tgt_depth = false;
   rows = cols = 0;
   arena_base = base; arena_bytes = bytes; arena_used = 0;
   if (base) {
-    d_pose = (PoseDev*)base;
-    d_gain = (double*)(base + 256);
+    d_pose.view((PoseDev*)base, 1);
+    d_gain.view((double*)(base + 256), PHOVO_MAX_LEVELS);
     arena_used = 512;
     static_assert(sizeof(PoseDev) <= 256 && sizeof(double) * PHOVO_MAX_LEVELS <= 256, "slot header layout");
   }
@@ -141,12 +97,6 @@ size_t phovo_internal_slot_bytes(const phovo_ctx* ctx, int rows, int cols) {
   return (total + 4095) & ~(size_t)4095;
 }
 
-static bool is_device_pointer(const void* p) {
-  cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-  return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
-}
-
 void phovo_ctx::invalidate_graph() {
   if (graph_exec) { cudaGraphExecDestroy(graph_exec); graph_exec = nullptr; }
   if (graph) { cudaGraphDestroy(graph); graph = nullptr; }
@@ -165,47 +115,36 @@ static int prepare_levels(phovo_ctx* ctx, int rows, int cols) {
     if (!ctx->level_active(l)) continue;
     const size_t n = (size_t)ctx->lrows[l] * ctx->lcols[l];
     if (n > max_px) max_px = n;
-    double** arrs[5] = {&ctx->I0[l], &ctx->D0[l], &ctx->I1[l], &ctx->Gx[l], &ctx->Gy[l]};
+    DeviceArray<double>* arrs[5] = {&ctx->I0[l], &ctx->D0[l], &ctx->I1[l], &ctx->Gx[l], &ctx->Gy[l]};
     for (int a = 0; a < 5; ++a) {
-      size_t cap = ctx->lcap[l][a];
-      double* before = *arrs[a];
-      CK(ctx_ensure(ctx, arrs[a], &cap, n));
-      ctx->lcap[l][a] = cap;
-      if (before != *arrs[a]) changed = true;
+      bool fresh;
+      CK(ctx_ensure(ctx, *arrs[a], n, &fresh));
+      changed |= fresh;
     }
   }
   if (max_px == 0) max_px = 1;
-  {
-    // (re)allocated <=> refill with -1.  NOT "the pointer changed": cudaFree + cudaMalloc may hand the same address back
-    // with a larger extent, whose tail is garbage -- winner indices nobody wrote (found by the randomised sweep on a
-    // pool of 8 contexts: illegal addresses in phase B after a frame-size change)
-    const bool reallocated = !(ctx->winner && ctx->winner_cap >= 2 * max_px);
-    int* before = ctx->winner;
-    CK(ctx_ensure(ctx, &ctx->winner, &ctx->winner_cap, 2 * max_px));   // the photometric + depth solver stacks 2N rows
-    if (reallocated || before != ctx->winner) {
-      changed = true;
-      launch_fill_i32(ctx->stream, ctx->winner, -1, ctx->winner_cap, ctx->sm_count);
-      ctx->launches += 1;
-    }
+  // new storage <=> refill with -1.  NOT "the pointer changed": cudaFree + cudaMalloc may hand the same address back
+  // with a larger extent, whose tail is garbage -- winner indices nobody wrote (found by the randomised sweep on a
+  // pool of 8 contexts: illegal addresses in phase B after a frame-size change)
+  bool fresh;
+  CK(ctx_ensure(ctx, ctx->winner, 2 * max_px, &fresh));   // the photometric + depth solver stacks 2N rows
+  if (fresh) {
+    changed = true;
+    launch_fill_i32(ctx->stream, ctx->winner.get(), -1, ctx->winner.capacity(), ctx->sm_count);
+    ctx->launches += 1;
   }
-  {
-    unsigned char* before = ctx->valid;
-    CK(ctx_ensure(ctx, &ctx->valid, &ctx->valid_cap, max_px));
-    if (before != ctx->valid) changed = true;
-  }
-  for (int s = 0; s < 2; ++s) CK(ctx_ensure(ctx, &ctx->scratch64[s], &ctx->scratch_cap[s], max_px));
-  {
-    double* before = ctx->partials;
-    CK(ctx_ensure(ctx, &ctx->partials, &ctx->partials_cap, (size_t)partials_blocks(ctx->sm_count) * PHOVO_ACC_STRIDE));
-    if (before != ctx->partials) changed = true;
-  }
+  CK(ctx_ensure(ctx, ctx->valid, max_px, &fresh));
+  changed |= fresh;
+  for (int s = 0; s < 2; ++s) CK(ctx_ensure(ctx, ctx->scratch64[s], max_px));
+  CK(ctx_ensure(ctx, ctx->partials, (size_t)partials_blocks(ctx->sm_count) * PHOVO_ACC_STRIDE, &fresh));
+  changed |= fresh;
   if (changed) ctx->invalidate_graph();
   return PHOVO_OK;
 }
 
 // copy a strided host/device image into a dense device staging buffer (or use it in place)
 static int stage_image(phovo_ctx* ctx, const void* src, size_t step, size_t elt, int rows, int cols,
-                       char** stage, size_t* stage_cap, const void** dev_out, size_t* dev_step) {
+                       DeviceArray<char>& stage, const void** dev_out, size_t* dev_step) {
   if (is_device_pointer(src)) {
     // used in place; the kernels that read it are drained before the call returns (wait_uploads), so the
     // caller may overwrite or free the buffer afterwards, exactly as with a host buffer.  Ordering
@@ -216,9 +155,9 @@ static int stage_image(phovo_ctx* ctx, const void* src, size_t step, size_t elt,
     return PHOVO_OK;
   }
   const size_t bytes = (size_t)rows * cols * elt;
-  CK(ensure(stage, stage_cap, bytes));
-  CK(cudaMemcpy2DAsync(*stage, (size_t)cols * elt, src, step, (size_t)cols * elt, rows, cudaMemcpyHostToDevice, ctx->stream));
-  *dev_out = *stage; *dev_step = (size_t)cols * elt;
+  CK(stage.ensure(bytes));
+  CK(cudaMemcpy2DAsync(stage.get(), (size_t)cols * elt, src, step, (size_t)cols * elt, rows, cudaMemcpyHostToDevice, ctx->stream));
+  *dev_out = stage.get(); *dev_step = (size_t)cols * elt;
   ctx->h2d_pending = true;
   return PHOVO_OK;
 }
@@ -226,7 +165,7 @@ static int stage_image(phovo_ctx* ctx, const void* src, size_t step, size_t elt,
 static int finish_uploads(phovo_ctx* ctx) {
   // inputs are borrowed for the duration of the call only: wait for the copies (not the kernels)
   if (ctx->h2d_pending) {
-    CK(cudaEventRecord(ctx->ev_copy, ctx->stream));
+    CK(cudaEventRecord(ctx->ev_copy.get(), ctx->stream));
     ctx->h2d_pending = false;
     ctx->copy_event_armed = true;
   }
@@ -240,19 +179,9 @@ static int wait_uploads(phovo_ctx* ctx) {
     if (!ctx->defer_device_input_drain) CK(cudaStreamSynchronize(ctx->stream));
     return PHOVO_OK;
   }
-  if (ctx->copy_event_armed) { CK(cudaEventSynchronize(ctx->ev_copy)); ctx->copy_event_armed = false; }
+  if (ctx->copy_event_armed) { CK(cudaEventSynchronize(ctx->ev_copy.get())); ctx->copy_event_armed = false; }
   return PHOVO_OK;
 }
-
-static int src_type_of_depth(int depth_type) {
-  switch (depth_type) {
-    case PHOVO_DEPTH_F64: return SRC_F64;
-    case PHOVO_DEPTH_F32: return SRC_F32;
-    case PHOVO_DEPTH_U16: return SRC_U16;
-  }
-  return -1;
-}
-static size_t depth_elt(int depth_type) { return depth_type == PHOVO_DEPTH_F64 ? 8 : depth_type == PHOVO_DEPTH_F32 ? 4 : 2; }
 
 // the active levels of the current size as a PyramidLevels block; false if one of them is blurred
 // (the fused kernel has no blur stage) or if the frame is big: one launch for all levels wins while
@@ -278,8 +207,8 @@ static int build_intensity(phovo_ctx* ctx, const void* dev_gray, size_t step, bo
   if (fused_levels(ctx, &P)) {
     for (int a = 0; a < P.num; ++a) {
       const int l = P.level[a];
-      P.dst[a] = target ? ctx->I1[l] : ctx->I0[l];
-      P.gx[a] = target ? ctx->Gx[l] : nullptr; P.gy[a] = target ? ctx->Gy[l] : nullptr;
+      P.dst[a] = target ? ctx->I1[l].get() : ctx->I0[l].get();
+      P.gx[a] = target ? ctx->Gx[l].get() : nullptr; P.gy[a] = target ? ctx->Gy[l].get() : nullptr;
     }
     ctx->launches += launch_build_levels(ctx->stream, dev_gray, SRC_U8, step, 1. / 255, ctx->rows, ctx->cols, P, target);
     CK(cudaGetLastError());
@@ -288,14 +217,14 @@ static int build_intensity(phovo_ctx* ctx, const void* dev_gray, size_t step, bo
   for (int l = 0; l < ctx->cfg.num_levels; ++l) {
     if (!ctx->level_active(l)) continue;
     const int r = ctx->lrows[l], c = ctx->lcols[l];
-    double* img = target ? ctx->I1[l] : ctx->I0[l];
+    double* img = target ? ctx->I1[l].get() : ctx->I0[l].get();
     ctx->launches += launch_build_level(ctx->stream, dev_gray, SRC_U8, step, 1. / 255, ctx->rows, ctx->cols, l, img, r, c);
     const int k = ctx->cfg.blur_filter_size[l];
     if (k > 1) {  // AN:144-148: GaussianBlur(k, sigma 3) twice
-      ctx->launches += launch_gaussian_blur(ctx->stream, img, ctx->scratch64[0], r, c, k, 3.);
-      ctx->launches += launch_gaussian_blur(ctx->stream, img, ctx->scratch64[0], r, c, k, 3.);
+      ctx->launches += launch_gaussian_blur(ctx->stream, img, ctx->scratch64[0].get(), r, c, k, 3.);
+      ctx->launches += launch_gaussian_blur(ctx->stream, img, ctx->scratch64[0].get(), r, c, k, 3.);
     }
-    if (target) ctx->launches += launch_scharr_store(ctx->stream, img, r, c, ctx->cfg.grad_scale[l], ctx->Gx[l], ctx->Gy[l]);
+    if (target) ctx->launches += launch_scharr_store(ctx->stream, img, r, c, ctx->cfg.grad_scale[l], ctx->Gx[l].get(), ctx->Gy[l].get());
   }
   CK(cudaGetLastError());
   return PHOVO_OK;
@@ -309,7 +238,7 @@ static int build_depth(phovo_ctx* ctx, const void* dev_depth, int depth_type, si
     const int a = P.num++;
     P.level[a] = l; P.orows[a] = ctx->lrows[l]; P.ocols[a] = ctx->lcols[l];
     P.px_offset[a + 1] = P.px_offset[a] + ctx->lrows[l] * ctx->lcols[l];
-    P.dst[a] = ctx->D0[l];
+    P.dst[a] = ctx->D0[l].get();
   }
   if (P.px_offset[P.num] <= (1 << 20)) {   // small frame: every active level in one launch (see fused_levels)
     ctx->launches += launch_build_levels(ctx->stream, dev_depth, src_type_of_depth(depth_type), step, depth_scale, ctx->rows, ctx->cols, P, false);
@@ -344,7 +273,7 @@ static int create_context(int device, phovo_ctx** out, bool slot) {
   if (device < 0 || device >= ndev) { g_create_error = "device index out of range"; return PHOVO_E_INVALID; }
   e = cudaSetDevice(device);
   if (e != cudaSuccess) { g_create_error = std::string("cudaSetDevice: ") + cudaGetErrorString(e); return PHOVO_E_CUDA; }
-  phovo_ctx* ctx = new phovo_ctx();
+  phovo_ctx* ctx = new phovo_ctx();   // on failure, `delete ctx` frees whatever was made so far
   ctx->device = device;
   {
     cudaDeviceProp prop;
@@ -361,25 +290,24 @@ static int create_context(int device, phovo_ctx** out, bool slot) {
   };
   ctx->is_slot = slot;
   if (!slot) {
-    if ((e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
-    ctx->own_stream = true;
+    if ((e = create_stream(ctx->own_stream)) != cudaSuccess) return bail("cudaStreamCreate", e);
+    ctx->stream = ctx->own_stream.get();
   }
-  if ((e = cudaEventCreate(&ctx->ev_copy)) != cudaSuccess) return bail("cudaEventCreate", e);
+  if ((e = create_event(ctx->ev_copy)) != cudaSuccess) return bail("cudaEventCreate", e);
   for (int i = 0; i < 4; ++i)
-    if ((e = cudaEventCreate(&ctx->ev_time[i])) != cudaSuccess) return bail("cudaEventCreate", e);
+    if ((e = create_event(ctx->ev_time[i])) != cudaSuccess) return bail("cudaEventCreate", e);
   if (slot) { *out = ctx; return PHOVO_OK; }   // device buffers come from the arena, results are gathered by the batch state
-  ctx->log_cap = 1024;
-  if ((e = cudaMalloc((void**)&ctx->d_pose, sizeof(PoseDev))) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMemset(ctx->d_pose, 0, sizeof(PoseDev))) != cudaSuccess) return bail("cudaMemset", e);
-  if ((e = cudaMalloc((void**)&ctx->d_log, sizeof(phovo_iter_stats) * ctx->log_cap)) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMalloc((void**)&ctx->d_state_in, sizeof(double) * 6)) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMalloc((void**)&ctx->d_shard, sizeof(double) * 32)) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMalloc((void**)&ctx->d_eval, sizeof(phovo_iter_stats))) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMallocHost((void**)&ctx->h_pose, sizeof(PoseDev))) != cudaSuccess) return bail("cudaMallocHost", e);
-  if ((e = cudaMallocHost((void**)&ctx->h_log, sizeof(phovo_iter_stats) * ctx->log_cap)) != cudaSuccess) return bail("cudaMallocHost", e);
-  if ((e = cudaMallocHost((void**)&ctx->h_state_in, sizeof(double) * 8)) != cudaSuccess) return bail("cudaMallocHost", e);
-  if ((e = cudaMallocHost((void**)&ctx->h_eval, sizeof(phovo_iter_stats))) != cudaSuccess) return bail("cudaMallocHost", e);
-  memset(ctx->h_pose, 0, sizeof(PoseDev));
+  if ((e = ctx->d_pose.ensure(1)) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = cudaMemset(ctx->d_pose.get(), 0, sizeof(PoseDev))) != cudaSuccess) return bail("cudaMemset", e);
+  if ((e = ctx->d_log.ensure(1024)) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = ctx->d_state_in.ensure(6)) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = ctx->d_shard.ensure(32)) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = ctx->d_eval.ensure(1)) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = ctx->h_pose.ensure(1)) != cudaSuccess) return bail("cudaMallocHost", e);
+  if ((e = ctx->h_log.ensure(1024)) != cudaSuccess) return bail("cudaMallocHost", e);
+  if ((e = ctx->h_state_in.ensure(8)) != cudaSuccess) return bail("cudaMallocHost", e);
+  if ((e = ctx->h_eval.ensure(1)) != cudaSuccess) return bail("cudaMallocHost", e);
+  memset(ctx->h_pose.get(), 0, sizeof(PoseDev));
   *out = ctx;
   return PHOVO_OK;
 }
@@ -394,23 +322,8 @@ extern "C" int phovo_destroy(phovo_ctx* ctx) {
   if (ctx->arena_base) ctx->arena_reset(nullptr, 0);   // arena-backed buffers belong to the batch state
   ctx->invalidate_graph();
   phovo_batch_release(ctx);
-  for (int l = 0; l < PHOVO_MAX_LEVELS; ++l) {
-    cudaFree(ctx->I0[l]); cudaFree(ctx->D0[l]); cudaFree(ctx->I1[l]); cudaFree(ctx->Gx[l]); cudaFree(ctx->Gy[l]);
-  }
-  for (int l = 0; l < PHOVO_MAX_LEVELS; ++l) { cudaFree(ctx->D1[l]); cudaFree(ctx->GxD[l]); cudaFree(ctx->GyD[l]); }
-  cudaFree(ctx->d_gain);
-  cudaFree(ctx->winner); cudaFree(ctx->valid); cudaFree(ctx->scratch64[0]); cudaFree(ctx->scratch64[1]); cudaFree(ctx->partials);
-  cudaFree(ctx->stage_gray[0]); cudaFree(ctx->stage_gray[1]); cudaFree(ctx->stage_depth);
-  cudaFree(ctx->d_pose); cudaFree(ctx->d_log); cudaFree(ctx->d_state_in); cudaFree(ctx->d_shard); cudaFree(ctx->d_level_dmin); cudaFree(ctx->d_eval);
-  cudaFree(ctx->dump_res); cudaFree(ctx->dump_jac);
-  for (int k = 0; k < 3; ++k) cudaFree(ctx->warp_io[k]);
-  for (int r = 0; r < 8; ++r)
+  for (int r = 0; r < 8; ++r)   // peers' areas are mappings, not allocations of this context
     if (ctx->xchg_opened[r]) cudaIpcCloseMemHandle(ctx->xchg_peer[r]);
-  cudaFree(ctx->xchg_own); cudaFree(ctx->xchg_peers_dev);
-  cudaFreeHost(ctx->h_pose); cudaFreeHost(ctx->h_log); cudaFreeHost(ctx->h_state_in); cudaFreeHost(ctx->h_eval);
-  cudaEventDestroy(ctx->ev_copy);
-  for (int i = 0; i < 4; ++i) cudaEventDestroy(ctx->ev_time[i]);
-  if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
   return PHOVO_OK;
 }
@@ -508,9 +421,8 @@ extern "C" int phovo_set_build_all_levels(phovo_ctx* ctx, int enable) {
 extern "C" int phovo_set_stream(phovo_ctx* ctx, void* cuda_stream) {
   if (!ctx) return PHOVO_E_INVALID;
   cudaStreamSynchronize(ctx->stream);
-  if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
+  ctx->own_stream.reset();
   ctx->stream = (cudaStream_t)cuda_stream;
-  ctx->own_stream = false;
   ctx->invalidate_graph();
   return PHOVO_OK;
 }
@@ -542,14 +454,14 @@ extern "C" int phovo_set_source(phovo_ctx* ctx, const uint8_t* gray, size_t gray
   CK(cudaSetDevice(ctx->device));
   int rc = prepare_levels(ctx, rows, cols);
   if (rc) return rc;
-  CK(cudaEventRecord(ctx->ev_time[0], ctx->stream));
+  CK(cudaEventRecord(ctx->ev_time[0].get(), ctx->stream));
   const void* dg; size_t dgs; const void* dd; size_t dds;
-  if ((rc = stage_image(ctx, gray, gray_step, 1, rows, cols, &ctx->stage_gray[0], &ctx->stage_gray_cap[0], &dg, &dgs))) return rc;
-  if ((rc = stage_image(ctx, depth, depth_step, depth_elt(depth_type), rows, cols, &ctx->stage_depth, &ctx->stage_depth_cap, &dd, &dds))) return rc;
+  if ((rc = stage_image(ctx, gray, gray_step, 1, rows, cols, ctx->stage_gray[0], &dg, &dgs))) return rc;
+  if ((rc = stage_image(ctx, depth, depth_step, depth_elt(depth_type), rows, cols, ctx->stage_depth, &dd, &dds))) return rc;
   if ((rc = finish_uploads(ctx))) return rc;
   if ((rc = build_intensity(ctx, dg, dgs, false))) return rc;
   if ((rc = build_depth(ctx, dd, depth_type, dds, depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0))) return rc;
-  CK(cudaEventRecord(ctx->ev_time[1], ctx->stream));
+  CK(cudaEventRecord(ctx->ev_time[1].get(), ctx->stream));
   ctx->have_src = true;
   ctx->setup_timed = true;
   ctx->level_dmin_valid = false;
@@ -565,11 +477,11 @@ extern "C" int phovo_set_target(phovo_ctx* ctx, const uint8_t* gray, size_t gray
   CK(cudaSetDevice(ctx->device));
   const void* dg; size_t dgs;
   int rc;
-  if (!ctx->setup_timed) CK(cudaEventRecord(ctx->ev_time[0], ctx->stream));
-  if ((rc = stage_image(ctx, gray, gray_step, 1, rows, cols, &ctx->stage_gray[1], &ctx->stage_gray_cap[1], &dg, &dgs))) return rc;
+  if (!ctx->setup_timed) CK(cudaEventRecord(ctx->ev_time[0].get(), ctx->stream));
+  if ((rc = stage_image(ctx, gray, gray_step, 1, rows, cols, ctx->stage_gray[1], &dg, &dgs))) return rc;
   if ((rc = finish_uploads(ctx))) return rc;
   if ((rc = build_intensity(ctx, dg, dgs, true))) return rc;
-  CK(cudaEventRecord(ctx->ev_time[1], ctx->stream));
+  CK(cudaEventRecord(ctx->ev_time[1].get(), ctx->stream));
   ctx->have_tgt = true;
   ctx->have_tgt_depth = false;
   return wait_uploads(ctx);
@@ -581,26 +493,26 @@ extern "C" int phovo_set_target_depth(phovo_ctx* ctx, const void* depth, int dep
   if (src_type_of_depth(depth_type) < 0) return ctx->fail(PHOVO_E_INVALID, "unknown depth_type");
   if (depth_step < (size_t)ctx->cols * depth_elt(depth_type)) return ctx->fail(PHOVO_E_INVALID, "row stride smaller than a row");
   CK(cudaSetDevice(ctx->device));
-  if (!ctx->d_gain) CK(cudaMalloc((void**)&ctx->d_gain, sizeof(double) * PHOVO_MAX_LEVELS));   // (a slot's lives in its arena)
+  CK(ctx->d_gain.ensure(PHOVO_MAX_LEVELS));   // (a slot's is a view of its arena)
   const void* dd; size_t dds; int rc;
-  if ((rc = stage_image(ctx, depth, depth_step, depth_elt(depth_type), ctx->rows, ctx->cols, &ctx->stage_depth, &ctx->stage_depth_cap, &dd, &dds))) return rc;
+  if ((rc = stage_image(ctx, depth, depth_step, depth_elt(depth_type), ctx->rows, ctx->cols, ctx->stage_depth, &dd, &dds))) return rc;
   if ((rc = finish_uploads(ctx))) return rc;
   for (int l = 0; l < ctx->cfg.num_levels; ++l) {
     if (!ctx->level_active(l)) continue;
     const int r = ctx->lrows[l], c = ctx->lcols[l];
     const size_t n = (size_t)r * c;
-    double** arrs[3] = {&ctx->D1[l], &ctx->GxD[l], &ctx->GyD[l]};
+    DeviceArray<double>* arrs[3] = {&ctx->D1[l], &ctx->GxD[l], &ctx->GyD[l]};
     for (int a = 0; a < 3; ++a) {
-      double* before = *arrs[a];
-      CK(ctx_ensure(ctx, arrs[a], &ctx->bcap[l][a], n));
-      if (before != *arrs[a]) ctx->invalidate_graph();
+      bool fresh;
+      CK(ctx_ensure(ctx, *arrs[a], n, &fresh));
+      if (fresh) ctx->invalidate_graph();
     }
     // BiObjective.h:574 (depth pyramid, no blur), :224-237 (Scharr of depth / m_MaxDepth), :299 (gain)
     ctx->launches += launch_build_level(ctx->stream, dd, src_type_of_depth(depth_type), dds, depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0,
-                                        ctx->rows, ctx->cols, l, ctx->D1[l], r, c);
-    ctx->launches += launch_scale(ctx->stream, ctx->D1[l], 1. / ctx->cfg.max_depth, ctx->scratch64[0], n);
-    ctx->launches += launch_scharr_store(ctx->stream, ctx->scratch64[0], r, c, ctx->cfg.grad_scale[l], ctx->GxD[l], ctx->GyD[l]);
-    ctx->launches += launch_mean_ratio(ctx->stream, ctx->I1[l], ctx->D1[l], n, ctx->d_gain + l);
+                                        ctx->rows, ctx->cols, l, ctx->D1[l].get(), r, c);
+    ctx->launches += launch_scale(ctx->stream, ctx->D1[l].get(), 1. / ctx->cfg.max_depth, ctx->scratch64[0].get(), n);
+    ctx->launches += launch_scharr_store(ctx->stream, ctx->scratch64[0].get(), r, c, ctx->cfg.grad_scale[l], ctx->GxD[l].get(), ctx->GyD[l].get());
+    ctx->launches += launch_mean_ratio(ctx->stream, ctx->I1[l].get(), ctx->D1[l].get(), n, ctx->d_gain.get() + l);
   }
   CK(cudaGetLastError());
   ctx->have_tgt_depth = true;
@@ -616,13 +528,12 @@ extern "C" int phovo_promote_target_to_source(phovo_ctx* ctx, const void* depth,
   // (same convert + resize + blur, AN:471-474 vs AN:484-487): swap the level buffers.
   for (int l = 0; l < ctx->cfg.num_levels; ++l) {
     if (!ctx->level_active(l)) continue;
-    double* t = ctx->I0[l]; ctx->I0[l] = ctx->I1[l]; ctx->I1[l] = t;
-    size_t c = ctx->lcap[l][0]; ctx->lcap[l][0] = ctx->lcap[l][2]; ctx->lcap[l][2] = c;
+    ctx->I0[l].swap(ctx->I1[l]);
   }
   ctx->invalidate_graph();
-  CK(cudaEventRecord(ctx->ev_time[0], ctx->stream));
+  CK(cudaEventRecord(ctx->ev_time[0].get(), ctx->stream));
   const void* dd; size_t dds; int rc;
-  if ((rc = stage_image(ctx, depth, depth_step, depth_elt(depth_type), ctx->rows, ctx->cols, &ctx->stage_depth, &ctx->stage_depth_cap, &dd, &dds))) return rc;
+  if ((rc = stage_image(ctx, depth, depth_step, depth_elt(depth_type), ctx->rows, ctx->cols, ctx->stage_depth, &dd, &dds))) return rc;
   if ((rc = finish_uploads(ctx))) return rc;
   if ((rc = build_depth(ctx, dd, depth_type, dds, depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0))) return rc;
   ctx->have_src = true; ctx->have_tgt = false; ctx->setup_timed = true;
@@ -654,26 +565,23 @@ static int total_iterations(const phovo_ctx* ctx) {
 }
 
 static int ensure_log(phovo_ctx* ctx, int want) {
-  if (want <= ctx->log_cap) return PHOVO_OK;
-  cudaFree(ctx->d_log); cudaFreeHost(ctx->h_log);
-  ctx->d_log = nullptr; ctx->h_log = nullptr;
-  ctx->log_cap = want;
-  CK(cudaMalloc((void**)&ctx->d_log, sizeof(phovo_iter_stats) * want));
-  CK(cudaMallocHost((void**)&ctx->h_log, sizeof(phovo_iter_stats) * want));
-  ctx->invalidate_graph();
+  if (want <= ctx->log_cap()) return PHOVO_OK;
+  ctx->invalidate_graph();   // it writes to d_log
+  CK(ctx->d_log.ensure(want));
+  CK(ctx->h_log.ensure(want));
   return PHOVO_OK;
 }
 
 static int read_back(phovo_ctx* ctx) {
   const int cap = total_iterations(ctx);
-  CK(cudaMemcpyAsync(ctx->h_pose, ctx->d_pose, sizeof(PoseDev), cudaMemcpyDeviceToHost, ctx->stream));
-  if (cap > 0) CK(cudaMemcpyAsync(ctx->h_log, ctx->d_log, sizeof(phovo_iter_stats) * (size_t)(cap < ctx->log_cap ? cap : ctx->log_cap), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaEventRecord(ctx->ev_time[3], ctx->stream));
+  CK(cudaMemcpyAsync(ctx->h_pose.get(), ctx->d_pose.get(), sizeof(PoseDev), cudaMemcpyDeviceToHost, ctx->stream));
+  if (cap > 0) CK(cudaMemcpyAsync(ctx->h_log.get(), ctx->d_log.get(), sizeof(phovo_iter_stats) * (size_t)std::min(cap, ctx->log_cap()), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaEventRecord(ctx->ev_time[3].get(), ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
-  memcpy(ctx->state, ctx->h_pose->state, sizeof(double) * 6);
-  int n = ctx->h_pose->log_count;
+  memcpy(ctx->state, ctx->h_pose.get()->state, sizeof(double) * 6);
+  int n = ctx->h_pose.get()->log_count;
   if (n > cap) n = cap;
-  ctx->log.assign(ctx->h_log, ctx->h_log + n);
+  ctx->log.assign(ctx->h_log.get(), ctx->h_log.get() + n);
   for (int k = 0; k < 6; ++k)
     if (!isfinite(ctx->state[k])) return ctx->fail(PHOVO_E_NUMERIC, "non-finite state after Optimize (singular normal equations?)");
   return PHOVO_OK;
@@ -681,26 +589,26 @@ static int read_back(phovo_ctx* ctx) {
 
 // Plain stream launches; the host polls the device-side termination flag every `poll` iterations.
 static int optimize_stream(phovo_ctx* ctx) {
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose, nullptr, ctx->state, ctx->log_cap);
+  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
   const int poll = 4;
   for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {   // AN:502-503
     const int M = ctx->cfg.max_num_iterations[level];
     if (M <= 0) continue;   // AN:526: an empty pass, then the iteration test breaks (AN:383)
     const LevelParams L = ctx->level_params(level);
     const LevelPtrs P = ctx->level_ptrs(level);
-    ctx->launches += launch_begin_level(ctx->stream, ctx->d_pose, M);
+    ctx->launches += launch_begin_level(ctx->stream, ctx->d_pose.get(), M);
     for (int it = 0; it < M;) {
       int chunk = M - it < poll ? M - it : poll;
       for (int k = 0; k < chunk; ++k) {
         int grid = 0;
-        ctx->launches += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose, ctx->partials, ctx->sm_count, &grid, nullptr, nullptr, false);
-        ctx->launches += launch_reduce_solve(ctx->stream, L, ctx->d_pose, ctx->partials, grid, ctx->d_log, 0ull);
+        ctx->launches += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->sm_count, &grid, nullptr, nullptr, false);
+        ctx->launches += launch_reduce_solve(ctx->stream, L, ctx->d_pose.get(), ctx->partials.get(), grid, ctx->d_log.get(), 0ull);
       }
       it += chunk;
       if (it < M) {
-        CK(cudaMemcpyAsync(&ctx->h_pose->done, &ctx->d_pose->done, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(&ctx->h_pose.get()->done, &ctx->d_pose.get()->done, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
-        if (ctx->h_pose->done) break;
+        if (ctx->h_pose.get()->done) break;
       }
     }
   }
@@ -736,13 +644,13 @@ static int build_graph(phovo_ctx* ctx) {
     return cudaSuccess;
   };
 
-  CK(capture(g, true, [&] { launches_per_run += launch_set_state(ctx->stream, ctx->d_pose, ctx->d_state_in, ctx->state, ctx->log_cap); }));
+  CK(capture(g, true, [&] { launches_per_run += launch_set_state(ctx->stream, ctx->d_pose.get(), ctx->d_state_in.get(), ctx->state, ctx->log_cap()); }));
   for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
     const int M = ctx->cfg.max_num_iterations[level];
     if (M <= 0) continue;
     const LevelParams L = ctx->level_params(level);
     const LevelPtrs P = ctx->level_ptrs(level);
-    CK(capture(g, true, [&] { launches_per_run += launch_begin_level(ctx->stream, ctx->d_pose, M); }));
+    CK(capture(g, true, [&] { launches_per_run += launch_begin_level(ctx->stream, ctx->d_pose.get(), M); }));
     cudaGraphConditionalHandle handle;
     CK(cudaGraphConditionalHandleCreate(&handle, g, 1, cudaGraphCondAssignDefault));
     cudaGraphNodeParams np = {};
@@ -756,8 +664,8 @@ static int build_graph(phovo_ctx* ctx) {
     int per_iter = 0;
     CK(capture(body, false, [&] {
       int grid = 0;
-      per_iter += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose, ctx->partials, ctx->sm_count, &grid, nullptr, nullptr, false);
-      per_iter += launch_reduce_solve(ctx->stream, L, ctx->d_pose, ctx->partials, grid, ctx->d_log, (unsigned long long)handle);
+      per_iter += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->sm_count, &grid, nullptr, nullptr, false);
+      per_iter += launch_reduce_solve(ctx->stream, L, ctx->d_pose.get(), ctx->partials.get(), grid, ctx->d_log.get(), (unsigned long long)handle);
     }));
     ctx->graph_launches_per_iter = per_iter;
     tail = cond_node; have_tail = true;
@@ -772,8 +680,8 @@ static int optimize_graph(phovo_ctx* ctx) {
     int rc = build_graph(ctx);
     if (rc) return rc;
   }
-  memcpy(ctx->h_state_in, ctx->state, sizeof(double) * 6);
-  CK(cudaMemcpyAsync(ctx->d_state_in, ctx->h_state_in, sizeof(double) * 6, cudaMemcpyHostToDevice, ctx->stream));
+  memcpy(ctx->h_state_in.get(), ctx->state, sizeof(double) * 6);
+  CK(cudaMemcpyAsync(ctx->d_state_in.get(), ctx->h_state_in.get(), sizeof(double) * 6, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaGraphLaunch(ctx->graph_exec, ctx->stream));
   return PHOVO_OK;
 }
@@ -781,7 +689,7 @@ static int optimize_graph(phovo_ctx* ctx) {
 // One cooperative persistent launch per active level: set-state, then for each level begin-level + loop kernel.
 static int optimize_coop(phovo_ctx* ctx, bool* unavailable) {
   *unavailable = false;
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose, nullptr, ctx->state, ctx->log_cap);
+  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
   for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {   // AN:502-503
     const int M = ctx->cfg.max_num_iterations[level];
     if (M <= 0) continue;
@@ -791,7 +699,7 @@ static int optimize_coop(phovo_ctx* ctx, bool* unavailable) {
     // and writes the whole PoseDev back when the level ends)
     int grid = 0; cudaError_t e = cudaSuccess;
     if (ctx->execution == 3 && !ctx->cluster_broken) {      // small level: one thread-block cluster, cluster barriers
-      const int rcl = launch_level_cluster(ctx->stream, L, P, ctx->d_pose, ctx->d_log, &ctx->launch_state, &e);
+      const int rcl = launch_level_cluster(ctx->stream, L, P, ctx->d_pose.get(), ctx->d_log.get(), &ctx->launch_state, &e);
       if (rcl > 0) { ctx->launches += rcl; continue; }
       if (rcl < 0) {
         cudaGetLastError();
@@ -799,7 +707,7 @@ static int optimize_coop(phovo_ctx* ctx, bool* unavailable) {
         ctx->graph_error = std::string("cluster launch unavailable: ") + cudaGetErrorString(e);
       }
     }
-    const int rc = launch_level_coop(ctx->stream, L, P, ctx->d_pose, ctx->partials, ctx->d_log, &ctx->launch_state, ctx->sm_count, &grid, &e);
+    const int rc = launch_level_coop(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->d_log.get(), &ctx->launch_state, ctx->sm_count, &grid, &e);
     if (rc < 0) {
       cudaGetLastError();
       ctx->graph_error = std::string("cooperative launch unavailable: ") + cudaGetErrorString(e);
@@ -818,7 +726,7 @@ static int optimize_ceres(phovo_ctx* ctx);
 // Ceres mode with the LM loop on the device: one cooperative launch per active level.
 static int optimize_ceres_coop(phovo_ctx* ctx, bool* unavailable) {
   *unavailable = false;
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose, nullptr, ctx->state, ctx->log_cap);
+  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
   for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
     const int M = ctx->cfg.max_num_iterations[level];
     if (!(M > 0)) continue;   // CE:437
@@ -828,7 +736,7 @@ static int optimize_ceres_coop(phovo_ctx* ctx, bool* unavailable) {
                           ctx->cfg.initial_trust_region_radius[level], ctx->cfg.max_trust_region_radius[level],
                           ctx->cfg.min_trust_region_radius[level], ctx->cfg.min_relative_decrease[level]};
     cudaError_t e = cudaSuccess;
-    const int rc = launch_level_coop_ceres(ctx->stream, L, P, ctx->d_pose, ctx->partials, ctx->d_log, lm, M, &ctx->launch_state, ctx->sm_count, &e);
+    const int rc = launch_level_coop_ceres(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->d_log.get(), lm, M, &ctx->launch_state, ctx->sm_count, &e);
     if (rc < 0) {
       cudaGetLastError();
       ctx->graph_error = std::string("cooperative launch unavailable: ") + cudaGetErrorString(e);
@@ -849,7 +757,7 @@ extern "C" int phovo_optimize(phovo_ctx* ctx) {
   CK(cudaSetDevice(ctx->device));
   if ((rc = ensure_log(ctx, total_iterations(ctx) + 1))) return rc;
   ctx->setup_timed = false;
-  CK(cudaEventRecord(ctx->ev_time[2], ctx->stream));
+  CK(cudaEventRecord(ctx->ev_time[2].get(), ctx->stream));
   ctx->last_used_graph = 0;
   ctx->last_path = 0;
   if (ctx->cfg.mode == PHOVO_MODE_CERES) {
@@ -878,7 +786,7 @@ extern "C" int phovo_optimize(phovo_ctx* ctx) {
         ctx->last_used_graph = 1;
         ctx->last_path = 1;
         int iters = 0;
-        for (int l = 0; l < ctx->cfg.num_levels; ++l) iters += ctx->h_pose->iters_per_level[l];
+        for (int l = 0; l < ctx->cfg.num_levels; ++l) iters += ctx->h_pose.get()->iters_per_level[l];
         ctx->launches += ctx->graph_launches_fixed + (int64_t)iters * ctx->graph_launches_per_iter;
         return rc;
       }
@@ -956,16 +864,16 @@ extern "C" int phovo_warp_image(phovo_ctx* ctx, const uint8_t* gray, size_t gray
   if (n > (size_t)INT32_MAX) return ctx->fail(PHOVO_E_UNSUPPORTED, "warpImage: frames of 2^31 pixels or more");
   CK(cudaSetDevice(ctx->device));
   const void* dg; size_t dgs; const void* dd; size_t dds; int rc;
-  if ((rc = stage_image(ctx, gray, gray_step, 1, rows, cols, &ctx->stage_gray[0], &ctx->stage_gray_cap[0], &dg, &dgs))) return rc;
-  if ((rc = stage_image(ctx, depth, depth_step, depth_elt(depth_type), rows, cols, &ctx->stage_depth, &ctx->stage_depth_cap, &dd, &dds))) return rc;
+  if ((rc = stage_image(ctx, gray, gray_step, 1, rows, cols, ctx->stage_gray[0], &dg, &dgs))) return rc;
+  if ((rc = stage_image(ctx, depth, depth_step, depth_elt(depth_type), rows, cols, ctx->stage_depth, &dd, &dds))) return rc;
   const void* dt = nullptr; size_t dts = 0;
-  if (target && (rc = stage_image(ctx, target, target_step, 1, rows, cols, &ctx->warp_io[1], &ctx->warp_io_cap[1], &dt, &dts))) return rc;
+  if (target && (rc = stage_image(ctx, target, target_step, 1, rows, cols, ctx->warp_io[1], &dt, &dts))) return rc;
   ctx->h2d_pending = false; ctx->device_input_in_flight = false;   // this call ends with a stream synchronise
   // outputs: write in place for device callers, through a dense device buffer for host callers
   uint8_t* dw = warped; size_t dws = warped_step; uint8_t* ddf = diff; size_t ddfs = diff_step;
   const bool w_host = !is_device_pointer(warped), d_host = diff && !is_device_pointer(diff);
-  if (w_host) { CK(ensure(&ctx->warp_io[0], &ctx->warp_io_cap[0], n)); dw = (uint8_t*)ctx->warp_io[0]; dws = cols; }
-  if (d_host) { CK(ensure(&ctx->warp_io[2], &ctx->warp_io_cap[2], n)); ddf = (uint8_t*)ctx->warp_io[2]; ddfs = cols; }
+  if (w_host) { CK(ctx->warp_io[0].ensure(n)); dw = (uint8_t*)ctx->warp_io[0].get(); dws = cols; }
+  if (d_host) { CK(ctx->warp_io[2].ensure(n)); ddf = (uint8_t*)ctx->warp_io[2].get(); ddfs = cols; }
   WarpImages W;
   memset(&W, 0, sizeof(W));
   W.rows = rows; W.cols = cols;
@@ -974,11 +882,7 @@ extern "C" int phovo_warp_image(phovo_ctx* ctx, const uint8_t* gray, size_t gray
   W.target = (const uint8_t*)dt; W.target_step = dts;
   W.warped = dw; W.warped_step = dws;
   W.diff = ddf; W.diff_step = ddfs;
-  const double p = pow(2, level);                                   // BASE:89-94: K / 2^level
-  WarpIntrinsics I;
-  I.fx = K[0] / p; I.fy = K[4] / p; I.ox = K[2] / p; I.oy = K[5] / p;
-  I.inv_fx = 1.f / I.fx; I.inv_fy = 1.f / I.fy;                    // BASE:91-92
-  if ((rc = phovo_internal_warp_images(ctx, W, src_type_of_depth(depth_type), I, 1, rt))) return rc;
+  if ((rc = phovo_internal_warp_images(ctx, W, src_type_of_depth(depth_type), scaled_intrinsics(K, level), 1, rt))) return rc;
   if (w_host) CK(cudaMemcpy2DAsync(warped, warped_step, dw, dws, cols, rows, cudaMemcpyDeviceToHost, ctx->stream));
   if (d_host) CK(cudaMemcpy2DAsync(diff, diff_step, ddf, ddfs, cols, rows, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
@@ -1004,7 +908,7 @@ extern "C" int phovo_get_level_image(phovo_ctx* ctx, int which, int level, doubl
   if (cols) *cols = ctx->lcols[level];
   if (!dst) return PHOVO_OK;
   CK(cudaSetDevice(ctx->device));
-  const double* src = which == 0 ? ctx->I0[level] : which == 1 ? ctx->D0[level] : which == 2 ? ctx->I1[level] : which == 3 ? ctx->Gx[level] : ctx->Gy[level];
+  const double* src = which == 0 ? ctx->I0[level].get() : which == 1 ? ctx->D0[level].get() : which == 2 ? ctx->I1[level].get() : which == 3 ? ctx->Gx[level].get() : ctx->Gy[level].get();
   CK(cudaMemcpyAsync(dst, src, sizeof(double) * (size_t)ctx->lrows[level] * ctx->lcols[level], cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return PHOVO_OK;
@@ -1013,14 +917,14 @@ extern "C" int phovo_get_level_image(phovo_ctx* ctx, int which, int level, doubl
 static int eval_at(phovo_ctx* ctx, int level, const double state[6], phovo_iter_stats* out, double* dres, double* djac) {
   const LevelParams L = ctx->level_params(level);
   const LevelPtrs P = ctx->level_ptrs(level);
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose, nullptr, state, 0);
+  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, state, 0);
   int grid = 0;
-  ctx->launches += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose, ctx->partials, ctx->sm_count, &grid, dres, djac, false);
-  ctx->launches += launch_reduce_only(ctx->stream, L, ctx->d_pose, ctx->partials, grid, ctx->d_eval);
+  ctx->launches += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->sm_count, &grid, dres, djac, false);
+  ctx->launches += launch_reduce_only(ctx->stream, L, ctx->d_pose.get(), ctx->partials.get(), grid, ctx->d_eval.get());
   CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(ctx->h_eval, ctx->d_eval, sizeof(phovo_iter_stats), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(ctx->h_eval.get(), ctx->d_eval.get(), sizeof(phovo_iter_stats), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
-  *out = *ctx->h_eval;
+  *out = *ctx->h_eval.get();
   return PHOVO_OK;
 }
 
@@ -1040,22 +944,22 @@ extern "C" int phovo_eval_residuals(phovo_ctx* ctx, int level, const double stat
   if (level < 0 || level >= ctx->cfg.num_levels || !ctx->level_active(level)) return ctx->fail(PHOVO_E_INVALID, "level not built");
   CK(cudaSetDevice(ctx->device));
   const size_t n = (size_t)ctx->lrows[level] * ctx->lcols[level] * (ctx->cfg.mode == PHOVO_MODE_BIOBJECTIVE ? 2 : 1);
-  CK(ensure(&ctx->dump_res, &ctx->dump_res_cap, n));
-  CK(ensure(&ctx->dump_jac, &ctx->dump_jac_cap, n * 6));
-  CK(cudaMemsetAsync(ctx->dump_res, 0, sizeof(double) * n, ctx->stream));
-  CK(cudaMemsetAsync(ctx->dump_jac, 0, sizeof(double) * n * 6, ctx->stream));
+  CK(ctx->dump_res.ensure(n));
+  CK(ctx->dump_jac.ensure(n * 6));
+  CK(cudaMemsetAsync(ctx->dump_res.get(), 0, sizeof(double) * n, ctx->stream));
+  CK(cudaMemsetAsync(ctx->dump_jac.get(), 0, sizeof(double) * n * 6, ctx->stream));
   phovo_iter_stats tmp;
-  if ((rc = eval_at(ctx, level, state, &tmp, ctx->dump_res, ctx->dump_jac))) return rc;
-  if (residuals) CK(cudaMemcpy(residuals, ctx->dump_res, sizeof(double) * n, cudaMemcpyDeviceToHost));
-  if (jacobian) CK(cudaMemcpy(jacobian, ctx->dump_jac, sizeof(double) * n * 6, cudaMemcpyDeviceToHost));
+  if ((rc = eval_at(ctx, level, state, &tmp, ctx->dump_res.get(), ctx->dump_jac.get()))) return rc;
+  if (residuals) CK(cudaMemcpy(residuals, ctx->dump_res.get(), sizeof(double) * n, cudaMemcpyDeviceToHost));
+  if (jacobian) CK(cudaMemcpy(jacobian, ctx->dump_jac.get(), sizeof(double) * n * 6, cudaMemcpyDeviceToHost));
   return PHOVO_OK;
 }
 
 extern "C" int phovo_get_timings(const phovo_ctx* ctx, float* setup_ms, float* optimize_ms) {
   if (!ctx) return PHOVO_E_INVALID;
   float a = 0, b = 0;
-  if (setup_ms) { if (cudaEventElapsedTime(&a, ctx->ev_time[0], ctx->ev_time[1]) != cudaSuccess) { a = -1; cudaGetLastError(); } *setup_ms = a; }
-  if (optimize_ms) { if (cudaEventElapsedTime(&b, ctx->ev_time[2], ctx->ev_time[3]) != cudaSuccess) { b = -1; cudaGetLastError(); } *optimize_ms = b; }
+  if (setup_ms) { if (cudaEventElapsedTime(&a, ctx->ev_time[0].get(), ctx->ev_time[1].get()) != cudaSuccess) { a = -1; cudaGetLastError(); } *setup_ms = a; }
+  if (optimize_ms) { if (cudaEventElapsedTime(&b, ctx->ev_time[2].get(), ctx->ev_time[3].get()) != cudaSuccess) { b = -1; cudaGetLastError(); } *optimize_ms = b; }
   return PHOVO_OK;
 }
 
@@ -1164,7 +1068,7 @@ static int optimize_ceres(phovo_ctx* ctx) {
     }
   }
   memcpy(ctx->state, x, sizeof(x));
-  CK(cudaEventRecord(ctx->ev_time[3], ctx->stream));
+  CK(cudaEventRecord(ctx->ev_time[3].get(), ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   for (int k = 0; k < 6; ++k)
     if (!isfinite(ctx->state[k])) return ctx->fail(PHOVO_E_NUMERIC, "non-finite state after Optimize");
@@ -1186,14 +1090,14 @@ extern "C" int phovo_shard_configure(phovo_ctx* ctx, int rank, int world) {
 
 extern "C" int phovo_shard_buffer(phovo_ctx* ctx, double** dev_ptr) {
   if (!ctx || !dev_ptr) return PHOVO_E_INVALID;
-  *dev_ptr = ctx->d_shard;
+  *dev_ptr = ctx->d_shard.get();
   return PHOVO_OK;
 }
 
 extern "C" int phovo_shard_read_buffer(phovo_ctx* ctx, double out[32]) {
   if (!ctx || !out) return PHOVO_E_INVALID;
   CK(cudaSetDevice(ctx->device));
-  CK(cudaMemcpyAsync(out, ctx->d_shard, sizeof(double) * 32, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(out, ctx->d_shard.get(), sizeof(double) * 32, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return PHOVO_OK;
 }
@@ -1201,7 +1105,7 @@ extern "C" int phovo_shard_read_buffer(phovo_ctx* ctx, double out[32]) {
 extern "C" int phovo_shard_write_buffer(phovo_ctx* ctx, const double in[32]) {
   if (!ctx || !in) return PHOVO_E_INVALID;
   CK(cudaSetDevice(ctx->device));
-  CK(cudaMemcpyAsync(ctx->d_shard, in, sizeof(double) * 32, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(ctx->d_shard.get(), in, sizeof(double) * 32, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return PHOVO_OK;
 }
@@ -1212,8 +1116,8 @@ extern "C" int phovo_shard_begin(phovo_ctx* ctx) {
   if (rc) return rc;
   CK(cudaSetDevice(ctx->device));
   if ((rc = ensure_log(ctx, total_iterations(ctx) + 1))) return rc;
-  CK(cudaEventRecord(ctx->ev_time[2], ctx->stream));
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose, nullptr, ctx->state, ctx->log_cap);
+  CK(cudaEventRecord(ctx->ev_time[2].get(), ctx->stream));
+  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
   ctx->shard_level = -1;
   return PHOVO_OK;
 }
@@ -1223,7 +1127,7 @@ extern "C" int phovo_shard_begin_level(phovo_ctx* ctx, int level) {
   if (!ctx->level_active(level)) return ctx->fail(PHOVO_E_INVALID, "level not built");
   CK(cudaSetDevice(ctx->device));
   ctx->shard_level = level;
-  ctx->launches += launch_begin_level(ctx->stream, ctx->d_pose, ctx->cfg.max_num_iterations[level]);
+  ctx->launches += launch_begin_level(ctx->stream, ctx->d_pose.get(), ctx->cfg.max_num_iterations[level]);
   return PHOVO_OK;
 }
 
@@ -1233,8 +1137,8 @@ extern "C" int phovo_shard_partial(phovo_ctx* ctx) {
   const LevelParams L = ctx->level_params(ctx->shard_level);
   const LevelPtrs P = ctx->level_ptrs(ctx->shard_level);
   int grid = 0;
-  ctx->launches += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose, ctx->partials, ctx->sm_count, &grid, nullptr, nullptr, false);
-  ctx->launches += launch_reduce_to_buffer(ctx->stream, ctx->partials, grid, ctx->d_shard);
+  ctx->launches += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->sm_count, &grid, nullptr, nullptr, false);
+  ctx->launches += launch_reduce_to_buffer(ctx->stream, ctx->partials.get(), grid, ctx->d_shard.get());
   CK(cudaGetLastError());
   return PHOVO_OK;
 }
@@ -1243,15 +1147,15 @@ extern "C" int phovo_shard_peer_export(phovo_ctx* ctx, void* handle_out) {
   if (!ctx || !handle_out) return PHOVO_E_INVALID;
   static_assert(sizeof(cudaIpcMemHandle_t) == PHOVO_IPC_HANDLE_BYTES, "IPC handle size");
   CK(cudaSetDevice(ctx->device));
-  if (!ctx->xchg_own) {
-    CK(cudaMalloc((void**)&ctx->xchg_own, sizeof(ShardExchange)));
-    CK(cudaMemset(ctx->xchg_own, 0, sizeof(ShardExchange)));
+  if (!ctx->xchg_own.get()) {
+    CK(ctx->xchg_own.ensure(1));
+    CK(cudaMemset(ctx->xchg_own.get(), 0, sizeof(ShardExchange)));
     CK(cudaDeviceSynchronize());
   }
   cudaIpcMemHandle_t h;
-  CK(cudaIpcGetMemHandle(&h, ctx->xchg_own));
+  CK(cudaIpcGetMemHandle(&h, ctx->xchg_own.get()));
   memcpy(handle_out, &h, sizeof(h));
-  ctx->xchg_peer[ctx->shard_rank] = ctx->xchg_own;
+  ctx->xchg_peer[ctx->shard_rank] = ctx->xchg_own.get();
   ctx->xchg_table_dirty = true;
   return PHOVO_OK;
 }
@@ -1279,9 +1183,9 @@ extern "C" int phovo_shard_partial_exchange(phovo_ctx* ctx) {
   const LevelParams L = ctx->level_params(ctx->shard_level);
   const LevelPtrs P = ctx->level_ptrs(ctx->shard_level);
   int grid = 0;
-  ctx->launches += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose, ctx->partials, ctx->sm_count, &grid, nullptr, nullptr, false);
+  ctx->launches += launch_iteration_kernels(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->sm_count, &grid, nullptr, nullptr, false);
   ctx->xchg_epoch += 1;
-  ctx->launches += launch_reduce_exchange(ctx->stream, ctx->d_pose, ctx->partials, grid, ctx->d_shard, ctx->xchg_peers_dev,
+  ctx->launches += launch_reduce_exchange(ctx->stream, ctx->d_pose.get(), ctx->partials.get(), grid, ctx->d_shard.get(), ctx->xchg_peers_dev.get(),
                                           ctx->shard_rank, ctx->shard_world, ctx->xchg_epoch);
   CK(cudaGetLastError());
   return PHOVO_OK;
@@ -1290,9 +1194,9 @@ extern "C" int phovo_shard_partial_exchange(phovo_ctx* ctx) {
 static int upload_peer_table(phovo_ctx* ctx) {
   for (int r = 0; r < ctx->shard_world; ++r)
     if (!ctx->xchg_peer[r]) return ctx->fail(PHOVO_E_INVALID, "peer exchange areas are not all imported (phovo_shard_peer_export / _import)");
-  if (!ctx->xchg_peers_dev) CK(cudaMalloc((void**)&ctx->xchg_peers_dev, sizeof(ShardExchange*) * PHOVO_SHARD_MAX_WORLD));
+  CK(ctx->xchg_peers_dev.ensure(PHOVO_SHARD_MAX_WORLD));
   if (ctx->xchg_table_dirty) {
-    CK(cudaMemcpyAsync(ctx->xchg_peers_dev, ctx->xchg_peer, sizeof(ShardExchange*) * PHOVO_SHARD_MAX_WORLD, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->xchg_peers_dev.get(), ctx->xchg_peer, sizeof(ShardExchange*) * PHOVO_SHARD_MAX_WORLD, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->xchg_table_dirty = false;
   }
@@ -1311,16 +1215,16 @@ extern "C" int phovo_shard_optimize(phovo_ctx* ctx, int min_shard_pixels) {
   if (ctx->shard_world > 1 && (rc = upload_peer_table(ctx))) return rc;
   if ((rc = ensure_log(ctx, total_iterations(ctx) + 1))) return rc;
   if (ctx->shard_world > 1 && !ctx->level_dmin_valid) {   // once per source frame: what bounds the row displacement (ShardArgs)
-    if (!ctx->d_level_dmin) CK(cudaMalloc((void**)&ctx->d_level_dmin, sizeof(double) * PHOVO_MAX_LEVELS));
+    CK(ctx->d_level_dmin.ensure(PHOVO_MAX_LEVELS));
     for (int level = 0; level < ctx->cfg.num_levels; ++level)
       if (ctx->cfg.max_num_iterations[level] > 0)
-        ctx->launches += launch_min_valid_depth(ctx->stream, ctx->D0[level], ctx->lrows[level] * ctx->lcols[level], ctx->cfg.min_depth,
-                                                ctx->cfg.max_depth, ctx->d_level_dmin + level, ctx->sm_count);
+        ctx->launches += launch_min_valid_depth(ctx->stream, ctx->D0[level].get(), ctx->lrows[level] * ctx->lcols[level], ctx->cfg.min_depth,
+                                                ctx->cfg.max_depth, ctx->d_level_dmin.get() + level, ctx->sm_count);
     ctx->level_dmin_valid = true;
   }
   ctx->setup_timed = false;
-  CK(cudaEventRecord(ctx->ev_time[2], ctx->stream));
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose, nullptr, ctx->state, ctx->log_cap);
+  CK(cudaEventRecord(ctx->ev_time[2].get(), ctx->stream));
+  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
   for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {   // AN:502-503
     const int M = ctx->cfg.max_num_iterations[level];
     if (M <= 0) continue;
@@ -1329,9 +1233,9 @@ extern "C" int phovo_shard_optimize(phovo_ctx* ctx, int min_shard_pixels) {
     const bool shard = ctx->shard_world > 1 && (long long)L.rows * L.cols >= (long long)min_shard_pixels;
     if (!shard) { L.row_begin = 0; L.row_end = L.rows; }
     int grid = 0; cudaError_t e = cudaSuccess;
-    const int n = launch_level_coop(ctx->stream, L, P, ctx->d_pose, ctx->partials, ctx->d_log, &ctx->launch_state, ctx->sm_count, &grid, &e,
-                                    shard ? ctx->xchg_peers_dev : nullptr, ctx->shard_rank, ctx->shard_world, ctx->xchg_epoch,
-                                    shard ? ctx->d_level_dmin + level : nullptr);
+    const int n = launch_level_coop(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->d_log.get(), &ctx->launch_state, ctx->sm_count, &grid, &e,
+                                    shard ? ctx->xchg_peers_dev.get() : nullptr, ctx->shard_rank, ctx->shard_world, ctx->xchg_epoch,
+                                    shard ? ctx->d_level_dmin.get() + level : nullptr);
     if (n < 0) { cudaGetLastError(); return ctx->cuda_fail("cooperative launch of the sharded level loop", e); }
     ctx->launches += n;
     if (shard) ctx->xchg_epoch += (unsigned long long)M;               // every rank advances by the same amount
@@ -1339,9 +1243,9 @@ extern "C" int phovo_shard_optimize(phovo_ctx* ctx, int min_shard_pixels) {
   CK(cudaGetLastError());
   ctx->last_path = 2;
   rc = read_back(ctx);
-  if (ctx->xchg_own) {
+  if (ctx->xchg_own.get()) {
     int err = 0;
-    CK(cudaMemcpy(&err, &ctx->xchg_own->error, sizeof(int), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&err, &ctx->xchg_own.get()->error, sizeof(int), cudaMemcpyDeviceToHost));
     if (err) return ctx->fail(PHOVO_E_CUDA, "peer exchange timed out waiting for another rank");
   }
   return rc;
@@ -1351,12 +1255,12 @@ extern "C" int phovo_shard_step(phovo_ctx* ctx, int* done) {
   if (!ctx || ctx->shard_level < 0) return PHOVO_E_INVALID;
   CK(cudaSetDevice(ctx->device));
   const LevelParams L = ctx->level_params(ctx->shard_level);
-  ctx->launches += launch_solve_from_buffer(ctx->stream, L, ctx->d_pose, ctx->d_shard, ctx->d_log);
+  ctx->launches += launch_solve_from_buffer(ctx->stream, L, ctx->d_pose.get(), ctx->d_shard.get(), ctx->d_log.get());
   CK(cudaGetLastError());
   if (done) {
-    CK(cudaMemcpyAsync(&ctx->h_pose->done, &ctx->d_pose->done, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&ctx->h_pose.get()->done, &ctx->d_pose.get()->done, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    *done = ctx->h_pose->done;
+    *done = ctx->h_pose.get()->done;
   }
   return PHOVO_OK;
 }
@@ -1365,9 +1269,9 @@ extern "C" int phovo_shard_finish(phovo_ctx* ctx) {
   if (!ctx) return PHOVO_E_INVALID;
   CK(cudaSetDevice(ctx->device));
   int rc = read_back(ctx);
-  if (ctx->xchg_own) {
+  if (ctx->xchg_own.get()) {
     int err = 0;
-    CK(cudaMemcpy(&err, &ctx->xchg_own->error, sizeof(int), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&err, &ctx->xchg_own.get()->error, sizeof(int), cudaMemcpyDeviceToHost));
     if (err) return ctx->fail(PHOVO_E_CUDA, "peer exchange timed out waiting for another rank");
   }
   return rc;

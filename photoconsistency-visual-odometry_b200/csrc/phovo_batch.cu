@@ -13,6 +13,7 @@
 #include <mutex>
 #include <string>
 #include <chrono>
+#include <memory>
 #include <cstdio>
 #include <cstdlib>
 #include <thread>
@@ -25,142 +26,138 @@ using namespace phovo;
 
 constexpr int kWaveSetupThreads = 4;   // host threads (and streams) that build the pyramids of a wave's slots
 
-struct phovo_batch_state {
-  // packed level records
-  uint8_t* store = nullptr; size_t store_cap = 0;
-  // outputs of the last call (device)
-  double* states = nullptr; size_t states_cap = 0;
-  int32_t* iters = nullptr; size_t iters_cap = 0;
-  double* init = nullptr; size_t init_cap = 0;
-  phovo_iter_stats* log = nullptr; size_t log_cap_entries = 0;
-  int32_t* log_counts = nullptr; size_t log_counts_cap = 0;
-  // host mirrors of the stats (filled on demand)
-  std::vector<phovo_iter_stats> h_log; std::vector<int32_t> h_log_counts;
-  int log_per_pair = 0; int last_pairs = 0; bool log_fetched = false;
-  bool record_stats = false;
-  int debug_flags = 0;
-  unsigned long long last_h2d_bytes = 0;
-  // staging for host inputs: two slots
-  uint8_t* stage_g0[2] = {nullptr, nullptr}; uint8_t* stage_g1[2] = {nullptr, nullptr}; char* stage_d[2] = {nullptr, nullptr};
-  size_t stage_cap_g[2] = {0, 0}, stage_cap_g1[2] = {0, 0}, stage_cap_d[2] = {0, 0};
-  cudaStream_t copy_stream = nullptr;
-  cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr};
-  double* h_states_pinned = nullptr; int32_t* h_iters_pinned = nullptr; size_t h_out_cap = 0;
-  size_t prepared_smem = 0;
-  unsigned int* next_pair = nullptr;   // work counter of the persistent align kernel
-  int sm_count = 0;
-  cudaEvent_t ev_k[3] = {nullptr, nullptr, nullptr};   // before pyramid / between / after align
-  bool timed = false;
-  // batches the shared-memory-resident kernels cannot take (Ceres / photometric + depth solver, blurred levels, levels
-  // beyond the shared-memory budget) run pair by pair on a small pool of per-pair contexts, one host thread each
-  std::vector<phovo_ctx*> pool;
-  int last_path = 0;                                   // 1: shared-memory-resident batch kernels, 2: pool of per-pair contexts, 3: slot waves
-  // slot waves (batch_waves): two halves of per-pair slots; one half aligns while the other is being set up
-  std::vector<phovo_ctx*> slots;
-  cudaStream_t setup_stream[kWaveSetupThreads] = {}; cudaEvent_t ev_setup[kWaveSetupThreads] = {};
-  cudaStream_t align_stream[2] = {nullptr, nullptr}; cudaEvent_t ev_wave_done[2] = {nullptr, nullptr}; cudaEvent_t ev_wave_in[2] = {nullptr, nullptr};
-  char* arena = nullptr; size_t arena_cap = 0, slot_bytes = 0; int arena_rows = 0, arena_cols = 0, arena_slots = 0, wave_half = 0; phovo_config arena_cfg = {};
-  SlotArgs* d_slot_args = nullptr; size_t slot_args_cap = 0; std::vector<SlotArgs> h_slot_args;
-  double* d_wave_init[2] = {nullptr, nullptr}; double* d_wave_states[2] = {nullptr, nullptr}; int32_t* d_wave_iters[2] = {nullptr, nullptr};
-  double* h_wave_states[2] = {nullptr, nullptr}; int32_t* h_wave_iters[2] = {nullptr, nullptr}; size_t wave_cap = 0;
-  uint8_t* wave_g0[2] = {nullptr, nullptr}; uint8_t* wave_g1[2] = {nullptr, nullptr}; char* wave_d0[2] = {nullptr, nullptr}; char* wave_d1[2] = {nullptr, nullptr};
-  size_t wave_g_cap[2] = {0, 0}, wave_g1_cap[2] = {0, 0}, wave_d0_cap[2] = {0, 0}, wave_d1_cap[2] = {0, 0};
-  // warpImage (phovo_batch_warp_image, phovo_warp_image): splat keys of one chunk of pairs (zero between calls while
-  // warp_keys_clean), Rt of the pairs, per-pair summaries, device copies of host inputs and outputs of one chunk
-  uint32_t* warp_keys = nullptr; size_t warp_keys_cap = 0; bool warp_keys_clean = false;
-  double* warp_rts = nullptr; size_t warp_rts_cap = 0;
-  int32_t* warp_landed = nullptr; size_t warp_landed_cap = 0;
-  int64_t* warp_sum = nullptr; size_t warp_sum_cap = 0;
-  uint8_t* warp_io[4] = {nullptr, nullptr, nullptr, nullptr}; size_t warp_io_cap[4] = {0, 0, 0, 0};   // gray0, gray1, warped, diff
-  char* warp_depth = nullptr; size_t warp_depth_cap = 0;
-  int l2_bytes = 0;
-  // normal equations at given states (phovo_batch_eval_normal_equations): winner keys (zero between calls while
-  // eval_keys_clean) and validity of one chunk, its level records and tile partials; states, poses and results of
-  // every pair.  Host inputs are staged through warp_io[0] / warp_io[1] / warp_depth.
-  uint32_t* eval_keys = nullptr; size_t eval_keys_cap = 0; bool eval_keys_clean = false;
-  uint8_t* eval_valid = nullptr; size_t eval_valid_cap = 0;
-  uint8_t* eval_store = nullptr; size_t eval_store_cap = 0;
-  double* eval_partials = nullptr; size_t eval_partials_cap = 0;
-  double* eval_states = nullptr; size_t eval_states_cap = 0;
-  PoseDev* eval_poses = nullptr; size_t eval_poses_cap = 0;
-  double* eval_out = nullptr; size_t eval_out_cap = 0;        // [P][21] H, [P][6] g, [P] cost
-  int32_t* eval_nvalid = nullptr; size_t eval_nvalid_cap = 0;
+// [pairs][rows * cols] frame stacks of a call: gray0, gray1, depth0, depth1 (nullptr: not part of the call)
+struct Frames {
+  const uint8_t* gray0; const uint8_t* gray1; const void* depth0; const void* depth1;
+  Frames offset(size_t p0, size_t frame, size_t delt) const {
+    return {gray0 + p0 * frame, gray1 ? gray1 + p0 * frame : nullptr, (const char*)depth0 + p0 * frame * delt,
+            depth1 ? (const char*)depth1 + p0 * frame * delt : nullptr};
+  }
 };
 
-#define CK(call)                                                      \
-  do {                                                                \
-    cudaError_t e_ = (call);                                          \
-    if (e_ != cudaSuccess) return ctx->cuda_fail((std::string(__func__) + ": " #call).c_str(), e_); \
-  } while (0)
+// Device copies of a chunk of host frames, for the stacks a call has
+struct FrameStage {
+  DeviceArray<uint8_t> gray0, gray1;
+  DeviceArray<char> depth0, depth1;
+  cudaError_t reserve(const Frames& which, size_t pairs, size_t frame, size_t delt) {
+    cudaError_t e = gray0.ensure(pairs * frame);
+    if (e == cudaSuccess && which.gray1) e = gray1.ensure(pairs * frame);
+    if (e == cudaSuccess) e = depth0.ensure(pairs * frame * delt);
+    if (e == cudaSuccess && which.depth1) e = depth1.ensure(pairs * frame * delt);
+    return e;
+  }
+  // Pairs [p0, p0 + np) of `in` on the device: with `copy` copied in here on `stream`, otherwise used in place
+  cudaError_t stage(bool copy, const Frames& in, size_t frame, size_t delt, int p0, int np, cudaStream_t stream, Frames* out) {
+    const Frames f = in.offset(p0, frame, delt);
+    *out = f;
+    if (!copy) return cudaSuccess;
+    const size_t nb = frame * np;
+    cudaError_t e = reserve(in, np, frame, delt);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(gray0.get(), f.gray0, nb, cudaMemcpyDefault, stream);
+    if (e == cudaSuccess && f.gray1) e = cudaMemcpyAsync(gray1.get(), f.gray1, nb, cudaMemcpyDefault, stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(depth0.get(), f.depth0, nb * delt, cudaMemcpyDefault, stream);
+    if (e == cudaSuccess && f.depth1) e = cudaMemcpyAsync(depth1.get(), f.depth1, nb * delt, cudaMemcpyDefault, stream);
+    *out = {gray0.get(), f.gray1 ? gray1.get() : nullptr, depth0.get(), f.depth1 ? depth1.get() : nullptr};
+    return e;
+  }
+};
 
-template <class T>
-static cudaError_t ensure(T** p, size_t* cap, size_t want) {
-  if (*cap >= want && *p) return cudaSuccess;
-  if (*p) cudaFree(*p);
-  *p = nullptr; *cap = 0;
-  cudaError_t e = cudaMalloc((void**)p, want * sizeof(T));
-  if (e == cudaSuccess) *cap = want;
-  return e;
-}
+struct ContextDestroy { void operator()(phovo_ctx* c) const { phovo_destroy(c); } };
+using ContextPtr = std::unique_ptr<phovo_ctx, ContextDestroy>;
+
+struct phovo_batch_state {
+  int sm_count = 0, l2_bytes = 0;
+  int debug_flags = 0;
+  bool record_stats = false;
+  int last_path = 0;                                   // 1: shared-memory-resident batch kernels, 2: pool of per-pair contexts, 3: slot waves
+  unsigned long long last_h2d_bytes = 0;
+  // host mirrors of the per-pair stats of the last call (filled on demand)
+  std::vector<phovo_iter_stats> h_log; std::vector<int32_t> h_log_counts;
+  int log_per_pair = 0; int last_pairs = 0; bool log_fetched = false;
+
+  // the shared-memory-resident kernels (phovo_batch_align, phovo_batch_align_device)
+  struct Resident {
+    DeviceArray<uint8_t> store;                        // packed level records
+    DeviceArray<double> states, init;                  // outputs / inputs of the last call
+    DeviceArray<int32_t> iters;
+    DeviceArray<phovo_iter_stats> log;
+    DeviceArray<int32_t> log_counts;
+    PinnedArray<double> h_states; PinnedArray<int32_t> h_iters;
+    FrameStage stage[2];                               // host inputs: two staging slots
+    Stream copy_stream;
+    Event ev_copied[2], ev_consumed[2];
+    DeviceArray<unsigned int> next_pair;               // work counter of the persistent align kernel
+    Event ev_k[3];                                     // before pyramid / between / after align
+    bool timed = false;
+    size_t prepared_smem = 0;
+  } res;
+
+  // batches the shared-memory-resident kernels cannot take (Ceres / photometric + depth solver, blurred levels, levels
+  // beyond the shared-memory budget) run pair by pair on a small pool of per-pair contexts, one host thread each
+  std::vector<ContextPtr> pool;
+
+  // slot waves (batch_waves): two halves of per-pair slots; one half aligns while the other is being set up
+  struct Waves {
+    Stream setup_stream[kWaveSetupThreads]; Event ev_setup[kWaveSetupThreads];
+    Stream align_stream[2]; Event ev_wave_done[2], ev_wave_in[2];
+    DeviceArray<char> arena;
+    size_t slot_bytes = 0; int arena_rows = 0, arena_cols = 0, arena_slots = 0, wave_half = 0; phovo_config arena_cfg = {};
+    DeviceArray<SlotArgs> d_slot_args; std::vector<SlotArgs> h_slot_args;
+    DeviceArray<double> d_init[2], d_states[2]; DeviceArray<int32_t> d_iters[2];
+    PinnedArray<double> h_states[2]; PinnedArray<int32_t> h_iters[2];
+    FrameStage stage[2];
+    // Declared last, so destroyed first: phovo_destroy synchronises a slot's stream, one of setup_stream, and the
+    // slot's buffers are views of the arena.
+    std::vector<ContextPtr> slots;
+  } waves;
+
+  // warpImage (phovo_batch_warp_image, phovo_warp_image): splat keys of one chunk of pairs (zero between calls while
+  // keys_clean), Rt of the pairs, per-pair summaries, device copies of host outputs of one chunk
+  struct Warp {
+    DeviceArray<uint32_t> keys; bool keys_clean = false;
+    DeviceArray<double> rts;
+    DeviceArray<int32_t> landed;
+    DeviceArray<int64_t> sum;
+    DeviceArray<uint8_t> warped, diff;
+  } warp;
+
+  // normal equations at given states (phovo_batch_eval_normal_equations): winner keys (zero between calls while
+  // keys_clean) and validity of one chunk, its level records and tile partials; states, poses and results of every pair
+  struct Eval {
+    DeviceArray<uint32_t> keys; bool keys_clean = false;
+    DeviceArray<uint8_t> valid, store;
+    DeviceArray<double> partials, states;
+    DeviceArray<PoseDev> poses;
+    DeviceArray<double> out;                           // [P][21] H, [P][6] g, [P] cost
+    DeviceArray<int32_t> nvalid;
+  } eval;
+
+  // device copies of one chunk of host frames, for warpImage and the normal equations alike
+  FrameStage chunk_frames;
+};
 
 void phovo_batch_release(phovo_ctx* ctx) {
-  phovo_batch_state* b = ctx->batch;
-  if (!b) return;
-  cudaFree(b->next_pair);
-  cudaFree(b->store); cudaFree(b->states); cudaFree(b->iters); cudaFree(b->init); cudaFree(b->log); cudaFree(b->log_counts);
-  for (int s = 0; s < 2; ++s) {
-    cudaFree(b->stage_g0[s]); cudaFree(b->stage_g1[s]); cudaFree(b->stage_d[s]);
-    if (b->ev_copied[s]) cudaEventDestroy(b->ev_copied[s]);
-    if (b->ev_consumed[s]) cudaEventDestroy(b->ev_consumed[s]);
-  }
-  if (b->copy_stream) cudaStreamDestroy(b->copy_stream);
-  cudaFreeHost(b->h_states_pinned); cudaFreeHost(b->h_iters_pinned);
-  for (phovo_ctx* c : b->pool) phovo_destroy(c);
-  for (phovo_ctx* c : b->slots) phovo_destroy(c);      // (their streams are the setup streams below: not owned)
-  for (int t = 0; t < kWaveSetupThreads; ++t) {
-    if (b->setup_stream[t]) cudaStreamDestroy(b->setup_stream[t]);
-    if (b->ev_setup[t]) cudaEventDestroy(b->ev_setup[t]);
-  }
-  for (int h = 0; h < 2; ++h) {
-    if (b->align_stream[h]) cudaStreamDestroy(b->align_stream[h]);
-    if (b->ev_wave_done[h]) cudaEventDestroy(b->ev_wave_done[h]);
-    if (b->ev_wave_in[h]) cudaEventDestroy(b->ev_wave_in[h]);
-    cudaFree(b->d_wave_init[h]); cudaFree(b->d_wave_states[h]); cudaFree(b->d_wave_iters[h]);
-    cudaFreeHost(b->h_wave_states[h]); cudaFreeHost(b->h_wave_iters[h]);
-    cudaFree(b->wave_g0[h]); cudaFree(b->wave_g1[h]); cudaFree(b->wave_d0[h]); cudaFree(b->wave_d1[h]);
-  }
-  cudaFree(b->d_slot_args);
-  cudaFree(b->arena);
-  cudaFree(b->warp_keys); cudaFree(b->warp_rts); cudaFree(b->warp_landed); cudaFree(b->warp_sum); cudaFree(b->warp_depth);
-  for (int k = 0; k < 4; ++k) cudaFree(b->warp_io[k]);
-  cudaFree(b->eval_keys); cudaFree(b->eval_valid); cudaFree(b->eval_store); cudaFree(b->eval_partials);
-  cudaFree(b->eval_states); cudaFree(b->eval_poses); cudaFree(b->eval_out); cudaFree(b->eval_nvalid);
-  delete b;
+  delete ctx->batch;
   ctx->batch = nullptr;
 }
 
 static int get_state(phovo_ctx* ctx, phovo_batch_state** out) {
   if (!ctx->batch) {
-    ctx->batch = new phovo_batch_state();
+    std::unique_ptr<phovo_batch_state> b(new phovo_batch_state());
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, ctx->device));
-    ctx->batch->sm_count = prop.multiProcessorCount;
-    ctx->batch->l2_bytes = prop.l2CacheSize;
-    CK(cudaStreamCreateWithFlags(&ctx->batch->copy_stream, cudaStreamNonBlocking));
-    CK(cudaMalloc((void**)&ctx->batch->next_pair, sizeof(unsigned int) * PHOVO_MAX_LEVELS));
+    b->sm_count = prop.multiProcessorCount;
+    b->l2_bytes = prop.l2CacheSize;
+    CK(create_stream(b->res.copy_stream));
+    CK(b->res.next_pair.ensure(PHOVO_MAX_LEVELS));
     for (int s = 0; s < 2; ++s) {
-      CK(cudaEventCreateWithFlags(&ctx->batch->ev_copied[s], cudaEventDisableTiming));
-      CK(cudaEventCreateWithFlags(&ctx->batch->ev_consumed[s], cudaEventDisableTiming));
+      CK(create_event(b->res.ev_copied[s], cudaEventDisableTiming));
+      CK(create_event(b->res.ev_consumed[s], cudaEventDisableTiming));
     }
+    ctx->batch = b.release();
   }
   *out = ctx->batch;
   return PHOVO_OK;
-}
-
-static void level_size(int rows, int cols, int level, int* orows, int* ocols) {
-  const double f = ldexp(1.0, -level);
-  *orows = level == 0 ? rows : (int)lrint(rows * f);
-  *ocols = level == 0 ? cols : (int)lrint(cols * f);
 }
 
 // Active level `a` of bp = pyramid level `level` of a rows x cols frame under the context's config: size, record
@@ -182,11 +179,8 @@ static int fill_level(phovo_ctx* ctx, int rows, int cols, int level, int a, Batc
   bp->off_I0[a] = *off; *off += n16;
   bp->off_I1[a] = *off; *off += n16;
   bp->off_D32[a] = *off; *off += ((unsigned long long)n * 4 + 15) & ~15ull;
-  // CPhotoconsistencyOdometryAnalytic.h:203-209
-  const double scaleFactor = 1.0 / pow(2, level);
-  bp->fx[a] = ctx->K[0] * scaleFactor; bp->fy[a] = ctx->K[4] * scaleFactor;
-  bp->ox[a] = ctx->K[2] * scaleFactor; bp->oy[a] = ctx->K[5] * scaleFactor;
-  bp->inv_fx[a] = 1.f / bp->fx[a]; bp->inv_fy[a] = 1.f / bp->fy[a];
+  const WarpIntrinsics I = scaled_intrinsics(ctx->K, level);
+  bp->fx[a] = I.fx; bp->fy[a] = I.fy; bp->ox[a] = I.ox; bp->oy[a] = I.oy; bp->inv_fx[a] = I.inv_fx; bp->inv_fy[a] = I.inv_fy;
   bp->lambda[a] = ctx->cfg.lambda_step[level]; bp->min_grad[a] = ctx->cfg.min_gradient_norm[level];
   bp->grad_k[a] = ctx->cfg.grad_scale[level] / 1020.0;
   return PHOVO_OK;
@@ -267,19 +261,20 @@ static int run_device(phovo_ctx* ctx, phovo_batch_state* b, const BatchParams& b
     else CK(cudaMemsetAsync(states, 0, sizeof(double) * 6 * (size_t)bp.num_pairs, stream));
     return PHOVO_OK;
   }
-  if (!b->prepared_smem) {
+  auto& r = b->res;
+  if (!r.prepared_smem) {
     CK(batch_align_prepare());
-    b->prepared_smem = 1;
+    r.prepared_smem = 1;
   }
-  const int src = depth_type == PHOVO_DEPTH_F64 ? SRC_F64 : depth_type == PHOVO_DEPTH_F32 ? SRC_F32 : SRC_U16;
-  if (!b->ev_k[0]) for (int i = 0; i < 3; ++i) CK(cudaEventCreate(&b->ev_k[i]));
-  CK(cudaEventRecord(b->ev_k[0], stream));
-  ctx->launches += launch_batch_pyramid(stream, bp, g0, d0, src, depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0, g1, store);
-  CK(cudaEventRecord(b->ev_k[1], stream));
-  CK(cudaMemsetAsync(b->next_pair, 0, sizeof(unsigned int) * PHOVO_MAX_LEVELS, stream));
-  ctx->launches += launch_batch_align(stream, bp, b->sm_count, store, init, states, iters, log, log_counts, b->next_pair);
-  CK(cudaEventRecord(b->ev_k[2], stream));
-  b->timed = true;
+  for (int i = 0; i < 3; ++i)
+    if (!r.ev_k[i]) CK(create_event(r.ev_k[i]));
+  CK(cudaEventRecord(r.ev_k[0].get(), stream));
+  ctx->launches += launch_batch_pyramid(stream, bp, g0, d0, src_type_of_depth(depth_type), depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0, g1, store);
+  CK(cudaEventRecord(r.ev_k[1].get(), stream));
+  CK(cudaMemsetAsync(r.next_pair.get(), 0, sizeof(unsigned int) * PHOVO_MAX_LEVELS, stream));
+  ctx->launches += launch_batch_align(stream, bp, b->sm_count, store, init, states, iters, log, log_counts, r.next_pair.get());
+  CK(cudaEventRecord(r.ev_k[2].get(), stream));
+  r.timed = true;
   CK(cudaGetLastError());
   return PHOVO_OK;
 }
@@ -291,18 +286,17 @@ extern "C" int phovo_batch_get_last_h2d_bytes(const phovo_ctx* ctx, unsigned lon
 }
 
 extern "C" int phovo_batch_get_kernel_times(phovo_ctx* ctx, float* pyramid_ms, float* align_ms) {
-  if (!ctx || !ctx->batch || !ctx->batch->timed) return PHOVO_E_INVALID;
+  if (!ctx || !ctx->batch || !ctx->batch->res.timed) return PHOVO_E_INVALID;
   CK(cudaSetDevice(ctx->device));
-  CK(cudaEventSynchronize(ctx->batch->ev_k[2]));
+  const Event* ev = ctx->batch->res.ev_k;
+  CK(cudaEventSynchronize(ev[2].get()));
   float a = 0, c = 0;
-  CK(cudaEventElapsedTime(&a, ctx->batch->ev_k[0], ctx->batch->ev_k[1]));
-  CK(cudaEventElapsedTime(&c, ctx->batch->ev_k[1], ctx->batch->ev_k[2]));
+  CK(cudaEventElapsedTime(&a, ev[0].get(), ev[1].get()));
+  CK(cudaEventElapsedTime(&c, ev[1].get(), ev[2].get()));
   if (pyramid_ms) *pyramid_ms = a;
   if (align_ms) *align_ms = c;
   return PHOVO_OK;
 }
-
-static size_t depth_elt(int t) { return t == PHOVO_DEPTH_F64 ? 8 : t == PHOVO_DEPTH_F32 ? 4 : 2; }
 
 extern "C" int phovo_batch_set_record_stats(phovo_ctx* ctx, int enable) {
   if (!ctx) return PHOVO_E_INVALID;
@@ -335,8 +329,8 @@ static int prepare_log(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int*
   int total = 0;
   for (int l = 0; l < ctx->cfg.num_levels; ++l) total += ctx->cfg.max_num_iterations[l];
   if (total < 1) total = 1;
-  CK(ensure(&b->log, &b->log_cap_entries, (size_t)num_pairs * total));
-  CK(ensure(&b->log_counts, &b->log_counts_cap, (size_t)num_pairs));
+  CK(b->res.log.ensure((size_t)num_pairs * total));
+  CK(b->res.log_counts.ensure((size_t)num_pairs));
   b->log_per_pair = total;
   *log_cap = total;
   return PHOVO_OK;
@@ -358,12 +352,6 @@ static int pool_contexts() {
   return v >= 1 && v <= kPoolContextsMax ? v : kPoolContexts;
 }
 
-static bool host_readable(const void* p) {
-  cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return true; }
-  return a.type != cudaMemoryTypeDevice;
-}
-
 static int batch_general(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int rows, int cols, const uint8_t* gray0,
                          const void* depth0, int depth_type, double depth_scale, const uint8_t* gray1, const void* depth1,
                          const double* initial_states, double* states, int32_t* iterations) {
@@ -377,7 +365,7 @@ static int batch_general(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, in
   while ((int)b->pool.size() < workers) {
     phovo_ctx* c = nullptr;
     if (phovo_create(ctx->device, &c) != PHOVO_OK) return ctx->fail(PHOVO_E_CUDA, std::string("batch pool: ") + phovo_last_error(nullptr));
-    b->pool.push_back(c);
+    b->pool.emplace_back(c);
   }
   std::vector<double> init_host;
   if (initial_states && !host_readable(initial_states)) {
@@ -385,7 +373,7 @@ static int batch_general(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, in
     CK(cudaMemcpy(init_host.data(), initial_states, sizeof(double) * init_host.size(), cudaMemcpyDeviceToHost));
     initial_states = init_host.data();
   }
-  const size_t frame = (size_t)rows * cols, delt = depth_type == PHOVO_DEPTH_F64 ? 8 : depth_type == PHOVO_DEPTH_F32 ? 4 : 2;
+  const size_t frame = (size_t)rows * cols, delt = depth_elt(depth_type);
   // per-pair per-iteration stats (phovo_batch_set_record_stats): the children's logs, kept in the host mirrors
   int log_per_pair = 0;
   if (b->record_stats) {
@@ -434,12 +422,12 @@ static int batch_general(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, in
     }
   };
   std::vector<std::thread> threads;
-  for (int w = 1; w < workers; ++w) threads.emplace_back(work, b->pool[w]);
-  work(b->pool[0]);
+  for (int w = 1; w < workers; ++w) threads.emplace_back(work, b->pool[w].get());
+  work(b->pool[0].get());
   for (auto& t : threads) t.join();
   for (int w = 0; w < workers; ++w) ctx->launches += b->pool[w]->launches, b->pool[w]->launches = 0;
   b->last_pairs = log_per_pair ? num_pairs : 0; b->log_per_pair = log_per_pair; b->log_fetched = log_per_pair > 0;
-  b->last_h2d_bytes = 0; b->timed = false; b->last_path = 2;
+  b->last_h2d_bytes = 0; b->res.timed = false; b->last_path = 2;
   if (first_rc.load() != PHOVO_OK) return ctx->fail(first_rc.load(), "batch pool: " + message);
   return PHOVO_OK;
 }
@@ -459,74 +447,63 @@ static int batch_general(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, in
 static int wave_slots_per_half(const phovo_batch_state* b) { return PHOVO_SLOT_MINB * std::max(1, b->sm_count); }   // CTAs of k_align_slots resident per SM
 
 static int wave_resources(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int rows, int cols, int* half_out) {
-  for (int t = 0; t < kWaveSetupThreads; ++t)
-    if (!b->setup_stream[t]) {
-      CK(cudaStreamCreateWithFlags(&b->setup_stream[t], cudaStreamNonBlocking));
-      CK(cudaEventCreateWithFlags(&b->ev_setup[t], cudaEventDisableTiming));
-    }
-  for (int h = 0; h < 2; ++h)
-    if (!b->align_stream[h]) {
-      CK(cudaStreamCreateWithFlags(&b->align_stream[h], cudaStreamNonBlocking));
-      CK(cudaEventCreateWithFlags(&b->ev_wave_done[h], cudaEventDisableTiming));
-      CK(cudaEventCreateWithFlags(&b->ev_wave_in[h], cudaEventDisableTiming));
-    }
+  auto& w = b->waves;
+  for (int t = 0; t < kWaveSetupThreads; ++t) {
+    if (!w.setup_stream[t]) CK(create_stream(w.setup_stream[t]));
+    if (!w.ev_setup[t]) CK(create_event(w.ev_setup[t], cudaEventDisableTiming));
+  }
+  for (int h = 0; h < 2; ++h) {
+    if (!w.align_stream[h]) CK(create_stream(w.align_stream[h]));
+    if (!w.ev_wave_done[h]) CK(create_event(w.ev_wave_done[h], cudaEventDisableTiming));
+    if (!w.ev_wave_in[h]) CK(create_event(w.ev_wave_in[h], cudaEventDisableTiming));
+  }
   auto add_slots = [&](int want) -> int {
-    while ((int)b->slots.size() < want) {
+    while ((int)w.slots.size() < want) {
       phovo_ctx* c = nullptr;
       if (phovo_internal_create_slot(ctx->device, &c) != PHOVO_OK) return ctx->fail(PHOVO_E_CUDA, std::string("batch slots: ") + phovo_last_error(nullptr));
       c->defer_device_input_drain = true;   // the wave's inputs outlive its kernels (batch_waves waits for the wave before they go)
-      b->slots.push_back(c);
+      w.slots.emplace_back(c);
     }
     return PHOVO_OK;
   };
   int rc = add_slots(1);
   if (rc) return rc;
   // ---- bytes per slot under this configuration and frame size ----
-  phovo_ctx* c0 = b->slots[0];
+  phovo_ctx* c0 = w.slots[0].get();
   if (memcmp(&c0->cfg, &ctx->cfg, sizeof(phovo_config)) != 0 && (rc = phovo_set_config(c0, &ctx->cfg))) return ctx->fail(rc, phovo_last_error(c0));
   const size_t need = phovo_internal_slot_bytes(c0, rows, cols);
   // ---- slots per half: the CTAs of k_align_slots one wave keeps resident -- fewer if two halves of them would take more
   // than half of the device memory that is free (counting what the arena already holds) ----
   size_t free_b = 0, total_b = 0;
   CK(cudaMemGetInfo(&free_b, &total_b));
-  size_t budget = (free_b + b->arena_cap) / 2;
+  size_t budget = (free_b + w.arena.capacity()) / 2;
   if (const char* e = getenv("PHOVO_WAVE_BUDGET_MB")) budget = std::min(budget, (size_t)std::max(1LL, atoll(e)) << 20);   // test hook
   int half = wave_slots_per_half(b);
   if ((size_t)2 * half * need > budget) half = (int)std::max<size_t>(1, budget / need / 2);
   const int want = num_pairs > half ? 2 * half : num_pairs;
   if ((rc = add_slots(want))) return rc;
   // ---- the arena: ONE allocation, slot s at s * slot_bytes; laid out again whenever configuration, frame size or slot count change ----
-  const bool same = want <= b->arena_slots && half == b->wave_half && need == b->slot_bytes && rows == b->arena_rows && cols == b->arena_cols &&
-                    memcmp(&b->arena_cfg, &ctx->cfg, sizeof(phovo_config)) == 0;
+  const bool same = want <= w.arena_slots && half == w.wave_half && need == w.slot_bytes && rows == w.arena_rows && cols == w.arena_cols &&
+                    memcmp(&w.arena_cfg, &ctx->cfg, sizeof(phovo_config)) == 0;
   if (!same) {
     CK(cudaDeviceSynchronize());                       // nothing of an earlier call is still running on the old layout
-    const size_t total = need * (size_t)want;
-    if (total > b->arena_cap) {
-      cudaFree(b->arena); b->arena = nullptr; b->arena_cap = 0;
-      CK(cudaMalloc((void**)&b->arena, total));
-      b->arena_cap = total;
+    CK(w.arena.ensure(need * (size_t)want));
+    for (size_t s = 0; s < w.slots.size(); ++s) {
+      if ((int)s < want) w.slots[s]->arena_reset(w.arena.get() + s * need, need);
+      else w.slots[s]->arena_reset(nullptr, 0);       // not part of this layout (never used until the next one)
     }
-    for (size_t s = 0; s < b->slots.size(); ++s) {
-      if ((int)s < want) b->slots[s]->arena_reset(b->arena + s * need, need);
-      else b->slots[s]->arena_reset(nullptr, 0);       // not part of this layout (never used until the next one)
-    }
-    b->slot_bytes = need; b->arena_rows = rows; b->arena_cols = cols; b->arena_cfg = ctx->cfg; b->arena_slots = want; b->wave_half = half;
-    for (auto& a : b->h_slot_args) memset(&a, 0, sizeof(a));
+    w.slot_bytes = need; w.arena_rows = rows; w.arena_cols = cols; w.arena_cfg = ctx->cfg; w.arena_slots = want; w.wave_half = half;
+    for (auto& a : w.h_slot_args) memset(&a, 0, sizeof(a));
   }
-  if (b->wave_cap < (size_t)half) {
-    for (int h = 0; h < 2; ++h) {
-      cudaFree(b->d_wave_init[h]); cudaFree(b->d_wave_states[h]); cudaFree(b->d_wave_iters[h]);
-      cudaFreeHost(b->h_wave_states[h]); cudaFreeHost(b->h_wave_iters[h]);
-      CK(cudaMalloc((void**)&b->d_wave_init[h], sizeof(double) * 6 * half));
-      CK(cudaMalloc((void**)&b->d_wave_states[h], sizeof(double) * 6 * half));
-      CK(cudaMalloc((void**)&b->d_wave_iters[h], sizeof(int32_t) * PHOVO_MAX_LEVELS * half));
-      CK(cudaMallocHost((void**)&b->h_wave_states[h], sizeof(double) * 6 * half));
-      CK(cudaMallocHost((void**)&b->h_wave_iters[h], sizeof(int32_t) * PHOVO_MAX_LEVELS * half));
-    }
-    b->wave_cap = half;
+  for (int h = 0; h < 2; ++h) {
+    CK(w.d_init[h].ensure((size_t)6 * half));
+    CK(w.d_states[h].ensure((size_t)6 * half));
+    CK(w.d_iters[h].ensure((size_t)PHOVO_MAX_LEVELS * half));
+    CK(w.h_states[h].ensure((size_t)6 * half));
+    CK(w.h_iters[h].ensure((size_t)PHOVO_MAX_LEVELS * half));
   }
-  CK(ensure(&b->d_slot_args, &b->slot_args_cap, (size_t)2 * half));
-  if (b->h_slot_args.size() < (size_t)2 * half) b->h_slot_args.resize((size_t)2 * half);
+  CK(w.d_slot_args.ensure((size_t)2 * half));
+  if (w.h_slot_args.size() < (size_t)2 * half) w.h_slot_args.resize((size_t)2 * half);
   *half_out = half;
   return PHOVO_OK;
 }
@@ -544,8 +521,10 @@ static int batch_waves(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int 
   int half = 0;
   int rc = wave_resources(ctx, b, num_pairs, rows, cols, &half);
   if (rc) return rc;
+  auto& w = b->waves;
   const int waves = (num_pairs + half - 1) / half;
-  const size_t frame = (size_t)rows * cols, delt = depth_type == PHOVO_DEPTH_F64 ? 8 : depth_type == PHOVO_DEPTH_F32 ? 4 : 2;
+  const size_t frame = (size_t)rows * cols, delt = depth_elt(depth_type);
+  const Frames in = {gray0, gray1, depth0, bi ? depth1 : nullptr};
   b->last_h2d_bytes = 0;
   const bool host_in = host_readable(gray0) || host_readable(depth0) || host_readable(gray1) || (bi && host_readable(depth1));
 
@@ -556,14 +535,14 @@ static int batch_waves(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int 
 
   struct Pending { int start = 0, n = 0; bool active = false; } pend[2];
   const bool trace = getenv("PHOVO_WAVE_TRACE") != nullptr;   // stderr: host set-up time and device align time per wave
-  cudaEvent_t tr0[2] = {nullptr, nullptr}, tr1[2] = {nullptr, nullptr};
-  if (trace) for (int h = 0; h < 2; ++h) { cudaEventCreate(&tr0[h]); cudaEventCreate(&tr1[h]); }
+  Event tr0[2], tr1[2];
+  if (trace) for (int h = 0; h < 2; ++h) { create_event(tr0[h]); create_event(tr1[h]); }
   auto harvest = [&](int h) -> int {
     if (!pend[h].active) return PHOVO_OK;
-    CK(cudaEventSynchronize(b->ev_wave_done[h]));
-    if (trace) { float ms = 0.f; cudaEventElapsedTime(&ms, tr0[h], tr1[h]); fprintf(stderr, "[wave] start %d n %d align %.3f ms\n", pend[h].start, pend[h].n, ms); }
-    if (states) memcpy(states + (size_t)pend[h].start * 6, b->h_wave_states[h], sizeof(double) * 6 * (size_t)pend[h].n);
-    if (iterations) memcpy(iterations + (size_t)pend[h].start * PHOVO_MAX_LEVELS, b->h_wave_iters[h], sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)pend[h].n);
+    CK(cudaEventSynchronize(w.ev_wave_done[h].get()));
+    if (trace) { float ms = 0.f; cudaEventElapsedTime(&ms, tr0[h].get(), tr1[h].get()); fprintf(stderr, "[wave] start %d n %d align %.3f ms\n", pend[h].start, pend[h].n, ms); }
+    if (states) memcpy(states + (size_t)pend[h].start * 6, w.h_states[h].get(), sizeof(double) * 6 * (size_t)pend[h].n);
+    if (iterations) memcpy(iterations + (size_t)pend[h].start * PHOVO_MAX_LEVELS, w.h_iters[h].get(), sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)pend[h].n);
     pend[h].active = false;
     return PHOVO_OK;
   };
@@ -572,24 +551,16 @@ static int batch_waves(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int 
     const int h = k & 1, start = k * half, n = std::min(half, num_pairs - start);
     if ((rc = harvest(h))) return rc;          // wave k - 2 used these slots (and these input buffers)
     // ---- inputs of the wave on the device ----
-    const uint8_t* g0 = gray0 + (size_t)start * frame; const uint8_t* g1 = gray1 + (size_t)start * frame;
-    const char* d0 = (const char*)depth0 + (size_t)start * frame * delt;
-    const char* d1 = bi ? (const char*)depth1 + (size_t)start * frame * delt : nullptr;
+    cudaStream_t as = w.align_stream[h].get();
+    Frames f;
+    CK(w.stage[h].stage(host_in, in, frame, delt, start, n, as, &f));
     if (host_in) {
-      const size_t nb = (size_t)n * frame;
-      CK(ensure(&b->wave_g0[h], &b->wave_g_cap[h], nb)); CK(ensure(&b->wave_g1[h], &b->wave_g1_cap[h], nb));
-      CK(ensure(&b->wave_d0[h], &b->wave_d0_cap[h], nb * delt));
-      if (bi) CK(ensure(&b->wave_d1[h], &b->wave_d1_cap[h], nb * delt));
-      cudaStream_t cs = b->align_stream[h];
-      CK(cudaMemcpyAsync(b->wave_g0[h], g0, nb, cudaMemcpyDefault, cs));
-      CK(cudaMemcpyAsync(b->wave_g1[h], g1, nb, cudaMemcpyDefault, cs));
-      CK(cudaMemcpyAsync(b->wave_d0[h], d0, nb * delt, cudaMemcpyDefault, cs));
-      if (bi) CK(cudaMemcpyAsync(b->wave_d1[h], d1, nb * delt, cudaMemcpyDefault, cs));
-      CK(cudaEventRecord(b->ev_wave_in[h], cs));
-      for (int t = 0; t < kWaveSetupThreads; ++t) CK(cudaStreamWaitEvent(b->setup_stream[t], b->ev_wave_in[h], 0));
-      g0 = b->wave_g0[h]; g1 = b->wave_g1[h]; d0 = b->wave_d0[h]; d1 = bi ? b->wave_d1[h] : nullptr;
-      b->last_h2d_bytes += nb * (2 + delt * (bi ? 2 : 1));
+      CK(cudaEventRecord(w.ev_wave_in[h].get(), as));
+      for (int t = 0; t < kWaveSetupThreads; ++t) CK(cudaStreamWaitEvent(w.setup_stream[t].get(), w.ev_wave_in[h].get(), 0));
+      b->last_h2d_bytes += (size_t)n * frame * (2 + delt * (bi ? 2 : 1));
     }
+    const uint8_t* g0 = f.gray0; const uint8_t* g1 = f.gray1;
+    const char* d0 = (const char*)f.depth0; const char* d1 = (const char*)f.depth1;
     // ---- pyramids of the wave's slots: kWaveSetupThreads host threads, each on its own stream ----
     const auto t_setup = std::chrono::steady_clock::now();
     std::atomic<int> first_rc(PHOVO_OK);
@@ -597,8 +568,8 @@ static int batch_waves(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int 
     auto work = [&](int t) {
       for (int s = t; s < n; s += kWaveSetupThreads) {
         if (first_rc.load() != PHOVO_OK) return;
-        phovo_ctx* c = b->slots[(size_t)h * half + s];
-        c->stream = b->setup_stream[t];      // not owned: this thread's stream
+        phovo_ctx* c = w.slots[(size_t)h * half + s].get();
+        c->stream = w.setup_stream[t].get();   // not owned: this thread's stream
         int r = PHOVO_OK;
         if (memcmp(&c->cfg, &ctx->cfg, sizeof(phovo_config)) != 0) r = phovo_set_config(c, &ctx->cfg);
         if (!r) r = phovo_set_intrinsics(c, ctx->K);
@@ -624,29 +595,28 @@ static int batch_waves(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int 
       return ctx->fail(first_rc.load(), "batch slots: " + message);
     }
     if (trace) fprintf(stderr, "[wave] start %d n %d host set-up %.3f ms\n", start, n, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_setup).count());
-    cudaStream_t as = b->align_stream[h];
     for (int t = 0; t < kWaveSetupThreads; ++t) {
-      CK(cudaEventRecord(b->ev_setup[t], b->setup_stream[t]));
-      CK(cudaStreamWaitEvent(as, b->ev_setup[t], 0));
+      CK(cudaEventRecord(w.ev_setup[t].get(), w.setup_stream[t].get()));
+      CK(cudaStreamWaitEvent(as, w.ev_setup[t].get(), 0));
     }
     // ---- slot table (the buffers of a slot stay where they are once allocated for a frame size) ----
     bool table_changed = false;
     for (int s = 0; s < n; ++s) {
-      phovo_ctx* c = b->slots[(size_t)h * half + s];
+      phovo_ctx* c = w.slots[(size_t)h * half + s].get();
       SlotArgs A;
       memset(&A, 0, sizeof(A));
       for (int l = 0; l < c->cfg.num_levels; ++l) A.P[l] = c->level_ptrs(l);
-      A.pose = c->d_pose; A.partials = c->partials;
-      SlotArgs& cached = b->h_slot_args[(size_t)h * half + s];
+      A.pose = c->d_pose.get(); A.partials = c->partials.get();
+      SlotArgs& cached = w.h_slot_args[(size_t)h * half + s];
       if (memcmp(&cached, &A, sizeof(A)) != 0) { cached = A; table_changed = true; }
       ctx->launches += c->launches; c->launches = 0;
     }
     if (table_changed) {
-      CK(cudaMemcpyAsync(b->d_slot_args + (size_t)h * half, b->h_slot_args.data() + (size_t)h * half, sizeof(SlotArgs) * (size_t)n, cudaMemcpyHostToDevice, as));
+      CK(cudaMemcpyAsync(w.d_slot_args.get() + (size_t)h * half, w.h_slot_args.data() + (size_t)h * half, sizeof(SlotArgs) * (size_t)n, cudaMemcpyHostToDevice, as));
       CK(cudaStreamSynchronize(as));   // pageable source: keep it simple, this happens once per frame size
     }
     if (!levels_known) {
-      const phovo_ctx* c0 = b->slots[(size_t)h * half];
+      const phovo_ctx* c0 = w.slots[(size_t)h * half].get();
       for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
         const int M = ctx->cfg.max_num_iterations[level];
         if (!(M > 0)) continue;
@@ -663,34 +633,34 @@ static int batch_waves(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int 
     // ---- one launch aligns the wave; results to pinned memory ----
     const double* d_init = nullptr;
     if (initial_states) {
-      CK(cudaMemcpyAsync(b->d_wave_init[h], initial_states + (size_t)start * 6, sizeof(double) * 6 * (size_t)n, cudaMemcpyDefault, as));
-      d_init = b->d_wave_init[h];
+      CK(cudaMemcpyAsync(w.d_init[h].get(), initial_states + (size_t)start * 6, sizeof(double) * 6 * (size_t)n, cudaMemcpyDefault, as));
+      d_init = w.d_init[h].get();
     }
-    if (trace) cudaEventRecord(tr0[h], as);
+    if (trace) cudaEventRecord(tr0[h].get(), as);
     // CTAs per pair: one when the wave fills the GPU; a small wave gives every pair a thread-block cluster (2, 4 or 8 CTAs,
     // cluster barriers) so that the SMs it would leave idle shorten the wave instead
     int cluster = 1;
     for (int c = 8; c > 1; c >>= 1)
       if (n * c <= PHOVO_SLOT_MINB * b->sm_count) { cluster = c; break; }
     if (const char* e = getenv("PHOVO_WAVE_CLUSTER")) { const int v = atoi(e); if (v == 1 || v == 2 || v == 4 || v == 8) cluster = v; }   // experiment hook
-    int launched = launch_align_slots(as, ctx->cfg.mode, LS, b->d_slot_args + (size_t)h * half, n, d_init, cluster);
-    if (launched < 0 && cluster > 1) { cudaGetLastError(); launched = launch_align_slots(as, ctx->cfg.mode, LS, b->d_slot_args + (size_t)h * half, n, d_init, 1); }
+    SlotArgs* args = w.d_slot_args.get() + (size_t)h * half;
+    int launched = launch_align_slots(as, ctx->cfg.mode, LS, args, n, d_init, cluster);
+    if (launched < 0 && cluster > 1) { cudaGetLastError(); launched = launch_align_slots(as, ctx->cfg.mode, LS, args, n, d_init, 1); }
     if (launched < 0) return ctx->cuda_fail("k_align_slots", cudaGetLastError());
     ctx->launches += launched;
-    if (trace) cudaEventRecord(tr1[h], as);
-    ctx->launches += launch_gather_slots(as, b->d_slot_args + (size_t)h * half, n, b->d_wave_states[h], b->d_wave_iters[h]);
+    if (trace) cudaEventRecord(tr1[h].get(), as);
+    ctx->launches += launch_gather_slots(as, args, n, w.d_states[h].get(), w.d_iters[h].get());
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(b->h_wave_states[h], b->d_wave_states[h], sizeof(double) * 6 * (size_t)n, cudaMemcpyDeviceToHost, as));
-    CK(cudaMemcpyAsync(b->h_wave_iters[h], b->d_wave_iters[h], sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)n, cudaMemcpyDeviceToHost, as));
-    CK(cudaEventRecord(b->ev_wave_done[h], as));
+    CK(cudaMemcpyAsync(w.h_states[h].get(), w.d_states[h].get(), sizeof(double) * 6 * (size_t)n, cudaMemcpyDeviceToHost, as));
+    CK(cudaMemcpyAsync(w.h_iters[h].get(), w.d_iters[h].get(), sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)n, cudaMemcpyDeviceToHost, as));
+    CK(cudaEventRecord(w.ev_wave_done[h].get(), as));
     pend[h].start = start; pend[h].n = n; pend[h].active = true;
   }
   // in wave order: the older half first
   const int last = (waves - 1) & 1;
   if ((rc = harvest(1 - last))) return rc;
   if ((rc = harvest(last))) return rc;
-  if (trace) for (int h = 0; h < 2; ++h) { cudaEventDestroy(tr0[h]); cudaEventDestroy(tr1[h]); }
-  b->last_pairs = 0; b->log_per_pair = 0; b->log_fetched = false; b->timed = false; b->last_path = 3;
+  b->last_pairs = 0; b->log_per_pair = 0; b->log_fetched = false; b->res.timed = false; b->last_path = 3;
   return PHOVO_OK;
 }
 
@@ -742,15 +712,10 @@ extern "C" int phovo_batch_align_device(phovo_ctx* ctx, int num_pairs, int rows,
   }
   if (rc) return rc;
   b->last_path = 1;
-  CK(ensure(&b->store, &b->store_cap, (size_t)bp.record_bytes * num_pairs + kBatchStoreSlackBytes));
-  return run_device(ctx, b, bp, smem, ctx->stream, gray0, depth0, depth_type, depth_scale, gray1, b->store,
-                    initial_states, states, iters, log_cap ? b->log : nullptr, log_cap ? b->log_counts : nullptr);
-}
-
-static bool is_device_pointer(const void* p) {
-  cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-  return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+  auto& r = b->res;
+  CK(r.store.ensure((size_t)bp.record_bytes * num_pairs + kBatchStoreSlackBytes));
+  return run_device(ctx, b, bp, smem, ctx->stream, gray0, depth0, depth_type, depth_scale, gray1, r.store.get(),
+                    initial_states, states, iters, log_cap ? r.log.get() : nullptr, log_cap ? r.log_counts.get() : nullptr);
 }
 
 extern "C" int phovo_batch_align(phovo_ctx* ctx, int num_pairs, int rows, int cols, const uint8_t* gray0,
@@ -768,79 +733,75 @@ extern "C" int phovo_batch_align(phovo_ctx* ctx, int num_pairs, int rows, int co
     return batch_other(ctx, b, num_pairs, rows, cols, gray0, depth0, depth_type, depth_scale, gray1, nullptr, initial_states, states, iterations);
   if (rc) return rc;
   b->last_path = 1;
-  CK(ensure(&b->states, &b->states_cap, (size_t)num_pairs * 6));
-  CK(ensure(&b->iters, &b->iters_cap, (size_t)num_pairs * PHOVO_MAX_LEVELS));
-  CK(ensure(&b->store, &b->store_cap, (size_t)bp.record_bytes * num_pairs + kBatchStoreSlackBytes));
+  auto& r = b->res;
+  CK(r.states.ensure((size_t)num_pairs * 6));
+  CK(r.iters.ensure((size_t)num_pairs * PHOVO_MAX_LEVELS));
+  CK(r.store.ensure((size_t)bp.record_bytes * num_pairs + kBatchStoreSlackBytes));
   const double* d_init = nullptr;
   if (initial_states) {
-    CK(ensure(&b->init, &b->init_cap, (size_t)num_pairs * 6));
-    CK(cudaMemcpyAsync(b->init, initial_states, sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
-    d_init = b->init;
+    CK(r.init.ensure((size_t)num_pairs * 6));
+    CK(cudaMemcpyAsync(r.init.get(), initial_states, sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
+    d_init = r.init.get();
   }
-  if (b->h_out_cap < (size_t)num_pairs) {
-    cudaFreeHost(b->h_states_pinned); cudaFreeHost(b->h_iters_pinned);
-    b->h_states_pinned = nullptr; b->h_iters_pinned = nullptr; b->h_out_cap = 0;
-    CK(cudaMallocHost((void**)&b->h_states_pinned, sizeof(double) * 6 * (size_t)num_pairs));
-    CK(cudaMallocHost((void**)&b->h_iters_pinned, sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)num_pairs));
-    b->h_out_cap = num_pairs;
-  }
+  CK(r.h_states.ensure((size_t)num_pairs * 6));
+  CK(r.h_iters.ensure((size_t)num_pairs * PHOVO_MAX_LEVELS));
   const bool on_device = is_device_pointer(gray0) && is_device_pointer(depth0) && is_device_pointer(gray1);
   const size_t frame = (size_t)rows * cols, delt = depth_elt(depth_type);
+  phovo_iter_stats* log = log_cap ? r.log.get() : nullptr;
+  int32_t* log_counts = log_cap ? r.log_counts.get() : nullptr;
   if (on_device) {
-    rc = run_device(ctx, b, bp, smem, ctx->stream, gray0, depth0, depth_type, depth_scale, gray1, b->store, d_init,
-                    b->states, b->iters, log_cap ? b->log : nullptr, log_cap ? b->log_counts : nullptr);
+    rc = run_device(ctx, b, bp, smem, ctx->stream, gray0, depth0, depth_type, depth_scale, gray1, r.store.get(), d_init,
+                    r.states.get(), r.iters.get(), log, log_counts);
     if (rc) return rc;
   } else {
     // chunked, double-buffered upload: copies run on copy_stream, kernels on ctx->stream
     // a chunk is four waves of persistent CTAs: large enough to amortise the ragged tail of a
     // wave (pairs need different iteration counts), small enough to overlap with the next copy
     const int chunk = std::max(1, std::min(num_pairs, 4 * b->sm_count));
-    for (int s = 0; s < 2; ++s) {
-      CK(ensure(&b->stage_g0[s], &b->stage_cap_g[s], frame * chunk));
-      CK(ensure(&b->stage_g1[s], &b->stage_cap_g1[s], frame * chunk));
-      CK(ensure(&b->stage_d[s], &b->stage_cap_d[s], frame * chunk * delt));
-    }
-    CK(cudaMemsetAsync(b->iters, 0, sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)num_pairs, ctx->stream));
+    for (int s = 0; s < 2; ++s) CK(r.stage[s].reserve({gray0, gray1, depth0, nullptr}, chunk, frame, delt));
+    CK(cudaMemsetAsync(r.iters.get(), 0, sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)num_pairs, ctx->stream));
     int period, keep_begin, keep;
     row_compaction(ctx, rows, &period, &keep_begin, &keep);
     b->last_h2d_bytes = 0;
     int slot = 0, used[2] = {0, 0};
     for (int p0 = 0; p0 < num_pairs; p0 += chunk, slot ^= 1) {
       const int np = std::min(chunk, num_pairs - p0);
-      if (used[slot]) CK(cudaStreamWaitEvent(b->copy_stream, b->ev_consumed[slot], 0));
+      FrameStage& st = r.stage[slot];
+      cudaStream_t cs = r.copy_stream.get();
+      if (used[slot]) CK(cudaStreamWaitEvent(cs, r.ev_consumed[slot].get(), 0));
       if (period) {
         // one strided copy per image stack: `keep` of every `period` rows, frames are back to back
         const size_t groups = (size_t)(rows / period) * np;
         const size_t gw = (size_t)keep * cols, gp = (size_t)period * cols, go = (size_t)keep_begin * cols;
-        CK(cudaMemcpy2DAsync(b->stage_g0[slot], gw, gray0 + (size_t)p0 * frame + go, gp, gw, groups, cudaMemcpyHostToDevice, b->copy_stream));
-        CK(cudaMemcpy2DAsync(b->stage_g1[slot], gw, gray1 + (size_t)p0 * frame + go, gp, gw, groups, cudaMemcpyHostToDevice, b->copy_stream));
-        CK(cudaMemcpy2DAsync(b->stage_d[slot], gw * delt, (const char*)depth0 + ((size_t)p0 * frame + go) * delt, gp * delt, gw * delt, groups, cudaMemcpyHostToDevice, b->copy_stream));
+        CK(cudaMemcpy2DAsync(st.gray0.get(), gw, gray0 + (size_t)p0 * frame + go, gp, gw, groups, cudaMemcpyHostToDevice, cs));
+        CK(cudaMemcpy2DAsync(st.gray1.get(), gw, gray1 + (size_t)p0 * frame + go, gp, gw, groups, cudaMemcpyHostToDevice, cs));
+        CK(cudaMemcpy2DAsync(st.depth0.get(), gw * delt, (const char*)depth0 + ((size_t)p0 * frame + go) * delt, gp * delt, gw * delt, groups, cudaMemcpyHostToDevice, cs));
         b->last_h2d_bytes += groups * gw * (2 + delt);
       } else {
-        CK(cudaMemcpyAsync(b->stage_g0[slot], gray0 + (size_t)p0 * frame, frame * np, cudaMemcpyHostToDevice, b->copy_stream));
-        CK(cudaMemcpyAsync(b->stage_g1[slot], gray1 + (size_t)p0 * frame, frame * np, cudaMemcpyHostToDevice, b->copy_stream));
-        CK(cudaMemcpyAsync(b->stage_d[slot], (const char*)depth0 + (size_t)p0 * frame * delt, frame * np * delt, cudaMemcpyHostToDevice, b->copy_stream));
+        CK(cudaMemcpyAsync(st.gray0.get(), gray0 + (size_t)p0 * frame, frame * np, cudaMemcpyHostToDevice, cs));
+        CK(cudaMemcpyAsync(st.gray1.get(), gray1 + (size_t)p0 * frame, frame * np, cudaMemcpyHostToDevice, cs));
+        CK(cudaMemcpyAsync(st.depth0.get(), (const char*)depth0 + (size_t)p0 * frame * delt, frame * np * delt, cudaMemcpyHostToDevice, cs));
         b->last_h2d_bytes += (size_t)frame * np * (2 + delt);
       }
-      CK(cudaEventRecord(b->ev_copied[slot], b->copy_stream));
-      CK(cudaStreamWaitEvent(ctx->stream, b->ev_copied[slot], 0));
+      CK(cudaEventRecord(r.ev_copied[slot].get(), cs));
+      CK(cudaStreamWaitEvent(ctx->stream, r.ev_copied[slot].get(), 0));
       BatchParams cp = bp;
       cp.num_pairs = np;
       cp.src_period = period; cp.src_keep_begin = keep_begin; cp.src_keep = keep;
-      rc = run_device(ctx, b, cp, smem, ctx->stream, b->stage_g0[slot], b->stage_d[slot], depth_type, depth_scale, b->stage_g1[slot],
-                      b->store + (size_t)p0 * bp.record_bytes, d_init ? d_init + (size_t)p0 * 6 : nullptr,
-                      b->states + (size_t)p0 * 6, b->iters + (size_t)p0 * PHOVO_MAX_LEVELS,
-                      log_cap ? b->log + (size_t)p0 * log_cap : nullptr, log_cap ? b->log_counts + p0 : nullptr);
+      rc = run_device(ctx, b, cp, smem, ctx->stream, st.gray0.get(), st.depth0.get(), depth_type, depth_scale, st.gray1.get(),
+                      r.store.get() + (size_t)p0 * bp.record_bytes, d_init ? d_init + (size_t)p0 * 6 : nullptr,
+                      r.states.get() + (size_t)p0 * 6, r.iters.get() + (size_t)p0 * PHOVO_MAX_LEVELS,
+                      log ? log + (size_t)p0 * log_cap : nullptr, log_counts ? log_counts + p0 : nullptr);
       if (rc) return rc;
-      CK(cudaEventRecord(b->ev_consumed[slot], ctx->stream));
+      CK(cudaEventRecord(r.ev_consumed[slot].get(), ctx->stream));
       used[slot] = 1;
     }
   }
-  CK(cudaMemcpyAsync(b->h_states_pinned, b->states, sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(b->h_iters_pinned, b->iters, sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)num_pairs, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(r.h_states.get(), r.states.get(), sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(r.h_iters.get(), r.iters.get(), sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)num_pairs, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
-  if (states) memcpy(states, b->h_states_pinned, sizeof(double) * 6 * (size_t)num_pairs);
-  if (iterations) memcpy(iterations, b->h_iters_pinned, sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)num_pairs);
+  if (states) memcpy(states, r.h_states.get(), sizeof(double) * 6 * (size_t)num_pairs);
+  if (iterations) memcpy(iterations, r.h_iters.get(), sizeof(int32_t) * PHOVO_MAX_LEVELS * (size_t)num_pairs);
   return PHOVO_OK;
 }
 
@@ -853,8 +814,8 @@ static int fetch_log(const phovo_ctx* cctx) {
   CK(cudaStreamSynchronize(ctx->stream));
   b->h_log.resize((size_t)b->last_pairs * b->log_per_pair);
   b->h_log_counts.resize(b->last_pairs);
-  CK(cudaMemcpy(b->h_log.data(), b->log, sizeof(phovo_iter_stats) * b->h_log.size(), cudaMemcpyDeviceToHost));
-  CK(cudaMemcpy(b->h_log_counts.data(), b->log_counts, sizeof(int32_t) * b->last_pairs, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(b->h_log.data(), b->res.log.get(), sizeof(phovo_iter_stats) * b->h_log.size(), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(b->h_log_counts.data(), b->res.log_counts.get(), sizeof(int32_t) * b->last_pairs, cudaMemcpyDeviceToHost));
   b->log_fetched = true;
   return PHOVO_OK;
 }
@@ -916,24 +877,24 @@ int phovo_internal_warp_images(phovo_ctx* ctx, WarpImages W, int src_type, const
   if (rc) return rc;
   const size_t n = (size_t)W.rows * W.cols;
   const int chunk = warp_chunk_pairs(b, n, num_pairs);
-  if (b->warp_keys_cap < (size_t)chunk * n) {
-    CK(ensure(&b->warp_keys, &b->warp_keys_cap, (size_t)chunk * n));
-    b->warp_keys_clean = false;
-  }
+  auto& w = b->warp;
+  bool fresh;
+  CK(w.keys.ensure((size_t)chunk * n, &fresh));
+  if (fresh) w.keys_clean = false;
   const bool memset_each = (b->debug_flags & 16) != 0;
-  if (!b->warp_keys_clean && !memset_each) CK(cudaMemsetAsync(b->warp_keys, 0, b->warp_keys_cap * sizeof(uint32_t), ctx->stream));
-  b->warp_keys_clean = false;   // until every launch below has been enqueued
-  CK(ensure(&b->warp_rts, &b->warp_rts_cap, (size_t)num_pairs * 16));
-  CK(cudaMemcpyAsync(b->warp_rts, rts, sizeof(double) * 16 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
+  if (!w.keys_clean && !memset_each) CK(cudaMemsetAsync(w.keys.get(), 0, w.keys.capacity() * sizeof(uint32_t), ctx->stream));
+  w.keys_clean = false;   // until every launch below has been enqueued
+  CK(w.rts.ensure((size_t)num_pairs * 16));
+  CK(cudaMemcpyAsync(w.rts.get(), rts, sizeof(double) * 16 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
   for (int p0 = 0; p0 < num_pairs; p0 += chunk) {
     const int np = std::min(chunk, num_pairs - p0);
     WarpImages C = offset_pairs(W, p0);
-    C.rts = b->warp_rts + (size_t)p0 * 16;
-    if (memset_each) CK(cudaMemsetAsync(b->warp_keys, 0, (size_t)np * n * sizeof(uint32_t), ctx->stream));
-    ctx->launches += launch_warp_images(ctx->stream, C, src_type, I, np, b->warp_keys, !memset_each) + (memset_each ? 1 : 0);
+    C.rts = w.rts.get() + (size_t)p0 * 16;
+    if (memset_each) CK(cudaMemsetAsync(w.keys.get(), 0, (size_t)np * n * sizeof(uint32_t), ctx->stream));
+    ctx->launches += launch_warp_images(ctx->stream, C, src_type, I, np, w.keys.get(), !memset_each) + (memset_each ? 1 : 0);
     CK(cudaGetLastError());
   }
-  b->warp_keys_clean = !memset_each;
+  w.keys_clean = !memset_each;
   return PHOVO_OK;
 }
 
@@ -956,11 +917,12 @@ extern "C" int phovo_batch_warp_image(phovo_ctx* ctx, int num_pairs, int rows, i
   const uint8_t* target = diff || want_sum ? gray1 : nullptr;
   const bool in_dev = is_device_pointer(gray0) && is_device_pointer(depth0) && (!target || is_device_pointer(target));
   const bool w_host = warped && !is_device_pointer(warped), d_host = diff && !is_device_pointer(diff);
+  auto& w = b->warp;
   if (want_summary) {
-    CK(ensure(&b->warp_landed, &b->warp_landed_cap, (size_t)num_pairs));
-    CK(ensure(&b->warp_sum, &b->warp_sum_cap, (size_t)num_pairs));
-    CK(cudaMemsetAsync(b->warp_landed, 0, sizeof(int32_t) * num_pairs, ctx->stream));
-    CK(cudaMemsetAsync(b->warp_sum, 0, sizeof(int64_t) * num_pairs, ctx->stream));
+    CK(w.landed.ensure((size_t)num_pairs));
+    CK(w.sum.ensure((size_t)num_pairs));
+    CK(cudaMemsetAsync(w.landed.get(), 0, sizeof(int32_t) * num_pairs, ctx->stream));
+    CK(cudaMemsetAsync(w.sum.get(), 0, sizeof(int64_t) * num_pairs, ctx->stream));
   }
   WarpImages W;
   memset(&W, 0, sizeof(W));
@@ -971,45 +933,33 @@ extern "C" int phovo_batch_warp_image(phovo_ctx* ctx, int num_pairs, int rows, i
   W.target = target; W.target_step = cols; W.target_pair = n;
   W.warped = warped; W.warped_step = cols; W.warped_pair = n;
   W.diff = diff; W.diff_step = cols; W.diff_pair = n;
-  W.num_landed = want_summary ? b->warp_landed : nullptr;
-  W.sum_abs_diff = want_sum ? b->warp_sum : nullptr;
-  const double s = pow(2, level);                                  // BASE:89-94: K / 2^level
-  WarpIntrinsics I;
-  I.fx = K[0] / s; I.fy = K[4] / s; I.ox = K[2] / s; I.oy = K[5] / s;
-  I.inv_fx = 1.f / I.fx; I.inv_fy = 1.f / I.fy;                    // BASE:91-92
-  const int src = depth_type == PHOVO_DEPTH_F64 ? SRC_F64 : depth_type == PHOVO_DEPTH_F32 ? SRC_F32 : SRC_U16;
+  W.num_landed = want_summary ? w.landed.get() : nullptr;
+  W.sum_abs_diff = want_sum ? w.sum.get() : nullptr;
+  const WarpIntrinsics I = scaled_intrinsics(K, level);
+  const int src = src_type_of_depth(depth_type);
   if (in_dev && !w_host && !d_host) {
     if ((rc = phovo_internal_warp_images(ctx, W, src, I, num_pairs, rts))) return rc;
   } else {
     // host inputs (all rows: the warp reads every one) and host outputs go through device buffers of one chunk
     const int chunk = warp_chunk_pairs(b, n, num_pairs);
-    const size_t cn = (size_t)chunk * n;
-    if (!in_dev) {
-      CK(ensure(&b->warp_io[0], &b->warp_io_cap[0], cn));
-      CK(ensure(&b->warp_depth, &b->warp_depth_cap, cn * delt));
-      if (target) CK(ensure(&b->warp_io[1], &b->warp_io_cap[1], cn));
-    }
-    if (w_host) CK(ensure(&b->warp_io[2], &b->warp_io_cap[2], cn));
-    if (d_host) CK(ensure(&b->warp_io[3], &b->warp_io_cap[3], cn));
+    const Frames in = {gray0, target, depth0, nullptr};
+    if (w_host) CK(w.warped.ensure((size_t)chunk * n));
+    if (d_host) CK(w.diff.ensure((size_t)chunk * n));
     for (int p0 = 0; p0 < num_pairs; p0 += chunk) {
       const int np = std::min(chunk, num_pairs - p0);
       WarpImages C = offset_pairs(W, p0);
-      if (!in_dev) {
-        CK(cudaMemcpyAsync(b->warp_io[0], C.gray, n * np, cudaMemcpyDefault, ctx->stream));
-        CK(cudaMemcpyAsync(b->warp_depth, C.depth, n * np * delt, cudaMemcpyDefault, ctx->stream));
-        if (target) CK(cudaMemcpyAsync(b->warp_io[1], C.target, n * np, cudaMemcpyDefault, ctx->stream));
-        C.gray = b->warp_io[0]; C.depth = b->warp_depth;
-        if (target) C.target = b->warp_io[1];
-      }
-      if (w_host) C.warped = b->warp_io[2];
-      if (d_host) C.diff = b->warp_io[3];
+      Frames f;
+      CK(b->chunk_frames.stage(!in_dev, in, n, delt, p0, np, ctx->stream, &f));
+      C.gray = f.gray0; C.target = f.gray1; C.depth = f.depth0;
+      if (w_host) C.warped = w.warped.get();
+      if (d_host) C.diff = w.diff.get();
       if ((rc = phovo_internal_warp_images(ctx, C, src, I, np, rts + (size_t)p0 * 16))) return rc;
       if (w_host) CK(cudaMemcpyAsync(warped + (size_t)p0 * n, C.warped, n * np, cudaMemcpyDeviceToHost, ctx->stream));
       if (d_host) CK(cudaMemcpyAsync(diff + (size_t)p0 * n, C.diff, n * np, cudaMemcpyDeviceToHost, ctx->stream));
     }
   }
-  if (num_landed) CK(cudaMemcpyAsync(num_landed, b->warp_landed, sizeof(int32_t) * num_pairs, cudaMemcpyDefault, ctx->stream));
-  if (sum_abs_diff) CK(cudaMemcpyAsync(sum_abs_diff, b->warp_sum, sizeof(int64_t) * num_pairs, cudaMemcpyDefault, ctx->stream));
+  if (num_landed) CK(cudaMemcpyAsync(num_landed, w.landed.get(), sizeof(int32_t) * num_pairs, cudaMemcpyDefault, ctx->stream));
+  if (sum_abs_diff) CK(cudaMemcpyAsync(sum_abs_diff, w.sum.get(), sizeof(int64_t) * num_pairs, cudaMemcpyDefault, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return PHOVO_OK;
 }
@@ -1054,68 +1004,54 @@ extern "C" int phovo_batch_eval_normal_equations(phovo_ctx* ctx, int num_pairs, 
   const int ln = bp.lrows[0] * bp.lcols[0];
   EvalLevel E;
   memset(&E, 0, sizeof(E));
-  E.L.fx = bp.fx[0]; E.L.fy = bp.fy[0]; E.L.ox = bp.ox[0]; E.L.oy = bp.oy[0]; E.L.inv_fx = bp.inv_fx[0]; E.L.inv_fy = bp.inv_fy[0];
-  E.L.min_depth = bp.min_depth; E.L.max_depth = bp.max_depth;
-  E.L.lambda = bp.lambda[0]; E.L.min_grad_norm = bp.min_grad[0];
-  E.L.rows = bp.lrows[0]; E.L.cols = bp.lcols[0];
-  E.L.mode = bp.mode; E.L.level = level; E.L.row_begin = 0; E.L.row_end = E.L.rows;
+  E.L = make_level_params(ctx->cfg, ctx->K, level, bp.lrows[0], bp.lcols[0]);
   E.grad_k = bp.grad_k[0];
   E.tiles = (ln + kEvalTile - 1) / kEvalTile;
   E.depth_scale = depth_type == PHOVO_DEPTH_U16 ? depth_scale : 1.0;
   E.record_bytes = record_bytes; E.off_I0 = bp.off_I0[0]; E.off_I1 = bp.off_I1[0]; E.off_D0 = bp.off_D0[0];
-  const int src = depth_type == PHOVO_DEPTH_F64 ? SRC_F64 : depth_type == PHOVO_DEPTH_F32 ? SRC_F32 : SRC_U16;
+  const int src = src_type_of_depth(depth_type);
   const size_t delt = depth_elt(depth_type);
   const int chunk = eval_chunk_pairs(b, (size_t)ln, records ? record_bytes : 0, num_pairs);
   const size_t ck = (size_t)chunk * ln;
-  if (b->eval_keys_cap < ck) {
-    CK(ensure(&b->eval_keys, &b->eval_keys_cap, ck));
-    b->eval_keys_clean = false;
-  }
-  CK(ensure(&b->eval_valid, &b->eval_valid_cap, ck));
-  CK(ensure(&b->eval_partials, &b->eval_partials_cap, (size_t)chunk * E.tiles * PHOVO_ACC_STRIDE));
-  if (records) CK(ensure(&b->eval_store, &b->eval_store_cap, (size_t)chunk * record_bytes));
-  CK(ensure(&b->eval_states, &b->eval_states_cap, (size_t)num_pairs * 6));
-  CK(ensure(&b->eval_poses, &b->eval_poses_cap, (size_t)num_pairs));
-  CK(ensure(&b->eval_out, &b->eval_out_cap, (size_t)num_pairs * 28));
-  CK(ensure(&b->eval_nvalid, &b->eval_nvalid_cap, (size_t)num_pairs));
+  auto& v = b->eval;
+  bool fresh;
+  CK(v.keys.ensure(ck, &fresh));
+  if (fresh) v.keys_clean = false;
+  CK(v.valid.ensure(ck));
+  CK(v.partials.ensure((size_t)chunk * E.tiles * PHOVO_ACC_STRIDE));
+  if (records) CK(v.store.ensure((size_t)chunk * record_bytes));
+  CK(v.states.ensure((size_t)num_pairs * 6));
+  CK(v.poses.ensure((size_t)num_pairs));
+  CK(v.out.ensure((size_t)num_pairs * 28));
+  CK(v.nvalid.ensure((size_t)num_pairs));
   const bool in_dev = is_device_pointer(gray0) && is_device_pointer(depth0) && is_device_pointer(gray1);
-  if (!in_dev) {   // host frames go through device buffers of one chunk (every row: level 0 and the pyramid read them all)
-    CK(ensure(&b->warp_io[0], &b->warp_io_cap[0], (size_t)chunk * n));
-    CK(ensure(&b->warp_io[1], &b->warp_io_cap[1], (size_t)chunk * n));
-    CK(ensure(&b->warp_depth, &b->warp_depth_cap, (size_t)chunk * n * delt));
-  }
-  if (!b->eval_keys_clean) CK(cudaMemsetAsync(b->eval_keys, 0, b->eval_keys_cap * sizeof(uint32_t), ctx->stream));
-  b->eval_keys_clean = false;   // until every launch below has been enqueued
-  CK(cudaMemcpyAsync(b->eval_states, states, sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
-  ctx->launches += launch_eval_poses(ctx->stream, b->eval_states, num_pairs, b->eval_poses);
-  double* dH = b->eval_out; double* dg = dH + (size_t)num_pairs * 21; double* dcost = dg + (size_t)num_pairs * 6;
-  E.keys = b->eval_keys; E.valid = b->eval_valid; E.partials = b->eval_partials; E.store = b->eval_store;
+  const Frames in = {gray0, gray1, depth0, nullptr};
+  if (!v.keys_clean) CK(cudaMemsetAsync(v.keys.get(), 0, v.keys.capacity() * sizeof(uint32_t), ctx->stream));
+  v.keys_clean = false;   // until every launch below has been enqueued
+  CK(cudaMemcpyAsync(v.states.get(), states, sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
+  ctx->launches += launch_eval_poses(ctx->stream, v.states.get(), num_pairs, v.poses.get());
+  double* dH = v.out.get(); double* dg = dH + (size_t)num_pairs * 21; double* dcost = dg + (size_t)num_pairs * 6;
+  E.keys = v.keys.get(); E.valid = v.valid.get(); E.partials = v.partials.get(); E.store = v.store.get();
   for (int p0 = 0; p0 < num_pairs; p0 += chunk) {
     const int np = std::min(chunk, num_pairs - p0);
-    const uint8_t* c_g0 = gray0 + (size_t)p0 * n; const uint8_t* c_g1 = gray1 + (size_t)p0 * n;
-    const void* c_d = (const char*)depth0 + (size_t)p0 * n * delt;
-    if (!in_dev) {
-      CK(cudaMemcpyAsync(b->warp_io[0], c_g0, n * np, cudaMemcpyDefault, ctx->stream));
-      CK(cudaMemcpyAsync(b->warp_io[1], c_g1, n * np, cudaMemcpyDefault, ctx->stream));
-      CK(cudaMemcpyAsync(b->warp_depth, c_d, n * np * delt, cudaMemcpyDefault, ctx->stream));
-      c_g0 = b->warp_io[0]; c_g1 = b->warp_io[1]; c_d = b->warp_depth;
-    }
+    Frames f;
+    CK(b->chunk_frames.stage(!in_dev, in, n, delt, p0, np, ctx->stream, &f));   // host frames: every row (level 0 and the pyramid read them all)
     if (records) {
       bp.num_pairs = np;
-      ctx->launches += launch_batch_pyramid(ctx->stream, bp, c_g0, c_d, src, E.depth_scale, c_g1, b->eval_store);
+      ctx->launches += launch_batch_pyramid(ctx->stream, bp, f.gray0, f.depth0, src, E.depth_scale, f.gray1, v.store.get());
     } else {
-      E.gray0 = c_g0; E.gray1 = c_g1; E.depth = c_d;
+      E.gray0 = f.gray0; E.gray1 = f.gray1; E.depth = f.depth0;
     }
-    E.poses = b->eval_poses + p0;
+    E.poses = v.poses.get() + p0;
     ctx->launches += launch_eval_normal_equations(ctx->stream, E, src, records, np, dH + (size_t)p0 * 21, dg + (size_t)p0 * 6,
-                                                  dcost + p0, b->eval_nvalid + p0);
+                                                  dcost + p0, v.nvalid.get() + p0);
     CK(cudaGetLastError());
   }
-  b->eval_keys_clean = true;
+  v.keys_clean = true;
   if (H) CK(cudaMemcpyAsync(H, dH, sizeof(double) * 21 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
   if (g) CK(cudaMemcpyAsync(g, dg, sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
   if (cost) CK(cudaMemcpyAsync(cost, dcost, sizeof(double) * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
-  if (num_valid) CK(cudaMemcpyAsync(num_valid, b->eval_nvalid, sizeof(int32_t) * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
+  if (num_valid) CK(cudaMemcpyAsync(num_valid, v.nvalid.get(), sizeof(int32_t) * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return PHOVO_OK;
 }

@@ -4,18 +4,18 @@
 
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
-#include "phovo_internal.h"
-#include "phovo_kernels.h"
+#include "phovo_host.h"
 
 struct phovo_batch_state;  // phovo_batch.cu
 
 struct phovo_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
-  bool own_stream = false;
+  phovo::Stream own_stream;   // the stream phovo_create made; empty once phovo_set_stream names another (and for slots)
   std::string err, graph_error;
 
   phovo_config cfg;
@@ -30,36 +30,34 @@ struct phovo_ctx {
 
   // HBM layout (general path): per active level five dense row-major fp64 images -- bit-identical to the
   // reference's cv::Mat_<double> levels (fp32 storage makes ~15% of trajectories diverge, see DESIGN.md)
-  double* I0[PHOVO_MAX_LEVELS] = {nullptr};
-  double* D0[PHOVO_MAX_LEVELS] = {nullptr};
-  double* I1[PHOVO_MAX_LEVELS] = {nullptr};
-  double* Gx[PHOVO_MAX_LEVELS] = {nullptr};
-  double* Gy[PHOVO_MAX_LEVELS] = {nullptr};
-  size_t lcap[PHOVO_MAX_LEVELS][5] = {{0}};
+  phovo::DeviceArray<double> I0[PHOVO_MAX_LEVELS];
+  phovo::DeviceArray<double> D0[PHOVO_MAX_LEVELS];
+  phovo::DeviceArray<double> I1[PHOVO_MAX_LEVELS];
+  phovo::DeviceArray<double> Gx[PHOVO_MAX_LEVELS];
+  phovo::DeviceArray<double> Gy[PHOVO_MAX_LEVELS];
   // photometric + depth solver: target depth pyramid, Scharr of depth / max_depth, gain per level
-  double* D1[PHOVO_MAX_LEVELS] = {nullptr};
-  double* GxD[PHOVO_MAX_LEVELS] = {nullptr};
-  double* GyD[PHOVO_MAX_LEVELS] = {nullptr};
-  size_t bcap[PHOVO_MAX_LEVELS][3] = {{0}};
-  double* d_gain = nullptr;
+  phovo::DeviceArray<double> D1[PHOVO_MAX_LEVELS];
+  phovo::DeviceArray<double> GxD[PHOVO_MAX_LEVELS];
+  phovo::DeviceArray<double> GyD[PHOVO_MAX_LEVELS];
+  phovo::DeviceArray<double> d_gain;
   bool have_tgt_depth = false;
-  int* winner = nullptr; size_t winner_cap = 0;           // one int per pixel of the largest active level
-  unsigned char* valid = nullptr; size_t valid_cap = 0;   // one flag per pixel (K3a -> K3b)
-  double* scratch64[2] = {nullptr, nullptr}; size_t scratch_cap[2] = {0, 0};
-  double* partials = nullptr; size_t partials_cap = 0;    // [grid][32] per-block normal-equation partials
-  char* stage_gray[2] = {nullptr, nullptr}; size_t stage_gray_cap[2] = {0, 0};
-  char* stage_depth = nullptr; size_t stage_depth_cap = 0;
-  double* dump_res = nullptr; size_t dump_res_cap = 0;
-  double* dump_jac = nullptr; size_t dump_jac_cap = 0;
+  phovo::DeviceArray<int> winner;              // one int per pixel of the largest active level
+  phovo::DeviceArray<unsigned char> valid;     // one flag per pixel (K3a -> K3b)
+  phovo::DeviceArray<double> scratch64[2];
+  phovo::DeviceArray<double> partials;         // [grid][32] per-block normal-equation partials
+  phovo::DeviceArray<char> stage_gray[2];
+  phovo::DeviceArray<char> stage_depth;
+  phovo::DeviceArray<double> dump_res;
+  phovo::DeviceArray<double> dump_jac;
   // phovo_warp_image scratch (its keys belong to the batch state)
-  char* warp_io[3] = {nullptr, nullptr, nullptr}; size_t warp_io_cap[3] = {0, 0, 0};   // device copies of warped / target / diff for host callers
+  phovo::DeviceArray<char> warp_io[3];         // device copies of warped / target / diff for host callers
 
   // solver state
   double state[6] = {0};
-  PoseDev* d_pose = nullptr; PoseDev* h_pose = nullptr;
-  phovo_iter_stats* d_log = nullptr; phovo_iter_stats* h_log = nullptr; int log_cap = 0;
-  phovo_iter_stats* d_eval = nullptr; phovo_iter_stats* h_eval = nullptr;
-  double* d_state_in = nullptr; double* h_state_in = nullptr;
+  phovo::DeviceArray<PoseDev> d_pose; phovo::PinnedArray<PoseDev> h_pose;
+  phovo::DeviceArray<phovo_iter_stats> d_log; phovo::PinnedArray<phovo_iter_stats> h_log;
+  phovo::DeviceArray<phovo_iter_stats> d_eval; phovo::PinnedArray<phovo_iter_stats> h_eval;
+  phovo::DeviceArray<double> d_state_in; phovo::PinnedArray<double> h_state_in;
   std::vector<phovo_iter_stats> log;
 
   // CUDA graph of the whole Optimize()
@@ -72,19 +70,19 @@ struct phovo_ctx {
 
   // row sharding
   int shard_rank = 0, shard_world = 1, shard_level = -1;
-  double* d_shard = nullptr;
-  double* d_level_dmin = nullptr;          // [PHOVO_MAX_LEVELS] smallest valid depth per level of the current source frame
+  phovo::DeviceArray<double> d_shard;
+  phovo::DeviceArray<double> d_level_dmin;   // [PHOVO_MAX_LEVELS] smallest valid depth per level of the current source frame
   bool level_dmin_valid = false;
-  // fused peer-store exchange: own area (cudaMalloc, IPC-exported), peers' areas (IPC-opened)
-  phovo::ShardExchange* xchg_own = nullptr;
+  // fused peer-store exchange: own area (device memory, IPC-exported), peers' areas (IPC-opened)
+  phovo::DeviceArray<phovo::ShardExchange> xchg_own;
   phovo::ShardExchange* xchg_peer[8] = {nullptr};
   bool xchg_opened[8] = {false};
-  phovo::ShardExchange** xchg_peers_dev = nullptr;   // device copy of xchg_peer[]
+  phovo::DeviceArray<phovo::ShardExchange*> xchg_peers_dev;   // device copy of xchg_peer[]
   bool xchg_table_dirty = true;
   unsigned long long xchg_epoch = 0;
 
   // bookkeeping
-  cudaEvent_t ev_copy = nullptr; cudaEvent_t ev_time[4] = {nullptr, nullptr, nullptr, nullptr};
+  phovo::Event ev_copy, ev_time[4];
   bool h2d_pending = false, copy_event_armed = false, setup_timed = false;
   bool defer_device_input_drain = false; // batch slots: the owner of the context keeps device inputs alive and waits itself
   bool device_input_in_flight = false;   // a Set*Frame call was given a device pointer and its kernels are queued
@@ -102,6 +100,7 @@ struct phovo_ctx {
 
   int fail(int code, const std::string& what);
   int cuda_fail(const char* what, cudaError_t e);
+  int log_cap() const { return (int)std::min(d_log.capacity(), h_log.capacity()); }   // stats entries Optimize may write
   bool level_active(int l) const;
   LevelParams level_params(int level) const;
   phovo::LevelPtrs level_ptrs(int level) const;

@@ -16,6 +16,7 @@
 
 #include "phovo_device.cuh"
 #include "phovo_kernels.h"
+#include "phovo_lm.h"
 
 namespace phovo {
 namespace {
@@ -28,14 +29,19 @@ __global__ void k_fill_i32(int* p, int v, size_t n) {
   for (; i < n; i += stride) p[i] = v;
 }
 
+// state -> Pose -> PoseDev: the state and the rotation and trig values derived from it
+__device__ __forceinline__ void pose_set_state(PoseDev* d, const double s[6]) {
+  Pose P;
+  pose_from_state(s, P);
+  for (int k = 0; k < 6; ++k) d->state[k] = s[k];
+  pose_store(P, d);
+}
+
 __global__ void k_set_state(PoseDev* pose, const double* state_dev, int log_capacity, double s0, double s1, double s2, double s3, double s4, double s5) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   double s[6] = {s0, s1, s2, s3, s4, s5};
   if (state_dev) for (int k = 0; k < 6; ++k) s[k] = state_dev[k];
-  Pose P;
-  pose_from_state(s, P);
-  for (int k = 0; k < 6; ++k) pose->state[k] = s[k];
-  pose_store(P, pose);
+  pose_set_state(pose, s);
   pose->iteration = 0;
   pose->done = 0;
   pose->log_count = 0;
@@ -289,31 +295,52 @@ __device__ __forceinline__ void reduce_partials(const double* __restrict__ parti
   __syncthreads();
 }
 
-// The Gauss-Newton step and termination test of AN:538-549 / AN:376-392, single thread.
+// |g|, the quantity the termination test thresholds (AN:380)
+__device__ __forceinline__ double grad_norm(const double g[6]) {
+  double n2 = 0.;
+  for (int k = 0; k < 6; ++k) n2 = fma(g[k], g[k], n2);
+  return sqrt(n2);
+}
+
+// The fields of a stats entry that an evaluation's totals decide; iteration, accepted and the states are the caller's.
+__device__ __forceinline__ void entry_from_totals(phovo_iter_stats* e, int level, const double* totals) {
+  e->level = level; e->num_valid = (int)totals[28];
+  for (int k = 0; k < 21; ++k) e->H[k] = totals[k];
+  for (int k = 0; k < 6; ++k) e->g[k] = totals[21 + k];
+  e->grad_norm = grad_norm(totals + 21); e->cost = 0.5 * totals[27]; e->radius = 0.;
+}
+
+// The Gauss-Newton step and termination test of AN:538-549 / AN:376-392 for iteration `it` (0-based) of the level,
+// single thread: s_out from the totals at s_in.  Returns done.
+__device__ __forceinline__ int gn_update(const LevelParams& L, const double* totals, const double s_in[6], int it, double s_out[6]) {
+  double g[6], step[6], n2 = 0.;   // (n2 summed here, not by grad_norm after the solve: fewer spills in k_reduce_solve)
+  for (int k = 0; k < 6; ++k) { g[k] = totals[21 + k]; n2 = fma(g[k], g[k], n2); }
+  solve6_ldlt(totals, g, step);
+  for (int k = 0; k < 6; ++k) s_out[k] = s_in[k] - L.lambda * step[k];   // AN:539-540
+  return (it + 1 >= L.max_iters) || (sqrt(n2) < L.min_grad_norm);        // AN:383-392, 547
+}
+
+// The log entry of that iteration.  (The callers test whether to log after the step: testing before keeps the log
+// position live through the solve, which spills in k_reduce_solve.)
+__device__ __forceinline__ void gn_entry(phovo_iter_stats* e, const LevelParams& L, const double* totals, int it, const double s_in[6],
+                                         const double s_out[6]) {
+  entry_from_totals(e, L.level, totals);
+  e->iteration = it; e->accepted = 1;
+  for (int k = 0; k < 6; ++k) { e->state_in[k] = s_in[k]; e->state_out[k] = s_out[k]; }
+}
+
+// One Gauss-Newton iteration of the stream / graph drivers on the PoseDev in global memory.
 __device__ void gn_step(const LevelParams& L, PoseDev* pose, const double* totals, phovo_iter_stats* log,
                         unsigned long long cond_handle) {
-  double g[6], step[6], s_in[6], n2 = 0.;
-  for (int k = 0; k < 6; ++k) { g[k] = totals[21 + k]; n2 = fma(g[k], g[k], n2); s_in[k] = pose->state[k]; }
-  solve6_ldlt(totals, g, step);
-  double s_out[6];
-  for (int k = 0; k < 6; ++k) s_out[k] = s_in[k] - L.lambda * step[k];   // AN:539-540
-  const double gnorm = sqrt(n2);
-  const int it = pose->iteration + 1;                                     // AN:547
-  const int done = (it >= L.max_iters) || (gnorm < L.min_grad_norm);      // AN:383-392
-  if (log && pose->log_count < pose->log_capacity) {
-    phovo_iter_stats* e = log + pose->log_count;
-    e->level = L.level; e->iteration = it - 1; e->num_valid = (int)totals[28]; e->accepted = 1;
-    for (int k = 0; k < 21; ++k) e->H[k] = totals[k];
-    for (int k = 0; k < 6; ++k) { e->g[k] = g[k]; e->state_in[k] = s_in[k]; e->state_out[k] = s_out[k]; }
-    e->grad_norm = gnorm; e->cost = 0.5 * totals[27]; e->radius = 0.;
-  }
+  double s_in[6], s_out[6];
+  for (int k = 0; k < 6; ++k) s_in[k] = pose->state[k];
+  const int it = pose->iteration;
+  const int done = gn_update(L, totals, s_in, it, s_out);
+  if (log && pose->log_count < pose->log_capacity) gn_entry(log + pose->log_count, L, totals, it, s_in, s_out);
   pose->log_count += 1;
-  Pose P;
-  pose_from_state(s_out, P);
-  for (int k = 0; k < 6; ++k) pose->state[k] = s_out[k];
-  pose_store(P, pose);
-  pose->iteration = it;
-  pose->iters_per_level[L.level] = it;
+  pose_set_state(pose, s_out);
+  pose->iteration = it + 1;
+  pose->iters_per_level[L.level] = it + 1;
   pose->done = done;
   if (cond_handle) cudaGraphSetConditional((cudaGraphConditionalHandle)cond_handle, done ? 0u : 1u);
 }
@@ -334,11 +361,9 @@ __global__ void __launch_bounds__(1024) k_reduce_only(LevelParams L, const PoseD
   __shared__ double totals[32];
   reduce_partials(partials, grid, totals);
   if (threadIdx.x == 0) {
-    out->level = L.level; out->iteration = 0; out->num_valid = (int)totals[28]; out->accepted = 0;
-    double n2 = 0.;
-    for (int k = 0; k < 21; ++k) out->H[k] = totals[k];
-    for (int k = 0; k < 6; ++k) { out->g[k] = totals[21 + k]; n2 += totals[21 + k] * totals[21 + k]; out->state_in[k] = pose->state[k]; out->state_out[k] = pose->state[k]; }
-    out->grad_norm = sqrt(n2); out->cost = 0.5 * totals[27]; out->radius = 0.;
+    entry_from_totals(out, L.level, totals);
+    out->iteration = 0; out->accepted = 0;
+    for (int k = 0; k < 6; ++k) { out->state_in[k] = pose->state[k]; out->state_out[k] = pose->state[k]; }
   }
 }
 
@@ -410,34 +435,50 @@ __global__ void k_solve_from_buffer(LevelParams L, PoseDev* pose, const double* 
 // ---------------------------------------------------------------------------------------------
 constexpr int kCoopBlock = 256;
 
-// Jacobian row of a valid source pixel i (analytic modes): compact closed form of AN:243-342 with
-// the image gradient folded in (SURVEY appendix C).  Shared by the cooperative and the cluster kernel.
-template <int MODE>
-__device__ __forceinline__ void analytic_jacobian_core(const LevelParams& L, const Pose& T, double spsr, double spcr,
-                                                       int i, double d, double gx, double gy, double J[6]) {
+// Phase A of the analytic loops: whether source pixel i with depth d lands, and on which target slot t.
+// Estimate-then-verify (phovo_device.cuh): the exact reference arithmetic runs only for the pixels whose
+// estimate lies next to a rounding boundary (~2e-4 of them); the graph / stream drivers (k_winner) run it
+// for every pixel.
+__device__ __forceinline__ bool phase_a_target(const LevelParams& L, const Pose& T, const EstimateConst& E, int i, double d, int& t) {
   const int r = i / L.cols, c = i - r * L.cols;
-  const double px = ((double)c - L.ox) * d * L.inv_fx, py = ((double)r - L.oy) * d * L.inv_fy;
-  const double q0 = fma(T.R00, px, fma(T.R01, py, T.R02 * d));
-  const double q1 = fma(T.R10, px, fma(T.R11, py, T.R12 * d));
-  const double q2 = fma(T.R20, px, fma(T.R21, py, T.R22 * d));
-  const double iz = rcp_1ulp(q2 + T.z);
-  const double ga = gx * L.fx * iz, gb = gy * L.fy * iz;
-  const double A = MODE == 0 ? fma(px, T.x, q0) : q0 + T.x;   // AN:253 bug-compatible / Maxima-exact
-  const double B = q1 + T.y;
-  J[0] = ga;
-  J[1] = gb;
-  J[2] = -(fma(ga, A, gb * B) * iz);
-  J[3] = fma(gb, q0, -(ga * q1));
-  const double Zp = -fma(spsr, py, fma(spcr, d, T.cp * px));
-  J[4] = fma(q2, fma(ga, T.cy, gb * T.sy), Zp * J[2]);
-  const double Zr = fma(T.R22, py, -(T.R21 * d));
-  J[5] = fma(ga, fma(T.R02, py, -(T.R01 * d)), fma(gb, fma(T.R12, py, -(T.R11 * d)), Zr * J[2]));
+  const bool dep = (L.min_depth < d) & (d < L.max_depth);                  // strict bounds, AN:279-280
+  int tj, ti;
+  const bool unc = estimate_target(L, T, E, r, c, d, tj, ti);
+  bool ok = dep & ((unsigned)tj < (unsigned)L.cols) & ((unsigned)ti < (unsigned)L.rows);
+  t = L.cols * ti + tj;
+  if (dep & unc) {
+    Warped w;
+    ok = warp_pixel<false>(L, T, r, c, d, w);
+    t = w.t;
+  }
+  return ok;
 }
 
-template <int MODE>
-__device__ __forceinline__ void analytic_jacobian_row(const LevelParams& L, const LevelPtrs& P, const Pose& T, double spsr, double spcr,
-                                                      int i, double J[6]) {
-  analytic_jacobian_core<MODE>(L, T, spsr, spcr, i, __ldg(P.D0 + i), __ldg(P.Gx + i), __ldg(P.Gy + i), J);
+// Every CTA of a persistent loop: the fixed-order sum of all `nblk` CTAs' partials into s_tot (warp g of 8
+// takes blocks g, g+8, ..., then the eight warp sums in order).
+__device__ __forceinline__ void sum_all_partials(const double* partials, int nblk, double* smem, double* s_tot) {
+  const int tid = threadIdx.x, v = tid & 31, g = tid >> 5;
+  double s = 0.;
+  for (int b = g; b < nblk; b += kCoopBlock / 32) s += __ldcg(partials + (size_t)b * PHOVO_ACC_STRIDE + v);
+  smem[g * PHOVO_ACC_STRIDE + v] = s;
+  __syncthreads();
+  if (tid < 32) {
+    double t = 0.;
+#pragma unroll
+    for (int k = 0; k < kCoopBlock / 32; ++k) t += smem[k * PHOVO_ACC_STRIDE + tid];
+    s_tot[tid] = t;
+  }
+  __syncthreads();
+}
+
+// End of a level in a persistent loop (one thread of the pair's first CTA): the pose goes out with the level's
+// iteration count and log position.
+__device__ __forceinline__ void finish_level(PoseDev* pose, PoseDev& s_pose, int level, int iterations, int log_count) {
+  s_pose.iteration = iterations;
+  s_pose.iters_per_level[level] = iterations;
+  s_pose.done = 1;
+  s_pose.log_count = log_count;
+  *pose = s_pose;
 }
 
 // Row-sharded use (one 8K pair over several GPUs, SURVEY 8(e)): `S.world` > 1.  Every rank runs phase A over the
@@ -508,9 +549,7 @@ __device__ __forceinline__ void level_loop(const LevelParams& L, const LevelPtrs
   for (; it < L.max_iters; ++it) {
     Pose T;
     pose_load(&s_pose, T);
-    // ---- phase A: winner map + validity.  Estimate-then-verify (phovo_device.cuh): the exact
-    // reference arithmetic runs only for the pixels whose estimate lies next to a rounding boundary
-    // (~2e-4 of them); the graph / stream drivers (k_winner) run it for every pixel ----
+    // ---- phase A: winner map + validity ----
     const EstimateConst E = estimate_const(L, T);
     // row-sharded: the source rows that can reach this rank's band (see ShardArgs); otherwise the whole level
     int halo = 0, a_begin = 0, a_end = n;
@@ -520,18 +559,8 @@ __device__ __forceinline__ void level_loop(const LevelParams& L, const LevelPtrs
       a_end = min(L.rows, L.row_end + halo) * L.cols;
     }
     for (int i = a_begin + bid * kCoopBlock + tid; i < a_end; i += stride) {
-      const double d = __ldg(P.D0 + i);
-      const int r = i / L.cols, c = i - r * L.cols;
-      const bool dep = (L.min_depth < d) & (d < L.max_depth);                  // strict bounds, AN:279-280
-      int tj, ti;
-      const bool unc = estimate_target(L, T, E, r, c, d, tj, ti);
-      bool ok = dep & ((unsigned)tj < (unsigned)L.cols) & ((unsigned)ti < (unsigned)L.rows);
-      int t = L.cols * ti + tj;
-      if (dep & unc) {
-        Warped w;
-        ok = warp_pixel<false>(L, T, r, c, d, w);
-        t = w.t;
-      }
+      int t;
+      const bool ok = phase_a_target(L, T, E, i, __ldg(P.D0 + i), t);
       if (MODE == 3) {   // photometric + depth solver: two residual slots per pixel, keys 2i+1 / 2i+2 (see k_winner_bi)
         if (ok) { atomicMax(P.winner + t, 2 * i + 1); atomicMax(P.winner + 2 * t, 2 * i + 2); }
       } else if (ok) atomicMax(P.winner + t, i);
@@ -599,8 +628,9 @@ __device__ __forceinline__ void level_loop(const LevelParams& L, const LevelPtrs
             acc[27] = fma(res, res, acc[27]);
           }
           if (!ok) continue;
+          const int r = i / L.cols, c = i - r * L.cols;
           double J[6];
-          analytic_jacobian_core<MODE>(L, T, spsr, spcr, i, d, gx, gy, J);
+          analytic_jacobian<MODE>(L, T, spsr, spcr, r, c, d, gx, gy, J);
           accumulate_row(acc, J, res);
           acc[28] += 1.;
         }
@@ -629,8 +659,9 @@ __device__ __forceinline__ void level_loop(const LevelParams& L, const LevelPtrs
             acc[27] = fma(res, res, acc[27]);
           }
           if (!ok) continue;
+          const int r = i / L.cols, c = i - r * L.cols;
           double J[6];
-          analytic_jacobian_core<MODE>(L, T, spsr, spcr, i, d, gx, gy, J);
+          analytic_jacobian<MODE>(L, T, spsr, spcr, r, c, d, gx, gy, J);
           accumulate_row(acc, J, res);
           acc[28] += 1.;
         }
@@ -647,21 +678,7 @@ __device__ __forceinline__ void level_loop(const LevelParams& L, const LevelPtrs
       if (tid < PHOVO_NACC) partials[(size_t)bid * PHOVO_ACC_STRIDE + tid] = total;
     }
     level_barrier<SLOT>();
-    // ---- every CTA: fixed-order sum of all partials (group g of 8 takes blocks g, g+8, ...) ----
-    {
-      const int v = tid & 31, g = tid >> 5;
-      double s = 0.;
-      for (int b = g; b < nblk; b += kCoopBlock / 32) s += __ldcg(partials + (size_t)b * PHOVO_ACC_STRIDE + v);
-      smem[g * PHOVO_ACC_STRIDE + v] = s;
-      __syncthreads();
-      if (tid < 32) {
-        double t = 0.;
-#pragma unroll
-        for (int k = 0; k < kCoopBlock / 32; ++k) t += smem[k * PHOVO_ACC_STRIDE + tid];
-        s_tot[tid] = t;
-      }
-      __syncthreads();
-    }
+    sum_all_partials(partials, nblk, smem, s_tot);
     // ---- row-sharded: all-reduce of the 29 sums over NVLink peer memory, in rank order ----
     if (SHARD && S.world > 1) {
       const unsigned long long epoch = S.epoch_base + (unsigned long long)it + 1ull;
@@ -692,38 +709,20 @@ __device__ __forceinline__ void level_loop(const LevelParams& L, const LevelPtrs
       }
       __syncthreads();
     }
-    // ---- Gauss-Newton step + termination test (AN:538-549, 376-392), one thread per CTA ----
+    // ---- Gauss-Newton step + termination test, one thread per CTA ----
     if (tid == 0) {
-      double g[6], step[6], s_in[6], s_out[6], n2 = 0.;
-      for (int k = 0; k < 6; ++k) { g[k] = s_tot[21 + k]; n2 = fma(g[k], g[k], n2); s_in[k] = s_pose.state[k]; }
-      solve6_ldlt(s_tot, g, step);
-      for (int k = 0; k < 6; ++k) s_out[k] = s_in[k] - L.lambda * step[k];
-      const double gnorm = sqrt(n2);
-      const int done = (it + 1 >= L.max_iters) || (gnorm < L.min_grad_norm);
-      if (bid == 0 && log && log_count < log_capacity) {
-        phovo_iter_stats* e = log + log_count;
-        e->level = L.level; e->iteration = it; e->num_valid = (int)s_tot[28]; e->accepted = 1;
-        for (int k = 0; k < 21; ++k) e->H[k] = s_tot[k];
-        for (int k = 0; k < 6; ++k) { e->g[k] = g[k]; e->state_in[k] = s_in[k]; e->state_out[k] = s_out[k]; }
-        e->grad_norm = gnorm; e->cost = 0.5 * s_tot[27]; e->radius = 0.;
-      }
-      Pose Pn;
-      pose_from_state(s_out, Pn);
-      for (int k = 0; k < 6; ++k) s_pose.state[k] = s_out[k];
-      pose_store(Pn, &s_pose);
+      double s_in[6], s_out[6];
+      for (int k = 0; k < 6; ++k) s_in[k] = s_pose.state[k];
+      const int done = gn_update(L, s_tot, s_in, it, s_out);
+      if (bid == 0 && log && log_count < log_capacity) gn_entry(log + log_count, L, s_tot, it, s_in, s_out);
+      pose_set_state(&s_pose, s_out);
       s_done = done;
     }
     log_count += 1;
     __syncthreads();
     if (s_done) { ++it; break; }
   }
-  if (bid == 0 && tid == 0) {
-    s_pose.iteration = it;
-    s_pose.iters_per_level[L.level] = it;
-    s_pose.done = 1;
-    s_pose.log_count = log_count;
-    *pose = s_pose;
-  }
+  if (bid == 0 && tid == 0) finish_level(pose, s_pose, L.level, it, log_count);
 }
 
 template <int MODE, bool SHARD>
@@ -776,18 +775,8 @@ __global__ void __launch_bounds__(kClusterBlock, 1) k_level_cluster(LevelParams 
     // ---- phase A: bids of the owned source pixels into the owners of their target slots ----
     const EstimateConst E = estimate_const(L, T);
     for (int i = begin + tid; i < end; i += kClusterBlock) {
-      const double d = __ldg(P.D0 + i);
-      const int r = i / L.cols, c = i - r * L.cols;
-      const bool dep = (L.min_depth < d) & (d < L.max_depth);                  // strict bounds, AN:279-280
-      int tj, ti;
-      const bool unc = estimate_target(L, T, E, r, c, d, tj, ti);
-      bool ok = dep & ((unsigned)tj < (unsigned)L.cols) & ((unsigned)ti < (unsigned)L.rows);
-      int t = L.cols * ti + tj;
-      if (dep & unc) {
-        Warped w;
-        ok = warp_pixel<false>(L, T, r, c, d, w);
-        t = w.t;
-      }
+      int t;
+      const bool ok = phase_a_target(L, T, E, i, __ldg(P.D0 + i), t);
       if (ok) {
         const int owner = t / chunk;
         atomicMax(cluster.map_shared_rank(sWin, owner) + (t - owner * chunk), i);   // raster-order last writer wins (AN:358)
@@ -809,8 +798,9 @@ __global__ void __launch_bounds__(kClusterBlock, 1) k_level_cluster(LevelParams 
         acc[27] = fma(res, res, acc[27]);
       }
       if (!sValid[i - begin]) continue;
+      const int r = i / L.cols, c = i - r * L.cols;
       double J[6];
-      analytic_jacobian_row<MODE>(L, P, T, spsr, spcr, i, J);
+      analytic_jacobian<MODE>(L, T, spsr, spcr, r, c, __ldg(P.D0 + i), __ldg(P.Gx + i), __ldg(P.Gy + i), J);
       accumulate_row(acc, J, res);
       acc[28] += 1.;
     }
@@ -829,116 +819,31 @@ __global__ void __launch_bounds__(kClusterBlock, 1) k_level_cluster(LevelParams 
     }
     __syncthreads();
     if (tid == 0) {
-      double g[6], step[6], s_in[6], s_out[6], n2 = 0.;
-      for (int k = 0; k < 6; ++k) { g[k] = s_tot[21 + k]; n2 = fma(g[k], g[k], n2); s_in[k] = s_pose.state[k]; }
-      solve6_ldlt(s_tot, g, step);
-      for (int k = 0; k < 6; ++k) s_out[k] = s_in[k] - L.lambda * step[k];
-      const double gnorm = sqrt(n2);
-      const int done = (it + 1 >= L.max_iters) || (gnorm < L.min_grad_norm);
-      if (rank == 0 && log && log_count < log_capacity) {
-        phovo_iter_stats* e = log + log_count;
-        e->level = L.level; e->iteration = it; e->num_valid = (int)s_tot[28]; e->accepted = 1;
-        for (int k = 0; k < 21; ++k) e->H[k] = s_tot[k];
-        for (int k = 0; k < 6; ++k) { e->g[k] = g[k]; e->state_in[k] = s_in[k]; e->state_out[k] = s_out[k]; }
-        e->grad_norm = gnorm; e->cost = 0.5 * s_tot[27]; e->radius = 0.;
-      }
-      Pose Pn;
-      pose_from_state(s_out, Pn);
-      for (int k = 0; k < 6; ++k) s_pose.state[k] = s_out[k];
-      pose_store(Pn, &s_pose);
+      double s_in[6], s_out[6];
+      for (int k = 0; k < 6; ++k) s_in[k] = s_pose.state[k];
+      const int done = gn_update(L, s_tot, s_in, it, s_out);
+      if (rank == 0 && log && log_count < log_capacity) gn_entry(log + log_count, L, s_tot, it, s_in, s_out);
+      pose_set_state(&s_pose, s_out);
       s_done = done;
     }
     log_count += 1;
     __syncthreads();
     if (s_done) { ++it; break; }
   }
-  if (rank == 0 && tid == 0) {
-    s_pose.iteration = it;
-    s_pose.iters_per_level[L.level] = it;
-    s_pose.done = 1;
-    s_pose.log_count = log_count;
-    *pose = s_pose;
-  }
+  if (rank == 0 && tid == 0) finish_level(pose, s_pose, L.level, it, log_count);
   cluster.sync();                       // nobody leaves while its shared memory may still be written remotely
 }
 
 // ---------------------------------------------------------------------------------------------
 // Ceres mode on the device: the restated trust-region Levenberg-Marquardt loop of one level
 // (CE:433-500 -> ceres::Solve, SURVEY appendix A) inside ONE persistent cooperative launch.  Every loop
-// trip is one evaluation of the CE:156-269 residual + Jacobian at `eval_x` (phase A winner map by
+// trip is one evaluation of the CE:156-269 residual + Jacobian at S.xn (phase A winner map by
 // truncation, grid.sync, phase B bilinear samples + normal equations, grid.sync, fixed-order sum of
-// all partials in every CTA) followed by the LM decision, which thread 0 of every CTA takes
-// redundantly -- identical inputs, identical arithmetic, so all CTAs stay in lock step without a
-// broadcast.  CTA 0 writes the log.  The decision code mirrors the host loop in phovo_api.cu
-// (optimize_ceres), statement for statement.
+// all partials in every CTA) followed by the LM decision of phovo_lm.h -- the same functions the host
+// loop in phovo_api.cu (optimize_ceres) calls.  Thread 0 of every CTA takes the decision redundantly:
+// identical inputs, identical arithmetic, so all CTAs stay in lock step without a broadcast.  CTA 0
+// writes the log.
 // ---------------------------------------------------------------------------------------------
-struct LmState {
-  double x[6], xn[6], scale[6], step_norm, x_norm, model_cost_change;
-  double H[21], g[6], cost;       // `cur`
-  double radius, decrease_factor;
-  int num_valid, iteration, first, done;
-};
-
-__device__ bool chol_solve6_dev(const double M[36], const double b[6], double x[6]) {
-  double Lm[36];
-  for (int i = 0; i < 36; ++i) Lm[i] = 0.;
-  for (int i = 0; i < 6; ++i)
-    for (int j = 0; j <= i; ++j) {
-      double sum = M[i * 6 + j];
-      for (int k = 0; k < j; ++k) sum -= Lm[i * 6 + k] * Lm[j * 6 + k];
-      if (i == j) { if (!(sum > 0)) return false; Lm[i * 6 + i] = sqrt(sum); }
-      else Lm[i * 6 + j] = sum / Lm[j * 6 + j];
-    }
-  double y[6];
-  for (int i = 0; i < 6; ++i) { double sum = b[i]; for (int k = 0; k < i; ++k) sum -= Lm[i * 6 + k] * y[k]; y[i] = sum / Lm[i * 6 + i]; }
-  for (int i = 5; i >= 0; --i) { double sum = y[i]; for (int k = i + 1; k < 6; ++k) sum -= Lm[k * 6 + i] * x[k]; x[i] = sum / Lm[i * 6 + i]; }
-  return true;
-}
-
-__device__ void expand_sym_dev(const double H[21], double M[36]) {
-  int k = 0;
-  for (int a = 0; a < 6; ++a) for (int b = a; b < 6; ++b) { M[a * 6 + b] = H[k]; M[b * 6 + a] = H[k]; ++k; }
-}
-
-// log entry for the LM iteration being decided (host: `s`)
-__device__ void lm_log(const LevelParams& L, const LmState& S, phovo_iter_stats* log, int& log_count, int log_capacity, int accepted,
-                       const double* state_out) {
-  if (blockIdx.x == 0 && log && log_count < log_capacity) {
-    phovo_iter_stats* e = log + log_count;
-    e->level = L.level; e->iteration = S.iteration - 1; e->num_valid = S.num_valid; e->accepted = accepted;
-    double n2 = 0.;
-    for (int k = 0; k < 21; ++k) e->H[k] = S.H[k];
-    for (int k = 0; k < 6; ++k) { e->g[k] = S.g[k]; n2 += S.g[k] * S.g[k]; e->state_in[k] = S.x[k]; e->state_out[k] = state_out[k]; }
-    e->grad_norm = sqrt(n2); e->cost = S.cost; e->radius = S.radius;
-  }
-  log_count += 1;
-}
-
-// Prepare LM iteration `S.iteration + 1` from `cur`: returns false when the loop ends here.
-__device__ bool lm_next_step(const LevelParams& L, const LmParams& lm, LmState& S, phovo_iter_stats* log, int& log_count, int log_capacity) {
-  if (S.iteration >= lm.max_iterations) return false;
-  S.iteration += 1;
-  double M[36], Ms[36], gs[6], A[36], step[6];
-  expand_sym_dev(S.H, M);
-  for (int a = 0; a < 6; ++a) { gs[a] = S.g[a] * S.scale[a]; for (int b = 0; b < 6; ++b) Ms[a * 6 + b] = M[a * 6 + b] * S.scale[a] * S.scale[b]; }
-  for (int k = 0; k < 36; ++k) A[k] = Ms[k];
-  for (int a = 0; a < 6; ++a) { double d = Ms[a * 6 + a]; if (d < 1e-6) d = 1e-6; if (d > 1e32) d = 1e32; A[a * 6 + a] += d / S.radius; }
-  bool ok = chol_solve6_dev(A, gs, step);
-  for (int a = 0; a < 6; ++a) step[a] = -step[a];
-  double model_cost_change = 0;
-  if (ok) {
-    double dg = 0, dMd = 0;
-    for (int a = 0; a < 6; ++a) { dg += step[a] * gs[a]; double t = 0; for (int b = 0; b < 6; ++b) t += Ms[a * 6 + b] * step[b]; dMd += step[a] * t; }
-    model_cost_change = -(dg + 0.5 * dMd);
-    for (int a = 0; a < 6; ++a) if (!isfinite(step[a])) ok = false;
-  }
-  if (!ok || !(model_cost_change > 0)) { lm_log(L, S, log, log_count, log_capacity, 0, S.x); return false; }   // max_num_consecutive_invalid_steps = 0 (CE:477)
-  double step_norm = 0, x_norm = 0;
-  for (int a = 0; a < 6; ++a) { const double d = step[a] * S.scale[a]; S.xn[a] = S.x[a] + d; step_norm += d * d; x_norm += S.x[a] * S.x[a]; }
-  S.step_norm = sqrt(step_norm); S.x_norm = sqrt(x_norm); S.model_cost_change = model_cost_change;
-  return true;
-}
-
 template <int SLOT>
 __device__ __forceinline__ void level_loop_ceres(const LevelParams& L, const LevelPtrs& P, PoseDev* pose, double* partials,
                                                  phovo_iter_stats* log, const LmParams& lm) {
@@ -947,11 +852,12 @@ __device__ __forceinline__ void level_loop_ceres(const LevelParams& L, const Lev
   __shared__ double s_tot[32];
   __shared__ PoseDev s_pose;
   __shared__ LmState S;
+  __shared__ int s_first, s_done;
   const int tid = threadIdx.x;
   if (tid == 0) {
     s_pose = *pose;
     for (int k = 0; k < 6; ++k) { S.x[k] = s_pose.state[k]; S.xn[k] = s_pose.state[k]; }
-    S.radius = lm.initial_radius; S.decrease_factor = 2.0; S.iteration = 0; S.first = 1; S.done = 0;
+    S.radius = lm.initial_radius; S.decrease_factor = 2.0; S.iteration = 0; s_first = 1; s_done = 0;
   }
   __syncthreads();
   int log_count = s_pose.log_count;
@@ -960,12 +866,7 @@ __device__ __forceinline__ void level_loop_ceres(const LevelParams& L, const Lev
   const int stride = nblk * kCoopBlock;
   for (;;) {
     // ---- pose of the state to evaluate (every CTA, thread 0) ----
-    if (tid == 0) {
-      Pose Pn;
-      pose_from_state(S.xn, Pn);
-      for (int k = 0; k < 6; ++k) s_pose.state[k] = S.xn[k];
-      pose_store(Pn, &s_pose);
-    }
+    if (tid == 0) pose_set_state(&s_pose, S.xn);
     __syncthreads();
     Pose T;
     pose_load(&s_pose, T);
@@ -1012,79 +913,30 @@ __device__ __forceinline__ void level_loop_ceres(const LevelParams& L, const Lev
       if (tid < PHOVO_NACC) partials[(size_t)bid * PHOVO_ACC_STRIDE + tid] = total;
     }
     level_barrier<SLOT>();   // partials complete, every winner slot back to -1
-    {
-      const int v = tid & 31, g = tid >> 5;
-      double sum = 0.;
-      for (int b = g; b < nblk; b += kCoopBlock / 32) sum += __ldcg(partials + (size_t)b * PHOVO_ACC_STRIDE + v);
-      smem[g * PHOVO_ACC_STRIDE + v] = sum;
-      __syncthreads();
-      if (tid < 32) {
-        double t = 0.;
-#pragma unroll
-        for (int k = 0; k < kCoopBlock / 32; ++k) t += smem[k * PHOVO_ACC_STRIDE + tid];
-        s_tot[tid] = t;
-      }
-      __syncthreads();
-    }
-    // ---- LM decision (host twin: optimize_ceres in phovo_api.cu) ----
+    sum_all_partials(partials, nblk, smem, s_tot);
+    // ---- LM decision (phovo_lm.h) ----
     if (tid == 0) {
+      LmLog sink{log, log_count, log_capacity, bid == 0 && log != nullptr};
       bool go;
-      if (S.first) {
-        S.first = 0;
-        for (int k = 0; k < 21; ++k) S.H[k] = s_tot[k];
-        for (int k = 0; k < 6; ++k) S.g[k] = s_tot[21 + k];
-        S.cost = 0.5 * s_tot[27]; S.num_valid = (int)s_tot[28];
-        double M[36]; expand_sym_dev(S.H, M);
-        for (int a = 0; a < 6; ++a) S.scale[a] = 1.0 / (1.0 + sqrt(M[a * 6 + a]));
-        double gmax = 0; for (int a = 0; a < 6; ++a) gmax = fmax(gmax, fabs(S.g[a]));
-        go = !(gmax <= lm.gradient_tolerance) && lm_next_step(L, lm, S, log, log_count, log_capacity);
+      if (s_first) {
+        s_first = 0;
+        entry_from_totals(&S.cur, L.level, s_tot);
+        go = lm_start(lm, S) && lm_propose(lm, S, sink);
       } else {
-        const double cand_cost = 0.5 * s_tot[27];
-        go = true;
-        if (S.step_norm <= lm.parameter_tolerance * (S.x_norm + lm.parameter_tolerance)) { lm_log(L, S, log, log_count, log_capacity, 0, S.x); go = false; }
-        const double cost_change = S.cost - cand_cost;
-        if (go && fabs(cost_change) < lm.function_tolerance * S.cost) { lm_log(L, S, log, log_count, log_capacity, 0, S.x); go = false; }
-        if (go) {
-          const double rho = cost_change / S.model_cost_change;
-          if (rho > lm.min_relative_decrease) {
-            lm_log(L, S, log, log_count, log_capacity, 1, S.xn);
-            for (int k = 0; k < 6; ++k) S.x[k] = S.xn[k];
-            for (int k = 0; k < 21; ++k) S.H[k] = s_tot[k];
-            for (int k = 0; k < 6; ++k) S.g[k] = s_tot[21 + k];
-            S.cost = cand_cost; S.num_valid = (int)s_tot[28];
-            double gmax = 0; for (int a = 0; a < 6; ++a) gmax = fmax(gmax, fabs(S.g[a]));
-            if (gmax <= lm.gradient_tolerance) go = false;
-            else {
-              const double t = 2.0 * rho - 1.0;
-              double f = 1.0 - t * t * t; if (f < 1.0 / 3.0) f = 1.0 / 3.0;
-              S.radius = S.radius / f; if (S.radius > lm.max_radius) S.radius = lm.max_radius;
-              S.decrease_factor = 2.0;
-            }
-          } else {
-            lm_log(L, S, log, log_count, log_capacity, 0, S.x);
-            S.radius = S.radius / S.decrease_factor; S.decrease_factor *= 2.0;
-          }
-          if (go && S.radius < lm.min_radius) go = false;
-          if (go) go = lm_next_step(L, lm, S, log, log_count, log_capacity);
-        }
+        const int v = lm_judge(lm, S, 0.5 * s_tot[27], sink);
+        if (v == LM_ACCEPT) entry_from_totals(&S.cur, L.level, s_tot);
+        go = v != LM_STOP && lm_update_radius(lm, S, v == LM_ACCEPT) && lm_propose(lm, S, sink);
       }
-      S.done = go ? 0 : 1;
+      s_done = go ? 0 : 1;
       s_pose.log_count = log_count;
     }
     __syncthreads();
     log_count = s_pose.log_count;
-    if (S.done) break;
+    if (s_done) break;
   }
   if (bid == 0 && tid == 0) {
-    Pose Pn;
-    pose_from_state(S.x, Pn);
-    for (int k = 0; k < 6; ++k) s_pose.state[k] = S.x[k];
-    pose_store(Pn, &s_pose);
-    s_pose.iteration = S.iteration;
-    s_pose.iters_per_level[L.level] = S.iteration;
-    s_pose.done = 1;
-    s_pose.log_count = log_count;
-    *pose = s_pose;
+    pose_set_state(&s_pose, S.x);
+    finish_level(pose, s_pose, L.level, S.iteration, log_count);
   }
 }
 
@@ -1116,11 +968,8 @@ __global__ void __launch_bounds__(kCoopBlock, PHOVO_SLOT_MINB) k_align_slots(con
   if (level_block_rank<S>() == 0 && threadIdx.x == 0) {   // k_set_state for this slot: the caller's initial state (zero if none), counters cleared, no log
     double s[6];
     for (int k = 0; k < 6; ++k) s[k] = init_states ? init_states[(size_t)slot * 6 + k] : 0.;
-    Pose P0;
-    pose_from_state(s, P0);
     PoseDev* pose = A.pose;
-    for (int k = 0; k < 6; ++k) pose->state[k] = s[k];
-    pose_store(P0, pose);
+    pose_set_state(pose, s);
     pose->iteration = 0; pose->done = 0; pose->log_count = 0; pose->log_capacity = 0;
     for (int l = 0; l < PHOVO_MAX_LEVELS; ++l) pose->iters_per_level[l] = 0;
   }
@@ -1285,8 +1134,7 @@ int launch_level_cluster(cudaStream_t stream, const LevelParams& L, const LevelP
 }
 
 int launch_level_coop_ceres(cudaStream_t stream, const LevelParams& L, const LevelPtrs& P, PoseDev* pose, double* partials,
-                            phovo_iter_stats* log, const double lm_params[7], int max_iterations, LaunchState* ls, int sm_count,
-                            cudaError_t* err) {
+                            phovo_iter_stats* log, const LmParams& lm, LaunchState* ls, int sm_count, cudaError_t* err) {
   int& blocks_per_sm = ls->ceres_blocks_per_sm;
   void* fn = (void*)k_level_coop_ceres;
   if (blocks_per_sm < 0) {
@@ -1300,12 +1148,8 @@ int launch_level_coop_ceres(cudaStream_t stream, const LevelParams& L, const Lev
   const int cap = sm_count * (blocks_per_sm < 2 ? blocks_per_sm : 2);
   if (grid > cap) grid = cap;
   if (grid < 1) grid = 1;
-  LevelParams Lc = L; LevelPtrs Pc = P;
-  LmParams lm;
-  lm.function_tolerance = lm_params[0]; lm.gradient_tolerance = lm_params[1]; lm.parameter_tolerance = lm_params[2];
-  lm.initial_radius = lm_params[3]; lm.max_radius = lm_params[4]; lm.min_radius = lm_params[5]; lm.min_relative_decrease = lm_params[6];
-  lm.max_iterations = max_iterations;
-  void* args[] = {&Lc, &Pc, &pose, &partials, &log, &lm};
+  LevelParams Lc = L; LevelPtrs Pc = P; LmParams lmc = lm;
+  void* args[] = {&Lc, &Pc, &pose, &partials, &log, &lmc};
   *err = cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kCoopBlock), args, 0, stream);
   return *err == cudaSuccess ? 1 : -1;
 }

@@ -8,6 +8,7 @@
 #include <vector>
 
 #include "phovo_ctx.h"
+#include "phovo_lm.h"
 
 using namespace phovo;
 
@@ -732,11 +733,9 @@ static int optimize_ceres_coop(phovo_ctx* ctx, bool* unavailable) {
     if (!(M > 0)) continue;   // CE:437
     const LevelParams L = ctx->level_params(level);
     const LevelPtrs P = ctx->level_ptrs(level);
-    const double lm[7] = {ctx->cfg.function_tolerance[level], ctx->cfg.gradient_tolerance[level], ctx->cfg.parameter_tolerance[level],
-                          ctx->cfg.initial_trust_region_radius[level], ctx->cfg.max_trust_region_radius[level],
-                          ctx->cfg.min_trust_region_radius[level], ctx->cfg.min_relative_decrease[level]};
     cudaError_t e = cudaSuccess;
-    const int rc = launch_level_coop_ceres(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->d_log.get(), lm, M, &ctx->launch_state, ctx->sm_count, &e);
+    const int rc = launch_level_coop_ceres(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->d_log.get(), lm_params(ctx->cfg, level),
+                                           &ctx->launch_state, ctx->sm_count, &e);
     if (rc < 0) {
       cudaGetLastError();
       ctx->graph_error = std::string("cooperative launch unavailable: ") + cudaGetErrorString(e);
@@ -977,97 +976,29 @@ extern "C" int phovo_synchronize(phovo_ctx* ctx) {
 // itself is third-party and absent from the reference tree: trajectory parity is UNPINNED, the
 // residual/Jacobian kernel (K5) is pinned against the oracle.
 // ---------------------------------------------------------------------------------------------
-static void expand_sym(const double H[21], double M[36]) {
-  int k = 0;
-  for (int a = 0; a < 6; ++a) for (int b = a; b < 6; ++b) { M[a * 6 + b] = H[k]; M[b * 6 + a] = H[k]; ++k; }
-}
-static bool chol_solve6(const double M[36], const double b[6], double x[6]) {
-  double Lm[36]; memset(Lm, 0, sizeof(Lm));
-  for (int i = 0; i < 6; ++i)
-    for (int j = 0; j <= i; ++j) {
-      double s = M[i * 6 + j];
-      for (int k = 0; k < j; ++k) s -= Lm[i * 6 + k] * Lm[j * 6 + k];
-      if (i == j) { if (!(s > 0)) return false; Lm[i * 6 + i] = sqrt(s); }
-      else Lm[i * 6 + j] = s / Lm[j * 6 + j];
-    }
-  double y[6];
-  for (int i = 0; i < 6; ++i) { double s = b[i]; for (int k = 0; k < i; ++k) s -= Lm[i * 6 + k] * y[k]; y[i] = s / Lm[i * 6 + i]; }
-  for (int i = 5; i >= 0; --i) { double s = y[i]; for (int k = i + 1; k < 6; ++k) s -= Lm[k * 6 + i] * x[k]; x[i] = s / Lm[i * 6 + i]; }
-  return true;
-}
-
 static int optimize_ceres(phovo_ctx* ctx) {
   ctx->log.clear();
-  double x[6];
-  memcpy(x, ctx->state, sizeof(x));
+  int log_count = 0;
+  LmLog log{ctx->h_log.get(), log_count, ctx->log_cap(), true};
+  LmState S;
+  memcpy(S.x, ctx->state, sizeof(S.x));
   for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
-    const int max_it = ctx->cfg.max_num_iterations[level];
-    if (!(max_it > 0)) continue;   // CE:437
-    double radius = ctx->cfg.initial_trust_region_radius[level];
-    const double max_radius = ctx->cfg.max_trust_region_radius[level];
-    const double min_radius = ctx->cfg.min_trust_region_radius[level];
-    const double eta = ctx->cfg.min_relative_decrease[level];
-    double decrease_factor = 2.0;
-    phovo_iter_stats cur;
-    int rc = eval_at(ctx, level, x, &cur, nullptr, nullptr);
+    const LmParams lm = lm_params(ctx->cfg, level);
+    if (!(lm.max_iterations > 0)) continue;   // CE:437
+    S.radius = lm.initial_radius; S.decrease_factor = 2.0; S.iteration = 0;
+    int rc = eval_at(ctx, level, S.x, &S.cur, nullptr, nullptr);
     if (rc) return rc;
-    double scale[6];
-    { double M[36]; expand_sym(cur.H, M); for (int a = 0; a < 6; ++a) scale[a] = 1.0 / (1.0 + sqrt(M[a * 6 + a])); }
-    double gmax = 0; for (int a = 0; a < 6; ++a) gmax = fmax(gmax, fabs(cur.g[a]));
-    int iteration = 0;
-    if (!(gmax <= ctx->cfg.gradient_tolerance[level])) {
-      while (true) {
-        if (iteration >= max_it) break;
-        ++iteration;
-        phovo_iter_stats s = cur;
-        s.level = level; s.iteration = iteration - 1; s.radius = radius; s.accepted = 0;
-        memcpy(s.state_in, x, sizeof(x)); memcpy(s.state_out, x, sizeof(x));
-        double M[36], Ms[36], gs[6], A[36];
-        expand_sym(cur.H, M);
-        for (int a = 0; a < 6; ++a) { gs[a] = cur.g[a] * scale[a]; for (int b = 0; b < 6; ++b) Ms[a * 6 + b] = M[a * 6 + b] * scale[a] * scale[b]; }
-        memcpy(A, Ms, sizeof(A));
-        for (int a = 0; a < 6; ++a) { double d = Ms[a * 6 + a]; if (d < 1e-6) d = 1e-6; if (d > 1e32) d = 1e32; A[a * 6 + a] += d / radius; }
-        double step[6];
-        bool ok = chol_solve6(A, gs, step);
-        for (int a = 0; a < 6; ++a) step[a] = -step[a];
-        double model_cost_change = 0;
-        if (ok) {
-          double dg = 0, dMd = 0;
-          for (int a = 0; a < 6; ++a) { dg += step[a] * gs[a]; double t = 0; for (int b = 0; b < 6; ++b) t += Ms[a * 6 + b] * step[b]; dMd += step[a] * t; }
-          model_cost_change = -(dg + 0.5 * dMd);
-          for (int a = 0; a < 6; ++a) if (!isfinite(step[a])) ok = false;
-        }
-        if (!ok || !(model_cost_change > 0)) { ctx->log.push_back(s); break; }   // max_num_consecutive_invalid_steps = 0 (CE:477)
-        double xn[6], step_norm = 0, x_norm = 0;
-        for (int a = 0; a < 6; ++a) { const double d = step[a] * scale[a]; xn[a] = x[a] + d; step_norm += d * d; x_norm += x[a] * x[a]; }
-        step_norm = sqrt(step_norm); x_norm = sqrt(x_norm);
-        phovo_iter_stats cand;
-        if ((rc = eval_at(ctx, level, xn, &cand, nullptr, nullptr))) return rc;
-        const double ptol = ctx->cfg.parameter_tolerance[level];
-        if (step_norm <= ptol * (x_norm + ptol)) { ctx->log.push_back(s); break; }
-        const double cost_change = cur.cost - cand.cost;
-        if (fabs(cost_change) < ctx->cfg.function_tolerance[level] * cur.cost) { ctx->log.push_back(s); break; }
-        const double rho = cost_change / model_cost_change;
-        if (rho > eta) {
-          memcpy(x, xn, sizeof(x));
-          s.accepted = 1; memcpy(s.state_out, x, sizeof(x));
-          ctx->log.push_back(s);
-          cur = cand;
-          gmax = 0; for (int a = 0; a < 6; ++a) gmax = fmax(gmax, fabs(cur.g[a]));
-          if (gmax <= ctx->cfg.gradient_tolerance[level]) break;
-          const double t = 2.0 * rho - 1.0;
-          double f = 1.0 - t * t * t; if (f < 1.0 / 3.0) f = 1.0 / 3.0;
-          radius = radius / f; if (radius > max_radius) radius = max_radius;
-          decrease_factor = 2.0;
-        } else {
-          ctx->log.push_back(s);
-          radius = radius / decrease_factor; decrease_factor *= 2.0;
-        }
-        if (radius < min_radius) break;
-      }
+    bool go = lm_start(lm, S);
+    while (go && lm_propose(lm, S, log)) {
+      phovo_iter_stats cand;
+      if ((rc = eval_at(ctx, level, S.xn, &cand, nullptr, nullptr))) return rc;
+      const int v = lm_judge(lm, S, cand.cost, log);
+      if (v == LM_ACCEPT) S.cur = cand;
+      go = v != LM_STOP && lm_update_radius(lm, S, v == LM_ACCEPT);
     }
   }
-  memcpy(ctx->state, x, sizeof(x));
+  ctx->log.assign(ctx->h_log.get(), ctx->h_log.get() + std::min(log_count, ctx->log_cap()));
+  memcpy(ctx->state, S.x, sizeof(S.x));
   CK(cudaEventRecord(ctx->ev_time[3].get(), ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   for (int k = 0; k < 6; ++k)

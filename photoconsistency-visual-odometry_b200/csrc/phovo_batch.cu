@@ -622,11 +622,7 @@ static int batch_waves(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int 
         if (!(M > 0)) continue;
         const int a = LS.count++;
         LS.L[a] = c0->level_params(level);
-        LmParams& lm = LS.lm[a];
-        lm.function_tolerance = ctx->cfg.function_tolerance[level]; lm.gradient_tolerance = ctx->cfg.gradient_tolerance[level];
-        lm.parameter_tolerance = ctx->cfg.parameter_tolerance[level]; lm.initial_radius = ctx->cfg.initial_trust_region_radius[level];
-        lm.max_radius = ctx->cfg.max_trust_region_radius[level]; lm.min_radius = ctx->cfg.min_trust_region_radius[level];
-        lm.min_relative_decrease = ctx->cfg.min_relative_decrease[level]; lm.max_iterations = M;
+        LS.lm[a] = lm_params(ctx->cfg, level);
       }
       levels_known = true;
     }

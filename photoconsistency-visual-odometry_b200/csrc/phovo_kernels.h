@@ -8,6 +8,7 @@
 #include <stdint.h>
 
 #include "phovo_internal.h"
+#include "phovo_lm.h"
 
 namespace phovo {
 
@@ -71,13 +72,6 @@ struct LevelPtrs {
   const double* D1; const double* GxD; const double* GyD; const double* gain;
 };
 
-// Levenberg-Marquardt options of one level (Ceres mode, CE:464-477)
-struct LmParams {
-  double function_tolerance, gradient_tolerance, parameter_tolerance;
-  double initial_radius, max_radius, min_radius, min_relative_decrease;
-  int max_iterations;
-};
-
 // Batch wave path (phovo_batch.cu): a SLOT is the device side of a child context -- the pyramids of one pair, its
 // winner map, its PoseDev.  k_align_slots runs one CTA per slot through every active level (coarse to fine).
 struct SlotArgs {
@@ -139,11 +133,9 @@ int launch_min_valid_depth(cudaStream_t stream, const double* D, int n, double l
 // qualify: use launch_level_coop), -1 (launch error in *err).
 int launch_level_cluster(cudaStream_t stream, const LevelParams& L, const LevelPtrs& P, PoseDev* pose, phovo_iter_stats* log, LaunchState* ls, cudaError_t* err);
 
-// Ceres mode: the restated LM loop of one level in one cooperative launch.  lm_params: function, gradient, parameter
-// tolerance, initial / max / min trust-region radius, min relative decrease (CE:464-477).
+// Ceres mode: the restated LM loop of one level (phovo_lm.h) in one cooperative launch.
 int launch_level_coop_ceres(cudaStream_t stream, const LevelParams& L, const LevelPtrs& P, PoseDev* pose, double* partials,
-                            phovo_iter_stats* log, const double lm_params[7], int max_iterations, LaunchState* ls, int sm_count,
-                            cudaError_t* err);
+                            phovo_iter_stats* log, const LmParams& lm, LaunchState* ls, int sm_count, cudaError_t* err);
 
 // Exchange area of the fused peer-store all-reduce (one per rank, IPC-shared with the peers).
 struct ShardExchange {

@@ -188,8 +188,10 @@ int phovo_get_iter_stats(const phovo_ctx* ctx, int index, phovo_iter_stats* out)
 int phovo_get_level_image(phovo_ctx* ctx, int which, int level, double* dst, int* rows, int* cols);
 /* Evaluate the normal equations once at `state` on `level` without stepping (fills H,g,cost,num_valid). */
 int phovo_eval_normal_equations(phovo_ctx* ctx, int level, const double state[6], phovo_iter_stats* out);
-/* Ceres-mode parity hook: residual vector (rows*cols doubles) and optional Jacobian
- * (rows*cols x 6, row-major doubles) at `state` on `level` (CE:156-269).  Either may be NULL. */
+/* Parity hook: residual vector and Jacobian (row-major, 6 doubles per row) at `state` on `level`, with
+ * rows*cols rows of that level in the analytic and Ceres modes (CE:156-269) and 2*rows*cols rows in
+ * PHOVO_MODE_BIOBJECTIVE, which stacks the depth rows under the intensity rows (BI:422-452): the residual
+ * buffer takes rows*cols or 2*rows*cols doubles, the Jacobian buffer six times that.  Either may be NULL. */
 int phovo_eval_residuals(phovo_ctx* ctx, int level, const double state[6], double* residuals, double* jacobian);
 /* device time of the last phovo_optimize / frame setup in milliseconds (CUDA events) */
 int phovo_get_timings(const phovo_ctx* ctx, float* setup_ms, float* optimize_ms);

@@ -220,9 +220,16 @@ class CPhotoconsistencyOdometryCuda:
         self._check(self._L.phovo_eval_normal_equations(self._h, level, s.ctypes.data_as(capi._dp), C.byref(st)))
         return st.as_dict()
 
-    def EvalResiduals(self, level, state, shape):
+    def EvalResiduals(self, level, state, shape=None):
+        """Residual vector and Jacobian at `state` on `level`: rows*cols rows of that level, or 2*rows*cols in the
+        photometric + depth mode, which stacks a depth row under every intensity row.  The buffers are sized from the
+        level the context built; `shape`, if given, must be that level's (rows, cols)."""
         s = np.ascontiguousarray(state, dtype=np.float64).reshape(6)
-        n = shape[0] * shape[1]
+        r, c = C.c_int32(), C.c_int32()
+        self._check(self._L.phovo_get_level_image(self._h, 0, level, None, C.byref(r), C.byref(c)))
+        if shape is not None and tuple(shape) != (r.value, c.value):
+            raise ValueError("level %d is %dx%d, not %s" % (level, r.value, c.value, tuple(shape)))
+        n = r.value * c.value * (2 if self.GetConfig().mode == capi.MODE_BIOBJECTIVE else 1)
         res, jac = np.zeros(n), np.zeros((n, 6))
         self._check(self._L.phovo_eval_residuals(self._h, level, s.ctypes.data_as(capi._dp), res.ctypes.data, jac.ctypes.data))
         return res, jac
@@ -246,12 +253,21 @@ class CPhotoconsistencyOdometryCuda:
 
     def BatchAlign(self, gray0, depth0, gray1, initial_states=None, depth_scale=1.0, depth1=None):
         """Host (numpy / pinned torch) or device (torch) arrays [P,R,C]; returns (states[P,6], iterations[P,MAXL]).
-        `depth1` (target depth, same type as depth0) is read by the photometric + depth solver only."""
+        `depth1` (target depth, same type as depth0) is read by the photometric + depth solver only.  The library reads
+        dense frames: strided views are copied first."""
+        gray0, depth0, gray1, depth1 = (self._dense(a) for a in (gray0, depth0, gray1, depth1))
+        self._follow_producer_stream(gray0, depth0, gray1, depth1)     # (device copies made above are on torch's stream)
         P, R, Cc = tuple(gray0.shape)
         dtype = self._batch_depth_type(depth0)
+        if tuple(depth0.shape) != (P, R, Cc) or tuple(gray1.shape) != (P, R, Cc) or (depth1 is not None and tuple(depth1.shape) != (P, R, Cc)):
+            raise ValueError("gray0, depth0, gray1 and depth1 must all be [P, rows, cols]")
+        if depth1 is not None and self._batch_depth_type(depth1) != dtype:
+            raise TypeError("depth1 must have the element type of depth0 (one depth type is passed for both)")
         states = np.zeros((P, 6))
         iters = np.zeros((P, capi.MAXL), dtype=np.int32)
         init = None if initial_states is None else np.ascontiguousarray(initial_states, dtype=np.float64)
+        if init is not None and init.size != P * 6:
+            raise ValueError("initial_states must be [P, 6]")
         if depth1 is not None:
             self._check(self._L.phovo_batch_align_with_target_depth(self._h, P, R, Cc, capi._ptr(gray0), capi._ptr(depth0), dtype,
                                                                     float(depth_scale), capi._ptr(gray1), capi._ptr(depth1), capi._ptr(init),
@@ -282,9 +298,7 @@ class CPhotoconsistencyOdometryCuda:
         torch tensors on the device for device inputs, numpy otherwise -- and, as numpy [P], `num_landed` (source pixels
         that land in the target), `sum_abs_diff` (sum of |gray1 - warped| over them; None without gray1) and
         `mean_abs_diff` = sum_abs_diff / max(num_landed, 1)."""
-        def dense(a):
-            return None if a is None else np.ascontiguousarray(a) if isinstance(a, np.ndarray) else a.contiguous()
-        gray0, depth0, gray1 = dense(gray0), dense(depth0), dense(gray1)
+        gray0, depth0, gray1 = (self._dense(a) for a in (gray0, depth0, gray1))
         P, R, Cc = tuple(gray0.shape)
         dtype = self._batch_depth_type(depth0)
         if tuple(depth0.shape) != (P, R, Cc) or (gray1 is not None and tuple(gray1.shape) != (P, R, Cc)):
@@ -325,9 +339,7 @@ class CPhotoconsistencyOdometryCuda:
         Returns a dict of numpy arrays: `H` [P,6,6] = J^T J (symmetric), `g` [P,6] = J^T r, `cost` [P] = 0.5 |r|^2 and
         `num_valid` [P].  J scales the image gradients by the configured imageGradientsScalingFactor and, in mode 0,
         carries the reference's temp11 term (AN:253): H is the solver's J^T J, not a calibrated information matrix."""
-        def dense(a):
-            return np.ascontiguousarray(a) if isinstance(a, np.ndarray) else a.contiguous()
-        gray0, depth0, gray1 = dense(gray0), dense(depth0), dense(gray1)
+        gray0, depth0, gray1 = (self._dense(a) for a in (gray0, depth0, gray1))
         P, R, Cc = tuple(gray0.shape)
         dtype = self._batch_depth_type(depth0)
         if tuple(depth0.shape) != (P, R, Cc) or tuple(gray1.shape) != (P, R, Cc):
@@ -353,6 +365,11 @@ class CPhotoconsistencyOdometryCuda:
         H[:, iu[0], iu[1]] = Hu
         H[:, iu[1], iu[0]] = Hu
         return dict(H=H, g=g, cost=cost, num_valid=nv)
+
+    @staticmethod
+    def _dense(a):
+        """A batch entry reads dense [P, rows, cols] frames: a strided numpy array or torch view is copied."""
+        return None if a is None else np.ascontiguousarray(a) if isinstance(a, np.ndarray) else a.contiguous()
 
     @staticmethod
     def _batch_depth_type(depth0):

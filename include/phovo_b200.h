@@ -252,6 +252,14 @@ int phovo_batch_align_device(phovo_ctx* ctx, int num_pairs, int rows, int cols,
                              const uint8_t* gray0_dev, const void* depth0_dev, int depth_type,
                              double depth_scale, const uint8_t* gray1_dev,
                              const double* initial_states_dev, double* states_dev, int32_t* iters_dev);
+/* phovo_batch_align_device for the photometric + depth solver (PHOVO_MODE_BIOBJECTIVE), which also reads the TARGET
+ * depth depth1_dev ([P][rows][cols] on the device, same type / scale as depth0_dev).  In that mode the pairs run through
+ * the pool (< 24 pairs) or the slot waves, as phovo_batch_align_with_target_depth takes them, and the call returns once
+ * the results are in states_dev / iters_dev.  Other modes ignore depth1_dev and forward to phovo_batch_align_device. */
+int phovo_batch_align_device_with_target_depth(phovo_ctx* ctx, int num_pairs, int rows, int cols,
+                                               const uint8_t* gray0_dev, const void* depth0_dev, int depth_type,
+                                               double depth_scale, const uint8_t* gray1_dev, const void* depth1_dev,
+                                               const double* initial_states_dev, double* states_dev, int32_t* iters_dev);
 /* per-pair per-iteration stats of the last batch call (only recorded when enabled: costs HBM; what the resident
  * kernels do not take then goes through the pool of per-pair contexts, whose logs these are) */
 int phovo_batch_set_record_stats(phovo_ctx* ctx, int enable);
@@ -294,7 +302,8 @@ int phovo_batch_warp_image(phovo_ctx* ctx, int num_pairs, int rows, int cols,
  * states [P][6] (x y z yaw pitch roll) on the host or the device; each output may be NULL, host or device, at least
  * one must be given.  Blocking; device inputs are read on the context stream (see phovo_set_source).
  * Results are bitwise reproducible and independent of which pairs share a call.
- * PHOVO_E_UNSUPPORTED: Ceres mode and the photometric + depth solver, blurFilterSize[level] > 1, level 1 of a frame
+ * PHOVO_E_UNSUPPORTED: Ceres mode and the photometric + depth solver (which has
+ * phovo_batch_eval_normal_equations_with_target_depth), blurFilterSize[level] > 1, level 1 of a frame
  * whose size is 3 mod 4, frames of 2^31 pixels or more.  PHOVO_E_INVALID: no intrinsics, P < 1, bad sizes or level,
  * unknown depth type, no output.  Pairs run in chunks whose winner keys, validity flags and level records (5 B per
  * level pixel, + 20 B above level 0) fit in half of the L2. */
@@ -303,9 +312,25 @@ int phovo_batch_eval_normal_equations(phovo_ctx* ctx, int num_pairs, int rows, i
                                       const uint8_t* gray1, const double* states /* [P][6] */, int level,
                                       double* H /* [P][21] */, double* g /* [P][6] */, double* cost /* [P] */,
                                       int32_t* num_valid /* [P] */);
+/* phovo_batch_eval_normal_equations for the photometric + depth solver (PHOVO_MODE_BIOBJECTIVE).  depth1 [P][rows][cols]
+ * is the target depth, same type / scale as depth0, host or device like the frames.  For pair p it returns what
+ * phovo_eval_normal_equations(ctx, level, states[p]) returns after phovo_set_source(gray0[p], depth0[p]),
+ * phovo_set_target(gray1[p]) and phovo_set_target_depth(depth1[p]): H and g of the stacked 2N-row system (intensity and
+ * depth rows, the reference's row aliasing included: kernels_align.cu, k_winner_bi), cost = 0.5 sum over the 2N
+ * residual slots, num_valid = valid source pixels.  Agreement is to rounding; num_valid is exact.  Inputs, outputs,
+ * blocking behaviour, determinism and the other errors are those of phovo_batch_eval_normal_equations.  Pairs run in
+ * chunks whose 2N winner keys, validity flags, target depth and its gradients (33 B per level pixel, + 20 B above level 0)
+ * fit in half of the L2.  PHOVO_E_INVALID: depth1 NULL.  Other modes ignore depth1 and forward to
+ * phovo_batch_eval_normal_equations (Ceres mode: PHOVO_E_UNSUPPORTED). */
+int phovo_batch_eval_normal_equations_with_target_depth(phovo_ctx* ctx, int num_pairs, int rows, int cols,
+                                                        const uint8_t* gray0, const void* depth0, int depth_type,
+                                                        double depth_scale, const uint8_t* gray1, const void* depth1,
+                                                        const double* states /* [P][6] */, int level,
+                                                        double* H /* [P][21] */, double* g /* [P][6] */,
+                                                        double* cost /* [P] */, int32_t* num_valid /* [P] */);
 /* The batch entries keep what they allocate between calls: the packed level store, the slots' arena (up to half of the
  * free device memory for frames with large active levels), the pool's contexts, pinned result buffers, the warpImage
- * keys and staging buffers, the keys, level records, partial sums and results of phovo_batch_eval_normal_equations.
+ * keys and staging buffers, the keys, level records, target depths, partial sums and results of the batched normal equations.
  * This frees all of it (blocks until the device is idle); the next batch call allocates again.  Debug flags and the
  * record-stats switch return to their defaults. */
 int phovo_batch_release_memory(phovo_ctx* ctx);

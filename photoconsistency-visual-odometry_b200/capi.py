@@ -97,6 +97,8 @@ SIGNATURES = {
     "phovo_batch_align_with_target_depth": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp, _vp]),
     "phovo_batch_last_path": (C.c_int, [_vp]),
     "phovo_batch_align_device": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp]),
+    "phovo_batch_align_device_with_target_depth": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, _vp,
+                                                             _vp, _vp, _vp]),
     "phovo_batch_set_record_stats": (C.c_int, [_vp, C.c_int]),
     "phovo_batch_get_iter_stats": (C.c_int, [_vp, C.c_int, C.c_int, _stp]),
     "phovo_batch_num_iter_stats": (C.c_int, [_vp, C.c_int]),
@@ -105,6 +107,8 @@ SIGNATURES = {
                                          _vp, _vp, _vp, _vp]),
     "phovo_batch_eval_normal_equations": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, _vp,
                                                     C.c_int, _vp, _vp, _vp, _vp]),
+    "phovo_batch_eval_normal_equations_with_target_depth": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double,
+                                                                      _vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp]),
     "phovo_batch_release_memory": (C.c_int, [_vp]),
     "phovo_batch_get_last_h2d_bytes": (C.c_int, [_vp, C.POINTER(C.c_uint64)]),
     "phovo_synchronize": (C.c_int, [_vp]),

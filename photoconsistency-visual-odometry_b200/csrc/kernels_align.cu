@@ -195,47 +195,9 @@ __global__ void __launch_bounds__(kBlock) k_winner_bi(LevelParams L, LevelPtrs P
   }
 }
 
-// Jacobian row k of the stacked 2N-row system of the photometric + depth solver (see the comment
-// above k_winner_bi); returns false for a zero row.  CG: read the validity flags with ld.global.cg
-// (they were written by other SMs inside the same cooperative launch).
-// Row of pixel p (depth row or intensity row) from values already loaded: d = D0[p], (gx, gy) = the gradient of the
-// target intensity (intensity row) or of the target depth / max_depth (depth row) at index p.
-__device__ __forceinline__ void bi_jacobian_core(const LevelParams& L, const Pose& T, double spsr, double spcr, double gain,
-                                                 int p, bool depth_row, double d, double gx, double gy, double J[6]) {
-  const int r = p / L.cols, c = p - r * L.cols;
-  const double px = ((double)c - L.ox) * d * L.inv_fx, py = ((double)r - L.oy) * d * L.inv_fy;
-  const double q0 = fma(T.R00, px, fma(T.R01, py, T.R02 * d));
-  const double q1 = fma(T.R10, px, fma(T.R11, py, T.R12 * d));
-  const double q2 = fma(T.R20, px, fma(T.R21, py, T.R22 * d));
-  const double X = q0 + T.x, Y = q1 + T.y;
-  const double iz = 1.0 / (q2 + T.z);
-  // d(R p)/d(yaw, pitch, roll), BiObjective.h:364-377 in closed form
-  const double Zp = -fma(spsr, py, fma(spcr, d, T.cp * px));
-  const double dp0 = T.cy * q2, dp1 = T.sy * q2;
-  const double dr0 = fma(T.R02, py, -(T.R01 * d)), dr1 = fma(T.R12, py, -(T.R11 * d)), dr2 = fma(T.R22, py, -(T.R21 * d));
-  // v = gradient * projection Jacobian (:380-400), then v * jacobianRt
-  const double v0 = gx * L.fx * iz, v1 = gy * L.fy * iz;
-  const double v2 = -(fma(gx * L.fx, X, gy * L.fy * Y) * iz * iz);
-  J[0] = v0; J[1] = v1; J[2] = v2;
-  J[3] = fma(v1, q0, -(v0 * q1));
-  J[4] = fma(v0, dp0, fma(v1, dp1, v2 * Zp));
-  J[5] = fma(v0, dr0, fma(v1, dr1, v2 * dr2));
-  if (depth_row) {   // gain * (v * jacobianRt - jacobianRt_z), :404-414
-    J[0] = gain * J[0]; J[1] = gain * J[1]; J[2] = gain * (J[2] - 1.);
-    J[3] = gain * J[3]; J[4] = gain * (J[4] - Zp); J[5] = gain * (J[5] - dr2);
-  }
-}
-
-// Which pixel's row is Jacobian row k of the stacked 2N-row system (see the comment above k_winner_bi): vk = pixel k is
-// valid (false for k >= N), vh = pixel k/2 is valid.  Returns the pixel or -1 for a zero row.
-__device__ __forceinline__ int bi_row_owner(int k, bool vk, bool vh, bool* depth_row) {
-  *depth_row = false;
-  if (k > 0 && vk) return k;
-  if ((k & 1) == 0 && vh) { *depth_row = true; return k >> 1; }
-  return -1;
-}
-
-// Jacobian row k, loads included (the stream / graph drivers).
+// Jacobian row k of the stacked 2N-row system of the photometric + depth solver (see the comment above k_winner_bi;
+// bi_row_owner and bi_jacobian_core are in phovo_device.cuh), loads included (the stream / graph drivers); returns
+// false for a zero row.
 __device__ __forceinline__ bool bi_jacobian_row(const LevelParams& L, const LevelPtrs& P, const Pose& T, double spsr, double spcr,
                                                 double gain, int n, int k, double J[6]) {
   bool depth_row;

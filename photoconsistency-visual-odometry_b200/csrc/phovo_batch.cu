@@ -130,6 +130,8 @@ struct phovo_batch_state {
     DeviceArray<PoseDev> poses;
     DeviceArray<double> out;                           // [P][21] H, [P][6] g, [P] cost
     DeviceArray<int32_t> nvalid;
+    // photometric + depth solver: the chunk's target depth at the level (D1, its gradients), per-tile sums and gains
+    DeviceArray<double> d1, gxd, gyd, sums, gain;
   } eval;
 
   // device copies of one chunk of host frames, for warpImage and the normal equations alike
@@ -714,6 +716,27 @@ extern "C" int phovo_batch_align_device(phovo_ctx* ctx, int num_pairs, int rows,
                     initial_states, states, iters, log_cap ? r.log.get() : nullptr, log_cap ? r.log_counts.get() : nullptr);
 }
 
+extern "C" int phovo_batch_align_device_with_target_depth(phovo_ctx* ctx, int num_pairs, int rows, int cols, const uint8_t* gray0,
+                                                          const void* depth0, int depth_type, double depth_scale, const uint8_t* gray1,
+                                                          const void* depth1, const double* initial_states, double* states,
+                                                          int32_t* iters) {
+  if (!ctx || !gray0 || !depth0 || !gray1 || !depth1 || !states || !iters) return PHOVO_E_INVALID;
+  if (depth_type < 0 || depth_type > 2) return ctx->fail(PHOVO_E_INVALID, "unknown depth_type");
+  if (ctx->cfg.mode != PHOVO_MODE_BIOBJECTIVE)      // the other solvers ignore the target depth, like the reference (AN:484)
+    return phovo_batch_align_device(ctx, num_pairs, rows, cols, gray0, depth0, depth_type, depth_scale, gray1, initial_states, states, iters);
+  CK(cudaSetDevice(ctx->device));
+  phovo_batch_state* b; int rc = get_state(ctx, &b);
+  if (rc) return rc;
+  // the pool (< 24 pairs) or the slot waves, as phovo_batch_align_device takes them for the other solvers: synchronous;
+  // results go to the caller's device arrays through host temporaries
+  std::vector<double> hs((size_t)num_pairs * 6); std::vector<int32_t> hi((size_t)num_pairs * PHOVO_MAX_LEVELS);
+  if ((rc = batch_other(ctx, b, num_pairs, rows, cols, gray0, depth0, depth_type, depth_scale, gray1, depth1, initial_states, hs.data(), hi.data()))) return rc;
+  CK(cudaMemcpyAsync(states, hs.data(), sizeof(double) * hs.size(), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(iters, hi.data(), sizeof(int32_t) * hi.size(), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return PHOVO_OK;
+}
+
 extern "C" int phovo_batch_align(phovo_ctx* ctx, int num_pairs, int rows, int cols, const uint8_t* gray0,
                                  const void* depth0, int depth_type, double depth_scale, const uint8_t* gray1,
                                  const double* initial_states, double* states, int32_t* iterations) {
@@ -963,28 +986,25 @@ extern "C" int phovo_batch_warp_image(phovo_ctx* ctx, int num_pairs, int rows, i
 // ---------------------------------------------------------------------------------------------
 // Normal equations of many pairs at given states (kernels_eval.cu): what phovo_eval_normal_equations gives pair by pair
 // ---------------------------------------------------------------------------------------------
-// Pairs per chunk: the chunk's winner keys (4 B per pixel), validity flags (1 B) and, above level 0, its level records
-// fit in half of the L2, so that the two passes find them there (640x480 level 0 on a 126 MB L2: 41 pairs).
-static int eval_chunk_pairs(const phovo_batch_state* b, size_t n, unsigned long long record_bytes, int num_pairs) {
-  const size_t fit = (size_t)std::max(b->l2_bytes, 1) / 2 / (n * (sizeof(uint32_t) + 1) + record_bytes);
+// Pairs per chunk: the chunk's winner keys (4 B per pixel; 8 B for the 2N slots of the photometric + depth solver, which
+// also keeps D1, GxD and GyD: 24 B), validity flags (1 B) and, above level 0, its level records fit in half of the L2,
+// so that the passes find them there (640x480 level 0 on a 126 MB L2: 41 pairs, 6 for the photometric + depth solver).
+static int eval_chunk_pairs(const phovo_batch_state* b, size_t n, size_t px_bytes, unsigned long long record_bytes, int num_pairs) {
+  const size_t fit = (size_t)std::max(b->l2_bytes, 1) / 2 / (n * px_bytes + record_bytes);
   return (int)std::max<size_t>(1, std::min<size_t>({fit, (size_t)num_pairs, 65535}));
 }
 
-extern "C" int phovo_batch_eval_normal_equations(phovo_ctx* ctx, int num_pairs, int rows, int cols, const uint8_t* gray0,
-                                                 const void* depth0, int depth_type, double depth_scale, const uint8_t* gray1,
-                                                 const double* states, int level, double* H, double* g, double* cost,
-                                                 int32_t* num_valid) {
-  if (!ctx) return PHOVO_E_INVALID;
-  if (!gray0 || !depth0 || !gray1 || !states) return ctx->fail(PHOVO_E_INVALID, "gray0, depth0, gray1 and states are required");
-  if (!ctx->have_K) return ctx->fail(PHOVO_E_INVALID, "SetIntrinsicMatrix has not been called");
-  if (ctx->cfg.mode == PHOVO_MODE_CERES || ctx->cfg.mode == PHOVO_MODE_BIOBJECTIVE)
-    return ctx->fail(PHOVO_E_UNSUPPORTED, "batched normal equations: analytic modes only");
+// depth1 == nullptr: the analytic modes (k_eval_*); otherwise the photometric + depth solver (k_eval_*_bi)
+static int eval_normal_equations(phovo_ctx* ctx, int num_pairs, int rows, int cols, const uint8_t* gray0, const void* depth0,
+                                 int depth_type, double depth_scale, const uint8_t* gray1, const void* depth1,
+                                 const double* states, int level, double* H, double* g, double* cost, int32_t* num_valid) {
   if (num_pairs < 1 || rows < 1 || cols < 1 || level < 0 || level >= ctx->cfg.num_levels)
     return ctx->fail(PHOVO_E_INVALID, "bad batch size, image size or level");
   if (depth_type < 0 || depth_type > 2) return ctx->fail(PHOVO_E_INVALID, "unknown depth_type");
   if (!H && !g && !cost && !num_valid) return ctx->fail(PHOVO_E_INVALID, "no output requested");
   const size_t n = (size_t)rows * cols;
   if (n > (size_t)INT32_MAX) return ctx->fail(PHOVO_E_UNSUPPORTED, "batched normal equations: frames of 2^31 pixels or more");
+  const bool bi = depth1 != nullptr;
   BatchParams bp;
   memset(&bp, 0, sizeof(bp));
   bp.rows = rows; bp.cols = cols; bp.num_active = 1; bp.mode = ctx->cfg.mode;
@@ -1007,21 +1027,37 @@ extern "C" int phovo_batch_eval_normal_equations(phovo_ctx* ctx, int num_pairs, 
   E.record_bytes = record_bytes; E.off_I0 = bp.off_I0[0]; E.off_I1 = bp.off_I1[0]; E.off_D0 = bp.off_D0[0];
   const int src = src_type_of_depth(depth_type);
   const size_t delt = depth_elt(depth_type);
-  const int chunk = eval_chunk_pairs(b, (size_t)ln, records ? record_bytes : 0, num_pairs);
+  const size_t slots = bi ? 2 : 1;                  // residual slots per level pixel
+  const size_t px_bytes = slots * sizeof(uint32_t) + 1 + (bi ? 3 * sizeof(double) : 0);
+  const int chunk = eval_chunk_pairs(b, (size_t)ln, px_bytes, records ? record_bytes : 0, num_pairs);
   const size_t ck = (size_t)chunk * ln;
   auto& v = b->eval;
+  EvalTargetDepth D;
+  memset(&D, 0, sizeof(D));
+  if (bi) {
+    D.rows = rows; D.cols = cols; D.level = level; D.depth_scale = E.depth_scale;
+    D.inv_max_depth = 1. / ctx->cfg.max_depth;    // as phovo_set_target_depth: k_scale by 1 / max_depth, then k_scharr_store
+    D.ks0 = 3.; D.ks1 = 10.;
+    if (ctx->cfg.grad_scale[level] != 1.) { D.ks0 *= ctx->cfg.grad_scale[level]; D.ks1 *= ctx->cfg.grad_scale[level]; }
+    D.tiles2 = (int)((2 * (size_t)ln + kEvalTile - 1) / kEvalTile);
+    CK(v.d1.ensure(ck)); CK(v.gxd.ensure(ck)); CK(v.gyd.ensure(ck));
+    CK(v.sums.ensure((size_t)chunk * E.tiles * 2));
+    CK(v.gain.ensure((size_t)chunk));
+    D.D1 = v.d1.get(); D.GxD = v.gxd.get(); D.GyD = v.gyd.get(); D.sums = v.sums.get(); D.gain = v.gain.get();
+  }
   bool fresh;
-  CK(v.keys.ensure(ck, &fresh));
+  CK(v.keys.ensure(ck * slots, &fresh));
   if (fresh) v.keys_clean = false;
   CK(v.valid.ensure(ck));
-  CK(v.partials.ensure((size_t)chunk * E.tiles * PHOVO_ACC_STRIDE));
+  CK(v.partials.ensure((size_t)chunk * (bi ? D.tiles2 : E.tiles) * PHOVO_ACC_STRIDE));
   if (records) CK(v.store.ensure((size_t)chunk * record_bytes));
   CK(v.states.ensure((size_t)num_pairs * 6));
   CK(v.poses.ensure((size_t)num_pairs));
   CK(v.out.ensure((size_t)num_pairs * 28));
   CK(v.nvalid.ensure((size_t)num_pairs));
-  const bool in_dev = is_device_pointer(gray0) && is_device_pointer(depth0) && is_device_pointer(gray1);
-  const Frames in = {gray0, gray1, depth0, nullptr};
+  const bool in_dev = is_device_pointer(gray0) && is_device_pointer(depth0) && is_device_pointer(gray1) &&
+                      (!bi || is_device_pointer(depth1));
+  const Frames in = {gray0, gray1, depth0, depth1};
   if (!v.keys_clean) CK(cudaMemsetAsync(v.keys.get(), 0, v.keys.capacity() * sizeof(uint32_t), ctx->stream));
   v.keys_clean = false;   // until every launch below has been enqueued
   CK(cudaMemcpyAsync(v.states.get(), states, sizeof(double) * 6 * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
@@ -1039,8 +1075,14 @@ extern "C" int phovo_batch_eval_normal_equations(phovo_ctx* ctx, int num_pairs, 
       E.gray0 = f.gray0; E.gray1 = f.gray1; E.depth = f.depth0;
     }
     E.poses = v.poses.get() + p0;
-    ctx->launches += launch_eval_normal_equations(ctx->stream, E, src, records, np, dH + (size_t)p0 * 21, dg + (size_t)p0 * 6,
-                                                  dcost + p0, v.nvalid.get() + p0);
+    if (bi) {
+      D.depth1 = f.depth1;
+      ctx->launches += launch_eval_normal_equations_bi(ctx->stream, E, D, src, records, np, dH + (size_t)p0 * 21, dg + (size_t)p0 * 6,
+                                                       dcost + p0, v.nvalid.get() + p0);
+    } else {
+      ctx->launches += launch_eval_normal_equations(ctx->stream, E, src, records, np, dH + (size_t)p0 * 21, dg + (size_t)p0 * 6,
+                                                    dcost + p0, v.nvalid.get() + p0);
+    }
     CK(cudaGetLastError());
   }
   v.keys_clean = true;
@@ -1050,4 +1092,33 @@ extern "C" int phovo_batch_eval_normal_equations(phovo_ctx* ctx, int num_pairs, 
   if (num_valid) CK(cudaMemcpyAsync(num_valid, v.nvalid.get(), sizeof(int32_t) * (size_t)num_pairs, cudaMemcpyDefault, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return PHOVO_OK;
+}
+
+extern "C" int phovo_batch_eval_normal_equations(phovo_ctx* ctx, int num_pairs, int rows, int cols, const uint8_t* gray0,
+                                                 const void* depth0, int depth_type, double depth_scale, const uint8_t* gray1,
+                                                 const double* states, int level, double* H, double* g, double* cost,
+                                                 int32_t* num_valid) {
+  if (!ctx) return PHOVO_E_INVALID;
+  if (!gray0 || !depth0 || !gray1 || !states) return ctx->fail(PHOVO_E_INVALID, "gray0, depth0, gray1 and states are required");
+  if (!ctx->have_K) return ctx->fail(PHOVO_E_INVALID, "SetIntrinsicMatrix has not been called");
+  if (ctx->cfg.mode == PHOVO_MODE_CERES || ctx->cfg.mode == PHOVO_MODE_BIOBJECTIVE)
+    return ctx->fail(PHOVO_E_UNSUPPORTED, "batched normal equations: analytic modes only");
+  return eval_normal_equations(ctx, num_pairs, rows, cols, gray0, depth0, depth_type, depth_scale, gray1, nullptr, states, level,
+                               H, g, cost, num_valid);
+}
+
+extern "C" int phovo_batch_eval_normal_equations_with_target_depth(phovo_ctx* ctx, int num_pairs, int rows, int cols,
+                                                                   const uint8_t* gray0, const void* depth0, int depth_type,
+                                                                   double depth_scale, const uint8_t* gray1, const void* depth1,
+                                                                   const double* states, int level, double* H, double* g,
+                                                                   double* cost, int32_t* num_valid) {
+  if (!ctx) return PHOVO_E_INVALID;
+  if (!gray0 || !depth0 || !gray1 || !depth1 || !states)
+    return ctx->fail(PHOVO_E_INVALID, "gray0, depth0, gray1, depth1 and states are required");
+  if (ctx->cfg.mode != PHOVO_MODE_BIOBJECTIVE)      // the other solvers ignore the target depth, like the reference (AN:484)
+    return phovo_batch_eval_normal_equations(ctx, num_pairs, rows, cols, gray0, depth0, depth_type, depth_scale, gray1, states,
+                                             level, H, g, cost, num_valid);
+  if (!ctx->have_K) return ctx->fail(PHOVO_E_INVALID, "SetIntrinsicMatrix has not been called");
+  return eval_normal_equations(ctx, num_pairs, rows, cols, gray0, depth0, depth_type, depth_scale, gray1, depth1, states, level,
+                               H, g, cost, num_valid);
 }

@@ -68,12 +68,31 @@ struct EvalLevel {
   uint8_t* valid;                        // [pairs][n]: the exact warp accepted the source pixel
   double* partials;                      // [pairs][tiles][PHOVO_ACC_STRIDE]
 };
+// Photometric + depth solver (PHOVO_MODE_BIOBJECTIVE): the target depth of a chunk at the level, and what the kernels
+// derive from it.  The level images are built from the caller's full-resolution frames with the per-pair path's
+// arithmetic (phovo_level.cuh), so D1, GxD and GyD are the per-pair context's bits.
+struct EvalTargetDepth {
+  const void* depth1;                    // [pairs][rows][cols] of pair 0, full resolution, element type of depth0
+  int rows, cols, level;                 // full-resolution size, pyramid level
+  double depth_scale;                    // u16 only (1 otherwise)
+  double inv_max_depth;                  // 1 / max_depth: GxD, GyD are the Scharr of D1 / max_depth (BiObjective.h:224-237)
+  double ks0, ks1;                       // Scharr kernel scaled by the level's imageGradientsScalingFactor
+  int tiles2;                            // ceil(2 rows * cols / kEvalTile) at the level: tiles of the 2N residual slots
+  double* D1; double* GxD; double* GyD;  // [pairs][n] at the level
+  double* sums;                          // [pairs][tiles][2]: sum of the I1 tap sums, sum of D1 per tile of pixels
+  double* gain;                          // [pairs]: mean(I1) / mean(D1) at the level (BiObjective.h:299)
+};
+
 // Pose (rotation and trig values) of every state, as the per-pair path derives it: poses[p] from states[p * 6].
 int launch_eval_poses(cudaStream_t stream, const double* states, int num_pairs, PoseDev* poses);
 // Winner pass, accumulate pass (clears the keys) and the per-pair sums into H [21], g [6], cost, num_valid of pairs
 // [0, num_pairs) of E; `out_*` point at the chunk's first pair.  Returns the number of launches.
 int launch_eval_normal_equations(cudaStream_t stream, const EvalLevel& E, int src_type /* SRC_*; level 0 */, bool records,
                                  int num_pairs, double* out_H, double* out_g, double* out_cost, int32_t* out_valid);
+// The same for the photometric + depth solver: target depth set-up, gain, winner pass over 2N slots (E.keys [pairs][2n]),
+// accumulate pass over the 2N Jacobian rows (E.partials [pairs][D.tiles2]) and the per-pair sums.
+int launch_eval_normal_equations_bi(cudaStream_t stream, const EvalLevel& E, const EvalTargetDepth& D, int src_type, bool records,
+                                    int num_pairs, double* out_H, double* out_g, double* out_cost, int32_t* out_valid);
 bool batch_level_is_small(int rows, int cols);
 cudaError_t batch_align_prepare();
 

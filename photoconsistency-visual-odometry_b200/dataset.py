@@ -330,14 +330,17 @@ def run_visual_odometry(odometry, source, trajectory_file=None, depth_scaling_fa
             return poses
         pose = np.eye(4)
         k = 0
+        prev_depth = None
         for cur in it:
             k += 1
-            d, s = depth_of(prev)
+            d, s = depth_of(prev) if prev_depth is None else prev_depth
             if promote and k > 1:
                 odometry.PromoteTargetToSource(d, depth_scale=s)          # frame k-1's target pyramid is frame k's source
             else:
                 odometry.SetSourceFrame(prev[IntensityCameraIdentifier].GetData(), d, depth_scale=s)
-            odometry.SetTargetFrame(cur[IntensityCameraIdentifier].GetData())
+            # the app passes the current depth too; only the photometric + depth solver reads it
+            prev_depth = depth_of(cur)
+            odometry.SetTargetFrame(cur[IntensityCameraIdentifier].GetData(), prev_depth[0], depth_scale=prev_depth[1])
             odometry.SetInitialStateVector(state0)
             odometry.Optimize()
             Rt = odometry.GetOptimalRigidTransformationMatrix()

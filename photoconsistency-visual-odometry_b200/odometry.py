@@ -278,10 +278,26 @@ class CPhotoconsistencyOdometryCuda:
                                               states.ctypes.data, iters.ctypes.data))
         return states, iters
 
-    def BatchAlignDevice(self, gray0, depth0, gray1, states_out, iters_out, initial_states=None, depth_scale=1.0):
+    def BatchAlignDevice(self, gray0, depth0, gray1, states_out, iters_out, initial_states=None, depth_scale=1.0, depth1=None):
         """All torch device tensors; asynchronous on the context stream (torch's current stream of the
-        tensors' device: inputs are ordered after their producers, outputs before their consumers)."""
+        tensors' device: inputs are ordered after their producers, outputs before their consumers).
+        `depth1` (target depth, depth0's shape and element type) is read by the photometric + depth solver only; with it
+        that solver's pairs go through the pool or the slot waves and the call returns once the outputs are written."""
         import torch
+        if depth1 is not None:
+            gray0, depth0, gray1, depth1 = (self._dense(a) for a in (gray0, depth0, gray1, depth1))
+            self._follow_producer_stream(gray0, depth0, gray1, depth1)
+            P, R, Cc = tuple(gray0.shape)
+            dtype = self._batch_depth_type(depth0)
+            if tuple(depth0.shape) != (P, R, Cc) or tuple(gray1.shape) != (P, R, Cc) or tuple(depth1.shape) != (P, R, Cc):
+                raise ValueError("gray0, depth0, gray1 and depth1 must all be [P, rows, cols]")
+            if self._batch_depth_type(depth1) != dtype:
+                raise TypeError("depth1 must have the element type of depth0 (one depth type is passed for both)")
+            self._check(self._L.phovo_batch_align_device_with_target_depth(
+                self._h, P, R, Cc, gray0.data_ptr(), depth0.data_ptr(), dtype, float(depth_scale), gray1.data_ptr(),
+                depth1.data_ptr(), None if initial_states is None else initial_states.data_ptr(),
+                states_out.data_ptr(), iters_out.data_ptr()))
+            return
         self._follow_producer_stream(gray0)
         P, R, Cc = tuple(gray0.shape)
         dtype = {torch.float64: capi.DEPTH_F64, torch.float32: capi.DEPTH_F32, torch.uint16: capi.DEPTH_U16,
@@ -331,19 +347,27 @@ class CPhotoconsistencyOdometryCuda:
         return dict(warped=warped, diff=diff, num_landed=landed, sum_abs_diff=sums,
                     mean_abs_diff=None if sums is None else sums / np.maximum(landed, 1))
 
-    def BatchEvalNormalEquations(self, gray0, depth0, gray1, states, level=0, depth_scale=1.0):
+    def BatchEvalNormalEquations(self, gray0, depth0, gray1, states, level=0, depth_scale=1.0, depth1=None):
         """The normal equations of P pairs at the given states, at any pyramid level (built by the call, configured
         iterations or not): what EvalNormalEquations(level, states[p]) returns after SetSourceFrame(gray0[p], depth0[p])
         and SetTargetFrame(gray1[p]), to rounding.  gray0 / gray1 u8 [P,R,C] and depth0 [P,R,C] (f64 / f32 metres or
         u16 raw * depth_scale), numpy or torch, all on the host or all on the device; states [P,6] (numpy or torch).
         Returns a dict of numpy arrays: `H` [P,6,6] = J^T J (symmetric), `g` [P,6] = J^T r, `cost` [P] = 0.5 |r|^2 and
         `num_valid` [P].  J scales the image gradients by the configured imageGradientsScalingFactor and, in mode 0,
-        carries the reference's temp11 term (AN:253): H is the solver's J^T J, not a calibrated information matrix."""
-        gray0, depth0, gray1 = (self._dense(a) for a in (gray0, depth0, gray1))
+        carries the reference's temp11 term (AN:253): H is the solver's J^T J, not a calibrated information matrix.
+        `depth1` [P,R,C] (target depth, depth0's element type) is what the photometric + depth solver (MODE_BIOBJECTIVE)
+        needs: with it the results are EvalNormalEquations' after SetTargetFrame(gray1[p], depth1[p]) as well, i.e. of
+        the stacked intensity + depth system; the other modes ignore it."""
+        gray0, depth0, gray1, depth1 = (self._dense(a) for a in (gray0, depth0, gray1, depth1))
         P, R, Cc = tuple(gray0.shape)
         dtype = self._batch_depth_type(depth0)
         if tuple(depth0.shape) != (P, R, Cc) or tuple(gray1.shape) != (P, R, Cc):
             raise ValueError("gray0, depth0 and gray1 must all be [P, rows, cols]")
+        if depth1 is not None:
+            if tuple(depth1.shape) != (P, R, Cc):
+                raise ValueError("depth1 must be [P, rows, cols] like depth0")
+            if self._batch_depth_type(depth1) != dtype:
+                raise TypeError("depth1 must have the element type of depth0 (one depth type is passed for both)")
         if not isinstance(gray0, np.ndarray) and gray0.is_cuda:
             self._follow_producer_stream(gray0)
         if getattr(states, "is_cuda", False):
@@ -357,9 +381,14 @@ class CPhotoconsistencyOdometryCuda:
         g = np.zeros((P, 6))
         cost = np.zeros(P)
         nv = np.zeros(P, np.int32)
-        self._check(self._L.phovo_batch_eval_normal_equations(self._h, P, R, Cc, capi._ptr(gray0), capi._ptr(depth0), dtype,
-                                                              float(depth_scale), capi._ptr(gray1), capi._ptr(states), int(level),
-                                                              Hu.ctypes.data, g.ctypes.data, cost.ctypes.data, nv.ctypes.data))
+        if depth1 is not None:
+            self._check(self._L.phovo_batch_eval_normal_equations_with_target_depth(
+                self._h, P, R, Cc, capi._ptr(gray0), capi._ptr(depth0), dtype, float(depth_scale), capi._ptr(gray1),
+                capi._ptr(depth1), capi._ptr(states), int(level), Hu.ctypes.data, g.ctypes.data, cost.ctypes.data, nv.ctypes.data))
+        else:
+            self._check(self._L.phovo_batch_eval_normal_equations(self._h, P, R, Cc, capi._ptr(gray0), capi._ptr(depth0), dtype,
+                                                                  float(depth_scale), capi._ptr(gray1), capi._ptr(states), int(level),
+                                                                  Hu.ctypes.data, g.ctypes.data, cost.ctypes.data, nv.ctypes.data))
         iu = np.triu_indices(6)
         H = np.zeros((P, 6, 6))
         H[:, iu[0], iu[1]] = Hu
@@ -408,7 +437,9 @@ class CPhotoconsistencyOdometryCuda:
         states = torch.zeros((n - 1, 6), dtype=torch.float64, device=dev)
         iters = torch.zeros((n - 1, capi.MAXL), dtype=torch.int32, device=dev)
         self.SetStream(torch.cuda.current_stream(dev).cuda_stream)
-        self.BatchAlignDevice(g[:-1], d[:-1], g[1:], states, iters, depth_scale=depth_scale)   # overlapping views, no copies
+        # the photometric + depth solver also reads the target depth: frame k+1's depth for pair k
+        d1 = d[1:] if self.GetConfig().mode == capi.MODE_BIOBJECTIVE else None
+        self.BatchAlignDevice(g[:-1], d[:-1], g[1:], states, iters, depth_scale=depth_scale, depth1=d1)   # overlapping views, no copies
         st, it = states.cpu().numpy(), iters.cpu().numpy()
         rts = np.stack([capi.state_to_rt(s) for s in st])
         poses = np.tile(np.eye(4), (n, 1, 1))
@@ -424,7 +455,7 @@ class CPhotoconsistencyOdometryCuda:
             diag.update({k: s[k] for k in ("num_landed", "sum_abs_diff", "mean_abs_diff")})
         if information_level is not None:
             diag.update(self.BatchEvalNormalEquations(g[:-1], d[:-1], g[1:], states, level=int(information_level),
-                                                      depth_scale=depth_scale))
+                                                      depth_scale=depth_scale, depth1=d1))
         return st, it, poses, diag
 
     def BatchKernelTimes(self):

@@ -200,8 +200,9 @@ int64_t phovo_launch_count(const phovo_ctx* ctx);
 /* use a caller-provided stream (e.g. torch's current stream) instead of the ctx-owned one; required
  * for ordering when device-resident inputs are produced on that stream (see phovo_set_source) */
 int phovo_set_stream(phovo_ctx* ctx, void* cuda_stream);
-/* 0: plain stream launches with host-side convergence polling; 1 (default): whole Optimize as one
- * CUDA graph with a conditional WHILE node per level (no host sync inside) */
+/* enable != 0: path 1 of phovo_set_execution (whole Optimize as one CUDA graph with a conditional
+ * WHILE node per level, no host sync inside); 0: path 0 (plain stream launches with host-side
+ * convergence polling).  The default is path 2, see phovo_set_execution. */
 int phovo_set_use_graph(phovo_ctx* ctx, int enable);
 /* How phovo_optimize drives the iteration loop of a level (results agree to rounding; each path is
  * bitwise reproducible run to run):
@@ -214,8 +215,9 @@ int phovo_set_use_graph(phovo_ctx* ctx, int enable);
  * device the next one down is used (phovo_graph_error tells why). */
 int phovo_set_execution(phovo_ctx* ctx, int path);
 int phovo_last_optimize_path(const phovo_ctx* ctx);
-/* 1 if the last phovo_optimize ran as the CUDA graph (0: plain launches; see phovo_graph_error) */
+/* 1 if the last phovo_optimize ran as the CUDA graph (path 1), else 0 */
 int phovo_last_optimize_used_graph(const phovo_ctx* ctx);
+/* why the last path that failed on this context (graph, cooperative or cluster launch) was given up; "" if none */
 const char* phovo_graph_error(const phovo_ctx* ctx);
 /* build every pyramid level, not only those with max_num_iterations > 0 (the reference builds all,
  * AN:474-490, but never reads the others); needed only to inspect them with phovo_get_level_image */

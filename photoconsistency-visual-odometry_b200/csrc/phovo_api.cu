@@ -281,7 +281,7 @@ static int create_context(int device, phovo_ctx** out, bool slot) {
     memset(&prop, 0, sizeof(prop));
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) { cudaGetLastError(); prop.multiProcessorCount = 0; prop.cooperativeLaunch = 0; }
     ctx->sm_count = prop.multiProcessorCount > 0 ? prop.multiProcessorCount : 1;
-    if (!prop.cooperativeLaunch) ctx->coop_broken = true;
+    if (!prop.cooperativeLaunch) ctx->failed_paths |= 1u << 2;
   }
   phovo_internal_default_config(&ctx->cfg);
   auto bail = [&](const char* what, cudaError_t err) {
@@ -430,7 +430,6 @@ extern "C" int phovo_set_stream(phovo_ctx* ctx, void* cuda_stream) {
 
 extern "C" int phovo_set_use_graph(phovo_ctx* ctx, int enable) {
   if (!ctx) return PHOVO_E_INVALID;
-  ctx->use_graph = enable != 0;
   ctx->execution = enable ? 1 : 0;
   return PHOVO_OK;
 }
@@ -438,7 +437,6 @@ extern "C" int phovo_set_use_graph(phovo_ctx* ctx, int enable) {
 extern "C" int phovo_set_execution(phovo_ctx* ctx, int path) {
   if (!ctx || path < 0 || path > 3) return PHOVO_E_INVALID;
   ctx->execution = path;
-  ctx->use_graph = path >= 1;
   return PHOVO_OK;
 }
 
@@ -573,6 +571,22 @@ static int ensure_log(phovo_ctx* ctx, int want) {
   return PHOVO_OK;
 }
 
+// The start of every solve: the inputs are complete, the log has room for a whole run, the optimize timer starts.  The
+// initial state is uploaded by the driver (upload_state), because the graph driver captures its own upload.
+static int begin_solve(phovo_ctx* ctx) {
+  int rc = ready_to_solve(ctx);
+  if (rc) return rc;
+  CK(cudaSetDevice(ctx->device));
+  if ((rc = ensure_log(ctx, total_iterations(ctx) + 1))) return rc;
+  ctx->setup_timed = false;
+  CK(cudaEventRecord(ctx->ev_time[2].get(), ctx->stream));
+  return PHOVO_OK;
+}
+
+static void upload_state(phovo_ctx* ctx) {
+  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
+}
+
 static int read_back(phovo_ctx* ctx) {
   const int cap = total_iterations(ctx);
   CK(cudaMemcpyAsync(ctx->h_pose.get(), ctx->d_pose.get(), sizeof(PoseDev), cudaMemcpyDeviceToHost, ctx->stream));
@@ -588,13 +602,38 @@ static int read_back(phovo_ctx* ctx) {
   return PHOVO_OK;
 }
 
+// The end of a row-sharded solve: the read-back, then whether a wait for a peer timed out.
+static int end_solve(phovo_ctx* ctx) {
+  const int rc = read_back(ctx);
+  if (ctx->xchg_own.get()) {
+    int err = 0;
+    CK(cudaMemcpy(&err, &ctx->xchg_own.get()->error, sizeof(int), cudaMemcpyDeviceToHost));
+    if (err) return ctx->fail(PHOVO_E_CUDA, "peer exchange timed out waiting for another rank");
+  }
+  return rc;
+}
+
+// What a driver returns when its path cannot run on this context: positive, so never a PHOVO_* code.  phovo_optimize
+// then starts the solve over on the next path down.
+static const int kPathUnavailable = 1;
+
+static bool path_failed(const phovo_ctx* ctx, int path) { return (ctx->failed_paths >> path) & 1u; }
+
+// A launch of `path` was refused: clears the launch error, keeps the reason for phovo_graph_error, marks the path so that
+// no later Optimize() on this context tries it, and drains the stream.
+static int path_unavailable(phovo_ctx* ctx, int path, const char* launch, cudaError_t e) {
+  cudaGetLastError();
+  ctx->path_note = std::string(launch) + " unavailable: " + cudaGetErrorString(e);
+  ctx->failed_paths |= 1u << path;
+  CK(cudaStreamSynchronize(ctx->stream));
+  return kPathUnavailable;
+}
+
 // Plain stream launches; the host polls the device-side termination flag every `poll` iterations.
 static int optimize_stream(phovo_ctx* ctx) {
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
+  upload_state(ctx);
   const int poll = 4;
-  for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {   // AN:502-503
-    const int M = ctx->cfg.max_num_iterations[level];
-    if (M <= 0) continue;   // AN:526: an empty pass, then the iteration test breaks (AN:383)
+  return for_each_level(ctx->cfg, [&](int level, int M) {
     const LevelParams L = ctx->level_params(level);
     const LevelPtrs P = ctx->level_ptrs(level);
     ctx->launches += launch_begin_level(ctx->stream, ctx->d_pose.get(), M);
@@ -612,9 +651,8 @@ static int optimize_stream(phovo_ctx* ctx) {
         if (ctx->h_pose.get()->done) break;
       }
     }
-  }
-  CK(cudaGetLastError());
-  return PHOVO_OK;
+    return PHOVO_OK;
+  });
 }
 
 // One CUDA graph for the whole Optimize(): set-state -> for each active level { begin-level ->
@@ -646,9 +684,7 @@ static int build_graph(phovo_ctx* ctx) {
   };
 
   CK(capture(g, true, [&] { launches_per_run += launch_set_state(ctx->stream, ctx->d_pose.get(), ctx->d_state_in.get(), ctx->state, ctx->log_cap()); }));
-  for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
-    const int M = ctx->cfg.max_num_iterations[level];
-    if (M <= 0) continue;
+  const int rc = for_each_level(ctx->cfg, [&](int level, int M) {
     const LevelParams L = ctx->level_params(level);
     const LevelPtrs P = ctx->level_ptrs(level);
     CK(capture(g, true, [&] { launches_per_run += launch_begin_level(ctx->stream, ctx->d_pose.get(), M); }));
@@ -670,13 +706,15 @@ static int build_graph(phovo_ctx* ctx) {
     }));
     ctx->graph_launches_per_iter = per_iter;
     tail = cond_node; have_tail = true;
-  }
+    return PHOVO_OK;
+  });
+  if (rc) return rc;
   ctx->graph_launches_fixed = launches_per_run;
   CK(cudaGraphInstantiate(&ctx->graph_exec, g, 0));
   return PHOVO_OK;
 }
 
-static int optimize_graph(phovo_ctx* ctx) {
+static int run_graph(phovo_ctx* ctx) {
   if (!ctx->graph_exec) {
     int rc = build_graph(ctx);
     if (rc) return rc;
@@ -684,136 +722,109 @@ static int optimize_graph(phovo_ctx* ctx) {
   memcpy(ctx->h_state_in.get(), ctx->state, sizeof(double) * 6);
   CK(cudaMemcpyAsync(ctx->d_state_in.get(), ctx->h_state_in.get(), sizeof(double) * 6, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaGraphLaunch(ctx->graph_exec, ctx->stream));
-  return PHOVO_OK;
+  return read_back(ctx);
 }
 
-// One cooperative persistent launch per active level: set-state, then for each level begin-level + loop kernel.
-static int optimize_coop(phovo_ctx* ctx, bool* unavailable) {
-  *unavailable = false;
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
-  for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {   // AN:502-503
-    const int M = ctx->cfg.max_num_iterations[level];
-    if (M <= 0) continue;
+// The graph driver reads back itself: when building, launching or running the graph fails, the context stops using
+// graphs and the solve starts over on plain launches.
+static int optimize_graph(phovo_ctx* ctx) {
+  const int rc = run_graph(ctx);
+  if (rc == PHOVO_OK || rc == PHOVO_E_NUMERIC) {
+    int iters = 0;
+    for (int l = 0; l < ctx->cfg.num_levels; ++l) iters += ctx->h_pose.get()->iters_per_level[l];
+    ctx->launches += ctx->graph_launches_fixed + (int64_t)iters * ctx->graph_launches_per_iter;
+    return rc;
+  }
+  ctx->failed_paths |= 1u << 1;
+  ctx->path_note = ctx->err;
+  ctx->invalidate_graph();
+  cudaGetLastError();
+  cudaStreamCaptureStatus st;
+  if (cudaStreamIsCapturing(ctx->stream, &st) == cudaSuccess && st != cudaStreamCaptureStatusNone) {
+    cudaGraph_t junk = nullptr;
+    cudaStreamEndCapture(ctx->stream, &junk);
+    if (junk) cudaGraphDestroy(junk);
+  }
+  cudaGetLastError();
+  return kPathUnavailable;
+}
+
+// One cooperative persistent launch per active level (path 2); path 3 runs a level that qualifies inside one
+// thread-block cluster instead.
+static int optimize_coop(phovo_ctx* ctx, int path) {
+  upload_state(ctx);
+  return for_each_level(ctx->cfg, [&](int level, int) {
     const LevelParams L = ctx->level_params(level);
     const LevelPtrs P = ctx->level_ptrs(level);
     // (no k_begin_level: the persistent kernel keeps iteration / done in registers and shared memory
     // and writes the whole PoseDev back when the level ends)
     int grid = 0; cudaError_t e = cudaSuccess;
-    if (ctx->execution == 3 && !ctx->cluster_broken) {      // small level: one thread-block cluster, cluster barriers
-      const int rcl = launch_level_cluster(ctx->stream, L, P, ctx->d_pose.get(), ctx->d_log.get(), &ctx->launch_state, &e);
-      if (rcl > 0) { ctx->launches += rcl; continue; }
-      if (rcl < 0) {
-        cudaGetLastError();
-        ctx->cluster_broken = true;
-        ctx->graph_error = std::string("cluster launch unavailable: ") + cudaGetErrorString(e);
+    if (path == 3 && !path_failed(ctx, 3)) {      // small level: one thread-block cluster, cluster barriers
+      const int n = launch_level_cluster(ctx->stream, L, P, ctx->d_pose.get(), ctx->d_log.get(), &ctx->launch_state, &e);
+      if (n > 0) { ctx->launches += n; return PHOVO_OK; }
+      if (n < 0) {   // refused: this level and the rest take path 2
+        const int r = path_unavailable(ctx, 3, "cluster launch", e);
+        if (r != kPathUnavailable) return r;
       }
     }
-    const int rc = launch_level_coop(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->d_log.get(), &ctx->launch_state, ctx->sm_count, &grid, &e);
-    if (rc < 0) {
-      cudaGetLastError();
-      ctx->graph_error = std::string("cooperative launch unavailable: ") + cudaGetErrorString(e);
-      *unavailable = true;
-      CK(cudaStreamSynchronize(ctx->stream));
-      return PHOVO_OK;
-    }
-    ctx->launches += rc;
-  }
-  CK(cudaGetLastError());
-  return PHOVO_OK;
+    const int n = launch_level_coop(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->d_log.get(), &ctx->launch_state, ctx->sm_count, &grid, &e);
+    if (n < 0) return path_unavailable(ctx, 2, "cooperative launch", e);
+    ctx->launches += n;
+    return PHOVO_OK;
+  });
+}
+
+// Ceres mode with the LM loop on the device: one cooperative launch per active level (CE:437).
+static int optimize_ceres_coop(phovo_ctx* ctx) {
+  upload_state(ctx);
+  return for_each_level(ctx->cfg, [&](int level, int) {
+    cudaError_t e = cudaSuccess;
+    const int n = launch_level_coop_ceres(ctx->stream, ctx->level_params(level), ctx->level_ptrs(level), ctx->d_pose.get(), ctx->partials.get(),
+                                          ctx->d_log.get(), lm_params(ctx->cfg, level), &ctx->launch_state, ctx->sm_count, &e);
+    if (n < 0) return path_unavailable(ctx, 2, "cooperative launch", e);
+    ctx->launches += n;
+    return PHOVO_OK;
+  });
 }
 
 static int optimize_ceres(phovo_ctx* ctx);
 
-// Ceres mode with the LM loop on the device: one cooperative launch per active level.
-static int optimize_ceres_coop(phovo_ctx* ctx, bool* unavailable) {
-  *unavailable = false;
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
-  for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
-    const int M = ctx->cfg.max_num_iterations[level];
-    if (!(M > 0)) continue;   // CE:437
-    const LevelParams L = ctx->level_params(level);
-    const LevelPtrs P = ctx->level_ptrs(level);
-    cudaError_t e = cudaSuccess;
-    const int rc = launch_level_coop_ceres(ctx->stream, L, P, ctx->d_pose.get(), ctx->partials.get(), ctx->d_log.get(), lm_params(ctx->cfg, level),
-                                           &ctx->launch_state, ctx->sm_count, &e);
-    if (rc < 0) {
-      cudaGetLastError();
-      ctx->graph_error = std::string("cooperative launch unavailable: ") + cudaGetErrorString(e);
-      *unavailable = true;
-      CK(cudaStreamSynchronize(ctx->stream));
-      return PHOVO_OK;
-    }
-    ctx->launches += rc;
-  }
-  CK(cudaGetLastError());
-  return PHOVO_OK;
+// The driver of this Optimize(): the path phovo_set_execution asks for, or the next one down that has not failed on this
+// context.  Analytic and photometric + depth solvers: 3 -> 2 -> 1 (graph) -> 0 (stream); the cooperative paths need a
+// world of one.  Ceres mode: 3 and 2 run the device LM (path 2) and fall back to the host LM (path 0), which 1 and 0 select.
+static int choose_path(const phovo_ctx* ctx) {
+  const bool coop = ctx->execution >= 2 && ctx->shard_world == 1 && !path_failed(ctx, 2);
+  if (ctx->cfg.mode == PHOVO_MODE_CERES) return coop ? 2 : 0;
+  if (coop) return ctx->execution == 3 && !path_failed(ctx, 3) ? 3 : 2;
+  return ctx->execution >= 1 && !path_failed(ctx, 1) ? 1 : 0;
 }
 
 extern "C" int phovo_optimize(phovo_ctx* ctx) {
   if (!ctx) return PHOVO_E_INVALID;
-  int rc = ready_to_solve(ctx);
+  int rc = begin_solve(ctx);
   if (rc) return rc;
-  CK(cudaSetDevice(ctx->device));
-  if ((rc = ensure_log(ctx, total_iterations(ctx) + 1))) return rc;
-  ctx->setup_timed = false;
-  CK(cudaEventRecord(ctx->ev_time[2].get(), ctx->stream));
-  ctx->last_used_graph = 0;
+  const bool ceres = ctx->cfg.mode == PHOVO_MODE_CERES;
   ctx->last_path = 0;
-  if (ctx->cfg.mode == PHOVO_MODE_CERES) {
-    if (ctx->execution >= 2 && !ctx->coop_broken && ctx->shard_world == 1) {
-      bool unavailable = false;
-      rc = optimize_ceres_coop(ctx, &unavailable);
-      if (rc) return rc;
-      if (!unavailable) { ctx->last_path = 2; return read_back(ctx); }
-      ctx->coop_broken = true;
-    }
-    return optimize_ceres(ctx);   // host-driven LM over GPU evaluations
+  int path;
+  do {   // a driver that cannot run marks its path failed, and the solve starts over on the next one down
+    path = choose_path(ctx);
+    if (ceres && path == 0) return optimize_ceres(ctx);   // host-driven LM over GPU evaluations
+    if (ceres) rc = optimize_ceres_coop(ctx);
+    else if (path >= 2) rc = optimize_coop(ctx, path);
+    else if (path == 1) rc = optimize_graph(ctx);
+    else rc = optimize_stream(ctx);
+  } while (rc == kPathUnavailable);
+  if (rc == PHOVO_OK && path != 1) {   // (the graph driver has read back)
+    CK(cudaGetLastError());
+    rc = read_back(ctx);
   }
-  if (ctx->execution >= 2 && !ctx->coop_broken && ctx->shard_world == 1) {
-    bool unavailable = false;
-    rc = optimize_coop(ctx, &unavailable);
-    if (rc) return rc;
-    if (!unavailable) { ctx->last_path = (ctx->execution == 3 && !ctx->cluster_broken) ? 3 : 2; return read_back(ctx); }
-    ctx->coop_broken = true;   // remember and use the graph path from now on
-  }
-  bool done = false;
-  if (ctx->use_graph && !ctx->graph_broken) {
-    rc = optimize_graph(ctx);
-    if (rc == PHOVO_OK) {
-      rc = read_back(ctx);
-      if (rc == PHOVO_OK || rc == PHOVO_E_NUMERIC) {
-        ctx->last_used_graph = 1;
-        ctx->last_path = 1;
-        int iters = 0;
-        for (int l = 0; l < ctx->cfg.num_levels; ++l) iters += ctx->h_pose.get()->iters_per_level[l];
-        ctx->launches += ctx->graph_launches_fixed + (int64_t)iters * ctx->graph_launches_per_iter;
-        return rc;
-      }
-    }
-    // graph construction or execution failed: remember, clear the error state and use plain launches
-    ctx->graph_broken = true;
-    ctx->graph_error = ctx->err;
-    ctx->invalidate_graph();
-    cudaGetLastError();
-    cudaStreamCaptureStatus st;
-    if (cudaStreamIsCapturing(ctx->stream, &st) == cudaSuccess && st != cudaStreamCaptureStatusNone) {
-      cudaGraph_t junk = nullptr;
-      cudaStreamEndCapture(ctx->stream, &junk);
-      if (junk) cudaGraphDestroy(junk);
-    }
-    cudaGetLastError();
-    done = false;
-  }
-  if (!done) {
-    rc = optimize_stream(ctx);
-    if (rc) return rc;
-    return read_back(ctx);
-  }
-  return PHOVO_OK;
+  // a cluster launch refused during this solve: path 2 ran that level and the rest
+  if (rc == PHOVO_OK || rc == PHOVO_E_NUMERIC) ctx->last_path = path == 3 && path_failed(ctx, 3) ? 2 : path;
+  return rc;
 }
 
-extern "C" int phovo_last_optimize_used_graph(const phovo_ctx* ctx) { return ctx ? ctx->last_used_graph : 0; }
-extern "C" const char* phovo_graph_error(const phovo_ctx* ctx) { return ctx ? ctx->graph_error.c_str() : ""; }
+extern "C" int phovo_last_optimize_used_graph(const phovo_ctx* ctx) { return ctx ? ctx->last_path == 1 : 0; }
+extern "C" const char* phovo_graph_error(const phovo_ctx* ctx) { return ctx ? ctx->path_note.c_str() : ""; }
 
 extern "C" int phovo_get_state(const phovo_ctx* ctx, double state[6]) {
   if (!ctx || !state) return PHOVO_E_INVALID;
@@ -982,9 +993,8 @@ static int optimize_ceres(phovo_ctx* ctx) {
   LmLog log{ctx->h_log.get(), log_count, ctx->log_cap(), true};
   LmState S;
   memcpy(S.x, ctx->state, sizeof(S.x));
-  for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
+  const int status = for_each_level(ctx->cfg, [&](int level, int) {   // CE:437
     const LmParams lm = lm_params(ctx->cfg, level);
-    if (!(lm.max_iterations > 0)) continue;   // CE:437
     S.radius = lm.initial_radius; S.decrease_factor = 2.0; S.iteration = 0;
     int rc = eval_at(ctx, level, S.x, &S.cur, nullptr, nullptr);
     if (rc) return rc;
@@ -996,7 +1006,9 @@ static int optimize_ceres(phovo_ctx* ctx) {
       if (v == LM_ACCEPT) S.cur = cand;
       go = v != LM_STOP && lm_update_radius(lm, S, v == LM_ACCEPT);
     }
-  }
+    return PHOVO_OK;
+  });
+  if (status) return status;
   ctx->log.assign(ctx->h_log.get(), ctx->h_log.get() + std::min(log_count, ctx->log_cap()));
   memcpy(ctx->state, S.x, sizeof(S.x));
   CK(cudaEventRecord(ctx->ev_time[3].get(), ctx->stream));
@@ -1043,12 +1055,9 @@ extern "C" int phovo_shard_write_buffer(phovo_ctx* ctx, const double in[32]) {
 
 extern "C" int phovo_shard_begin(phovo_ctx* ctx) {
   if (!ctx) return PHOVO_E_INVALID;
-  int rc = ready_to_solve(ctx);
+  const int rc = begin_solve(ctx);
   if (rc) return rc;
-  CK(cudaSetDevice(ctx->device));
-  if ((rc = ensure_log(ctx, total_iterations(ctx) + 1))) return rc;
-  CK(cudaEventRecord(ctx->ev_time[2].get(), ctx->stream));
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
+  upload_state(ctx);
   ctx->shard_level = -1;
   return PHOVO_OK;
 }
@@ -1136,15 +1145,13 @@ static int upload_peer_table(phovo_ctx* ctx) {
 
 extern "C" int phovo_shard_optimize(phovo_ctx* ctx, int min_shard_pixels) {
   if (!ctx) return PHOVO_E_INVALID;
-  int rc = ready_to_solve(ctx);
-  if (rc) return rc;
   if (ctx->cfg.mode != PHOVO_MODE_ANALYTIC_REF && ctx->cfg.mode != PHOVO_MODE_ANALYTIC_FIXED)
     return ctx->fail(PHOVO_E_UNSUPPORTED, "the row-sharded loop implements the analytic solver only");
-  if (ctx->coop_broken) return ctx->fail(PHOVO_E_UNSUPPORTED, "cooperative launch is not available on this device");
+  if (path_failed(ctx, 2)) return ctx->fail(PHOVO_E_UNSUPPORTED, "cooperative launch is not available on this device");
   if (ctx->shard_world > PHOVO_SHARD_MAX_WORLD) return ctx->fail(PHOVO_E_UNSUPPORTED, "peer exchange supports up to 8 ranks");
-  CK(cudaSetDevice(ctx->device));
+  int rc = begin_solve(ctx);
+  if (rc) return rc;
   if (ctx->shard_world > 1 && (rc = upload_peer_table(ctx))) return rc;
-  if ((rc = ensure_log(ctx, total_iterations(ctx) + 1))) return rc;
   if (ctx->shard_world > 1 && !ctx->level_dmin_valid) {   // once per source frame: what bounds the row displacement (ShardArgs)
     CK(ctx->d_level_dmin.ensure(PHOVO_MAX_LEVELS));
     for (int level = 0; level < ctx->cfg.num_levels; ++level)
@@ -1153,12 +1160,8 @@ extern "C" int phovo_shard_optimize(phovo_ctx* ctx, int min_shard_pixels) {
                                                 ctx->cfg.max_depth, ctx->d_level_dmin.get() + level, ctx->sm_count);
     ctx->level_dmin_valid = true;
   }
-  ctx->setup_timed = false;
-  CK(cudaEventRecord(ctx->ev_time[2].get(), ctx->stream));
-  ctx->launches += launch_set_state(ctx->stream, ctx->d_pose.get(), nullptr, ctx->state, ctx->log_cap());
-  for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {   // AN:502-503
-    const int M = ctx->cfg.max_num_iterations[level];
-    if (M <= 0) continue;
+  upload_state(ctx);
+  rc = for_each_level(ctx->cfg, [&](int level, int M) {
     LevelParams L = ctx->level_params(level);                          // carries this rank's row band
     const LevelPtrs P = ctx->level_ptrs(level);
     const bool shard = ctx->shard_world > 1 && (long long)L.rows * L.cols >= (long long)min_shard_pixels;
@@ -1170,16 +1173,12 @@ extern "C" int phovo_shard_optimize(phovo_ctx* ctx, int min_shard_pixels) {
     if (n < 0) { cudaGetLastError(); return ctx->cuda_fail("cooperative launch of the sharded level loop", e); }
     ctx->launches += n;
     if (shard) ctx->xchg_epoch += (unsigned long long)M;               // every rank advances by the same amount
-  }
+    return PHOVO_OK;
+  });
+  if (rc) return rc;
   CK(cudaGetLastError());
   ctx->last_path = 2;
-  rc = read_back(ctx);
-  if (ctx->xchg_own.get()) {
-    int err = 0;
-    CK(cudaMemcpy(&err, &ctx->xchg_own.get()->error, sizeof(int), cudaMemcpyDeviceToHost));
-    if (err) return ctx->fail(PHOVO_E_CUDA, "peer exchange timed out waiting for another rank");
-  }
-  return rc;
+  return end_solve(ctx);
 }
 
 extern "C" int phovo_shard_step(phovo_ctx* ctx, int* done) {
@@ -1199,11 +1198,5 @@ extern "C" int phovo_shard_step(phovo_ctx* ctx, int* done) {
 extern "C" int phovo_shard_finish(phovo_ctx* ctx) {
   if (!ctx) return PHOVO_E_INVALID;
   CK(cudaSetDevice(ctx->device));
-  int rc = read_back(ctx);
-  if (ctx->xchg_own.get()) {
-    int err = 0;
-    CK(cudaMemcpy(&err, &ctx->xchg_own.get()->error, sizeof(int), cudaMemcpyDeviceToHost));
-    if (err) return ctx->fail(PHOVO_E_CUDA, "peer exchange timed out waiting for another rank");
-  }
-  return rc;
+  return end_solve(ctx);
 }

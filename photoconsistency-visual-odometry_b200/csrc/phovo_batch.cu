@@ -204,16 +204,17 @@ static int make_params(phovo_ctx* ctx, int num_pairs, int rows, int cols, int lo
   bp->min_depth = ctx->cfg.min_depth; bp->max_depth = ctx->cfg.max_depth;
   int a = 0, nmax = 0;
   unsigned long long off = 0;
-  for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
-    if (ctx->cfg.max_num_iterations[level] <= 0) continue;
+  const int status = for_each_level(ctx->cfg, [&](int level, int M) {
     const int rc = fill_level(ctx, rows, cols, level, a, bp, &off);
     if (rc) return rc;
     const int n = bp->lrows[a] * bp->lcols[a];
     if (n > kBatchMaxLevelPixels) return ctx->fail(PHOVO_E_UNSUPPORTED, "batch kernel: an active level exceeds the shared-memory budget (about 20K px); use the per-pair API");
     nmax = std::max(nmax, n);
-    bp->max_iters[a] = ctx->cfg.max_num_iterations[level];
+    bp->max_iters[a] = M;
     ++a;
-  }
+    return PHOVO_OK;
+  });
+  if (status) return status;
   bp->num_active = a;
   bp->record_bytes = off ? off : 16;
   *smem_out = 0;
@@ -619,13 +620,12 @@ static int batch_waves(phovo_ctx* ctx, phovo_batch_state* b, int num_pairs, int 
     }
     if (!levels_known) {
       const phovo_ctx* c0 = w.slots[(size_t)h * half].get();
-      for (int level = ctx->cfg.num_levels - 1; level >= 0; --level) {
-        const int M = ctx->cfg.max_num_iterations[level];
-        if (!(M > 0)) continue;
+      for_each_level(ctx->cfg, [&](int level, int) {
         const int a = LS.count++;
         LS.L[a] = c0->level_params(level);
         LS.lm[a] = lm_params(ctx->cfg, level);
-      }
+        return 0;
+      });
       levels_known = true;
     }
     // ---- one launch aligns the wave; results to pinned memory ----

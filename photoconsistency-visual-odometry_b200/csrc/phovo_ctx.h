@@ -16,7 +16,8 @@ struct phovo_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
   phovo::Stream own_stream;   // the stream phovo_create made; empty once phovo_set_stream names another (and for slots)
-  std::string err, graph_error;
+  std::string err;
+  std::string path_note;   // why the last driver that failed on this context could not run (phovo_graph_error)
 
   phovo_config cfg;
   double K[9] = {0};
@@ -60,13 +61,13 @@ struct phovo_ctx {
   phovo::DeviceArray<double> d_state_in; phovo::PinnedArray<double> h_state_in;
   std::vector<phovo_iter_stats> log;
 
-  // CUDA graph of the whole Optimize()
-  bool use_graph = true, graph_broken = false;
-  // 2 (default): persistent cooperative kernel per level; 1: CUDA graph with WHILE nodes; 0: stream launches + host polling
-  int execution = 2; bool coop_broken = false; bool cluster_broken = false; int sm_count = 0; int last_path = 0;
+  // driver of Optimize() (phovo_set_execution): 3 cluster for small levels, 2 (default) persistent cooperative kernel per
+  // level, 1 CUDA graph with WHILE nodes, 0 stream launches + host polling.  Bit p of failed_paths: path p could not run
+  // on this context, and Optimize() no longer tries it.
+  int execution = 2; unsigned failed_paths = 0; int last_path = 0;
+  int sm_count = 0;
   cudaGraph_t graph = nullptr; cudaGraphExec_t graph_exec = nullptr;
   int graph_launches_fixed = 0, graph_launches_per_iter = 0;
-  int last_used_graph = 0;
 
   // row sharding
   int shard_rank = 0, shard_world = 1, shard_level = -1;
@@ -106,6 +107,19 @@ struct phovo_ctx {
   phovo::LevelPtrs level_ptrs(int level) const;
   void invalidate_graph();
 };
+
+// The coarse-to-fine walk of every solve (AN:502-503): fn(level, M) for each level with M = max_num_iterations[level] > 0,
+// coarsest first; a level without iterations is an empty pass (AN:526).  Stops at, and returns, fn's first non-zero
+// return.  It reads the configuration only: batch contexts have no frames.
+template <class Fn>
+int for_each_level(const phovo_config& cfg, Fn&& fn) {
+  for (int level = cfg.num_levels - 1; level >= 0; --level) {
+    const int M = cfg.max_num_iterations[level];
+    if (M <= 0) continue;
+    if (const int rc = fn(level, M)) return rc;
+  }
+  return 0;
+}
 
 void phovo_batch_release(phovo_ctx* ctx);
 // phovo::warpImage of `num_pairs` pairs (device pointers in W; rts host or device [num_pairs][16]), enqueued on the
